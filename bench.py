@@ -65,6 +65,26 @@ def build_workload(spec, seed):
                 radii=np.asarray(radii, dtype=np.float32), res_start=np.asarray(res_start, dtype=np.int32))
 
 
+def dump_outputs(out, directory, limit=64 << 20):
+    """Writes the arrays one step returns to a caller (``VoxelPass.results()``) as ``directory/<name>.npy`` in float64, so that
+    two builds can be compared output for output on the same seeded inputs.  An array larger than its share of ``limit``
+    bytes is cut to a fixed seeded sample of its rows (written as ``<name>_rows.npy`` beside it)."""
+    arrays = {"cloud": out["cloud"], "region": out["region"], "blob_counts": out["blob_counts"]}
+    for tag in ("green", "red"):
+        for k in ("key", "label", "stats"):
+            arrays[tag + "_" + k] = out[tag][k]
+    os.makedirs(directory, exist_ok=True)
+    share = limit // (2 * len(arrays))              # an array and its row indices
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.nbytes > share:
+            keep = max(1, share // (a.nbytes // len(a)) - 1)
+            rows = np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))
+            np.save(os.path.join(directory, name + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------ clocks sampler
 class ClockSampler:
     Q = ("clocks.sm,clocks.max.sm,clocks_event_reasons.hw_slowdown,clocks_event_reasons.hw_thermal_slowdown,"
@@ -469,6 +489,8 @@ def main_gpu(args, rank, world, local_rank):
     barrier()
     ms_e2e = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
     h2d = h_dens.numel() * 4 + h_diff.numel() * 4 + h_xyz.numel() * 8
     d2h = (out["cloud"].nbytes + out["region"].nbytes + out["blob_counts"].nbytes +
            sum(out[t][k].nbytes for t in ("green", "red") for k in ("key", "label", "stats")))
@@ -582,7 +604,7 @@ def main_gpu(args, rank, world, local_rank):
             # BASELINE.json configs[2] on this one GPU: the pool the N > 1 runs shard (their strong-scaling reference point)
             del vp, dens, diff, d_dens, d_diff
             torch.cuda.empty_cache()
-            line["c3"] = run_c3_one_gpu(args.pool, 3, device, synthetic.defaultParams())[0]
+            line["c3"] = run_c3_one_gpu(args.pool, args.steps, device, synthetic.defaultParams())[0]
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -699,7 +721,7 @@ def main_c3(args, rank, world, local_rank):
                 mref.deviceMap.rho.copy_(h, non_blocking=True)
             return shard.analyze(**kw)
 
-    e2e_steps = max(args.steps // 4, 2)
+    e2e_steps = args.steps
     ms_e2e, _, _ = _time_passes(_E2E(), e2e_steps, 1, barrier, device=device)
     clocks = sampler.stop() if rank == 0 else None
     h2d = sum(h.numel() * 4 for h in host_maps)
@@ -719,7 +741,7 @@ def main_c3(args, rank, world, local_rank):
         # strong-scaling denominator measured in the same run: the same pool on this GPU alone
         del shard, entries
         torch.cuda.empty_cache()
-        one, one_summary = run_c3_one_gpu(args.pool, max(args.steps // 4, 2), device, params)
+        one, one_summary = run_c3_one_gpu(args.pool, args.steps, device, params)
         a, b = _summary_digest(summary), one["summary"]
         close = lambda x, y: abs(x - y) <= 1e-9 * max(abs(x), abs(y), 1e-300)
         one["same_results_as_%d_gpus" % world] = bool(
@@ -820,7 +842,7 @@ def run_c4(args, rank, world, device):
     dist.barrier()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    reps = 10
+    reps = args.steps
     e0.record()
     for _ in range(reps):
         parts = lab.label(mine, cut, -cut)
@@ -871,10 +893,15 @@ def main():
     ap.add_argument("--no-c4", action="store_true", help="N > 1: skip the config-4 slab run")
     ap.add_argument("--no-c3", action="store_true", help="N = 1: skip the config-3 pool key")
     ap.add_argument("--no-c1", action="store_true", help="reference arm: skip the full-size config-1 pass")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="N = 1: write what the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and (args.impl != "b200" or world > 1):
+        ap.error("--dump-outputs writes the outputs of the one-GPU B200 run (--impl b200 without torchrun)")
     if args.impl == "reference":
         main_reference(args, rank, world)
     elif world > 1:

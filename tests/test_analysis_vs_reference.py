@@ -13,6 +13,7 @@ import numpy as np
 import pytest
 
 import golden_checks as gc
+import recorded
 from pdb_eda_b200 import synthetic, structure
 
 pytestmark = pytest.mark.gpu
@@ -42,16 +43,29 @@ def _build(name):
 
 
 @pytest.fixture(scope="module", params=list(CASES))
-def pair(request, ref):
-    ref_ccp4, ref_da, ref_cutils, ref_pp = ref
+def pair(request):
+    """(reference DensityAnalysis, this package's) on the same inputs; the first is None without the reference installed,
+    and the tests then compare with the recorded results (tests/recorded.py)."""
     from pdb_eda_b200 import ccp4, densityAnalysis, pdbParser
     st, d1, d2, pdb_text = _build(request.param)
+    ref = recorded.reference()
+    if ref is None:
+        densityAnalysis.setGlobals(densityAnalysis._loadDefaultParams())
+        m = densityAnalysis.fromFile(io.StringIO(pdb_text), io.BytesIO(d1), io.BytesIO(d2))
+        assert m != 0
+        (m1, s1), (m2, s2) = recorded.host_mean_std(m.densityObj), recorded.host_mean_std(m.diffDensityObj)
+        cuts = recorded.inputs("pair-" + request.param, [m1 + 1.5 * s1, m2 + 3 * s2])
+        gc.close([m.densityObj.densityCutoff, m.diffDensityObj.diffDensityCutoff], cuts)
+        m.densityObj.densityCutoff, m.diffDensityObj.diffDensityCutoff = cuts
+        return None, m
+    ref_ccp4, ref_da, ref_cutils, ref_pp = ref
     densityAnalysis.setGlobals(ref_da.paramsGlobal)
     # reference side
     r_dens = ref_ccp4.parse(io.BytesIO(d1), "t")
     r_diff = ref_ccp4.parse(io.BytesIO(d2), "t")
     r_dens.densityCutoff = r_dens.meanDensity + 1.5 * r_dens.stdDensity
     r_diff.diffDensityCutoff = r_diff.meanDensity + 3 * r_diff.stdDensity
+    recorded.inputs("pair-" + request.param, [r_dens.densityCutoff, r_diff.diffDensityCutoff], live=True)
     r_pdb = ref_pp.readPDBfile(io.StringIO(pdb_text))
     r = ref_da.DensityAnalysis("t", r_dens, r_diff, st, r_pdb)
     # this package, through its own loader (exercises fromFile, the PDB reader and the header parser)
@@ -75,8 +89,21 @@ def _same_rows(a, b, float_from):
                 gc.close(np.asarray(xa, dtype=np.float64), np.asarray(xb, dtype=np.float64), rtol=1e-9, atol=1e-9)
 
 
-def test_loader_and_structure(pair):
+def _blob(b):
+    return [np.array(sorted(b.crsList), dtype=np.int64).reshape(-1, 3), b.totalDensity, b.volume, list(b.centroid), list(b.coordCenter)]
+
+
+def _atom(a):
+    return [a.name, a.parent.id, getattr(a, "symmetry", None), np.asarray(a.coord, dtype=np.float64)]
+
+
+def test_loader_and_structure(pair, request):
     r, m = pair
+    if r is None:
+        h = m.pdbObj.header
+        recorded.check(request.node.name, [[_atom(a) for a in m.biopdbObj.get_atoms()], list(h.rotationMats), h.spaceGroup, h.resolution],
+                       rtol=0, atol=0)
+        return
     ra, ma = list(r.biopdbObj.get_atoms()), list(m.biopdbObj.get_atoms())
     assert len(ra) == len(ma)
     assert all(np.array_equal(x.coord, y.coord) and x.name == y.name for x, y in zip(ra, ma))
@@ -85,10 +112,16 @@ def test_loader_and_structure(pair):
     assert r.pdbObj.header.spaceGroup == m.pdbObj.header.spaceGroup and r.pdbObj.header.resolution == m.pdbObj.header.resolution
 
 
-def test_aggregate_cloud(pair):
+def test_aggregate_cloud(pair, request):
     r, m = pair
-    r.aggregateCloud()
     m.aggregateCloud()
+    if r is None:
+        assert m.densityElectronRatio is not None
+        recorded.check(request.node.name, [m.numVoxelsAggregated, m.densityElectronRatio, m.totalAggregatedDensity, m.totalAggregatedElectrons,
+                                           dict(m.atomTypeOverlapCompleteness), dict(m.atomTypeOverlapIncompleteness),
+                                           m.residueCloudDescriptions, m.domainCloudDescriptions, m.atomCloudDescriptions, m.medians])
+        return
+    r.aggregateCloud()
     assert r.densityElectronRatio is not None and m.densityElectronRatio is not None
     assert r.numVoxelsAggregated == m.numVoxelsAggregated
     gc.close([m.densityElectronRatio, m.totalAggregatedDensity, m.totalAggregatedElectrons],
@@ -110,8 +143,13 @@ def test_aggregate_cloud(pair):
         gc.close([m.medians[column][t] for t in r.medians[column]], [r.medians[column][t] for t in r.medians[column]], rtol=1e-9, atol=1e-9)
 
 
-def test_symmetry_atoms(pair):
+def test_symmetry_atoms(pair, request):
     r, m = pair
+    if r is None:
+        assert m.symmetryAtomCoords.dtype == np.float64
+        recorded.check(request.node.name, [len(m.symmetryOnlyAtoms), len(m.asymmetryAtoms), [a.symmetry for a in m.symmetryAtoms],
+                                           [(a.name, a.parent.id) for a in m.symmetryAtoms], m.symmetryAtomCoords], rtol=1e-12, atol=1e-10)
+        return
     rs, ms = r.symmetryAtoms, m.symmetryAtoms
     assert len(rs) == len(ms) and len(r.symmetryOnlyAtoms) == len(m.symmetryOnlyAtoms) and len(r.asymmetryAtoms) == len(m.asymmetryAtoms)
     assert [a.symmetry for a in rs] == [a.symmetry for a in ms]
@@ -120,8 +158,15 @@ def test_symmetry_atoms(pair):
     assert m.symmetryAtomCoords.dtype == r.symmetryAtomCoords.dtype
 
 
-def test_blob_lists_and_statistics(pair):
+def test_blob_lists_and_statistics(pair, request):
     r, m = pair
+    if r is None:
+        assert len(m.greenBlobList) > 3 and len(m.redBlobList) > 3
+        blobs = [[_blob(b) for b in getattr(m, tag)] for tag in ("greenBlobList", "redBlobList")]
+        m.aggregateCloud()
+        stats = [m.calculateAtomSpecificBlobStatistics(getattr(m, tag)) for tag in ("greenBlobList", "redBlobList")]
+        recorded.check(request.node.name, [blobs, stats])
+        return
     for tag in ("greenBlobList", "redBlobList"):
         rb, mb = getattr(r, tag), getattr(m, tag)
         assert len(rb) == len(mb) and len(rb) > 3
@@ -141,11 +186,28 @@ def test_blob_lists_and_statistics(pair):
                      [x[0], x[2], x[4]] + list(np.asarray(x[10], dtype=np.float64)) + list(x[11]), rtol=1e-9, atol=1e-9)
 
 
-def test_region_density_and_discrepancy(pair):
+def test_region_density_and_discrepancy(pair, request):
     r, m = pair
+    mask = {"ALA": ["N", "CA", "C"]}
+    if r is None:
+        m.aggregateCloud()
+        out = [m.calculateResidueRegionDensity(3.5, 1.5, "", mask), m.calculateResidueRegionDensity(3.5, 1.5, "ALA", None, True)]
+        assert len(m.calculateResidueRegionDensity(3.5, 1.5, "HOH", None, True)) == 5
+        with pytest.raises(IndexError):
+            m.calculateResidueRegionDiscrepancies(3.5, 3.0, "", mask)
+        out += [m.calculateResidueRegionDiscrepancies(3.5, 3.0, "ALA", mask), m.calculateAtomRegionDensity(2.0, 1.5, "CA"),
+                m.calculateAtomRegionDiscrepancies(2.0, 3.0, "O")]
+        m._symmetryAtoms = m.symmetryAtoms[::23]
+        try:
+            out += [m.calculateSymmetryAtomRegionDensity(2.0, 1.5), m.calculateSymmetryAtomRegionDiscrepancies(2.0, 3.0, "CB")]
+        finally:
+            m._symmetryAtoms = None
+        one = [a.coord for a in list(m.biopdbObj.get_atoms())[:4]]
+        out += [m.calculateRegionDensity(one, 2.5), m.calculateRegionDiscrepancy(one, 2.5)]
+        recorded.check(request.node.name, out)
+        return
     r.aggregateCloud()
     m.aggregateCloud()
-    mask = {"ALA": ["N", "CA", "C"]}
     _same_rows(m.calculateResidueRegionDensity(3.5, 1.5, "", mask), r.calculateResidueRegionDensity(3.5, 1.5, "", mask), 4)
     # per-atom optimised radii; restricted to ALA because the reference raises TypeError on single-atom residues here
     # (pdb_eda/ccp4.py:457 hands the radius list to a Cython float parameter) -- this package handles them
@@ -179,10 +241,17 @@ def test_region_density_and_discrepancy(pair):
     gc.close(m.calculateRegionDiscrepancy(one, 2.5), r.calculateRegionDiscrepancy(one, 2.5), rtol=1e-9, atol=1e-12)
 
 
-def test_rscc_rsr_metrics(pair):
+def test_rscc_rsr_metrics(pair, request):
     """residueMetrics / atomMetrics / calculateRsccRsrMetrics / medianAbsFoFc (SURVEY.md section 8f-3)."""
     import warnings
     r, m = pair
+    if r is None:
+        rres = m.residueMetrics()
+        assert np.isfinite(np.array([x[3] for x in rres], dtype=np.float64)).sum() > len(rres) // 2
+        crs = m.densityObj.getSphereCrsFromXyz(m.asymmetryAtoms[3].coord, 1.4, 0.0)
+        recorded.check(request.node.name, [rres, m.atomMetrics(m.asymmetryAtoms[::7]), m.medianAbsFoFc(), m.calculateRsccRsrMetrics(crs),
+                                           np.asarray(m.fc.density)], rtol=1e-8)
+        return
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
         rres = r.residueMetrics()
@@ -203,10 +272,15 @@ def test_rscc_rsr_metrics(pair):
     assert np.array_equal(np.asarray(m.fc.density), r.fc.density)
 
 
-def test_blue_blob_list(pair):
+def test_blue_blob_list(pair, request):
     """blueBlobList: createFullBlobList(mean + 1.5 sigma) on the 2Fo-Fc map (pdb_eda/densityAnalysis.py:414-423) -- dense
     foreground (the reference warns that it "uses a LOT OF MEMORY at 1.5sd", pdb_eda/singleStructure.py:30)."""
     r, m = pair
+    if r is None:
+        mb = m.blueBlobList
+        assert len(mb) >= 1 and sum(len(q.crsList) for q in mb) > 1000
+        recorded.check(request.node.name, [_blob(b) for b in mb])
+        return
     rb, mb = r.blueBlobList, m.blueBlobList
     assert len(rb) == len(mb) >= 1 and sum(len(p.crsList) for p in rb) > 1000
     assert all(p.crsList == q.crsList for p, q in zip(rb, mb))                       # membership and order
@@ -215,10 +289,20 @@ def test_blue_blob_list(pair):
     gc.close([q.centroid for q in mb], [p.centroid for p in rb], rtol=1e-9, atol=1e-9)
 
 
-def test_fc_object_and_single_coordinate_regions(pair):
+def test_fc_object_and_single_coordinate_regions(pair, request):
     """ADVICE items: the public ``fc`` attribute answers the calls the reference's deep copy answers, and the region methods
     accept a single flat coordinate like findAberrantBlobs does (pdb_eda/ccp4.py:453)."""
     r, m = pair
+    if r is None:
+        cut = m.densityObj.densityCutoff
+        assert m.fc.meanDensity == m.densityObj.meanDensity
+        one = [float(v) for v in m.asymmetryAtoms[7].coord]
+        gc.close(m.calculateRegionDiscrepancy(one, 2.5), m.calculateRegionDiscrepancy([one], 2.5), rtol=0, atol=0)
+        recorded.check(request.node.name + "-exact", [[float(m.fc.getPointDensityFromCrs(crs)) for crs in ([3, 4, 5], [-2, 70, 1], [10 ** 3, 0, 0])],
+                                                      m.fc.getTotalAbsDensity(cut), m.calculateRegionDensity(one, 2.5)], rtol=1e-9, atol=1e-12)
+        blobs = m.fc.findAberrantBlobs(list(m.asymmetryAtoms[5].coord), 2.0, cut)       # float32-narrowed Fc on the device
+        recorded.check(request.node.name + "-fc-blobs", sorted(b.totalDensity for b in blobs), rtol=1e-5, atol=0)
+        return
     for crs in ([3, 4, 5], [-2, 70, 1], [10 ** 3, 0, 0]):
         assert float(m.fc.getPointDensityFromCrs(crs)) == float(r.fc.getPointDensityFromCrs(crs))
     cut = r.densityObj.densityCutoff
@@ -255,7 +339,7 @@ def test_from_pdbid_uses_the_cache(pair, tmp_path, monkeypatch):
     assert densityAnalysis.cleanPDBid("9xyz") and not os.path.exists("ccp4_data/9xyz.ccp4")
 
 
-def test_error_conventions(pair, ref):
+def test_error_conventions(pair):
     r, m = pair
     from pdb_eda_b200 import densityAnalysis
     assert densityAnalysis.fromFile("/nonexistent/file.pdb") == 0

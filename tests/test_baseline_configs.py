@@ -15,27 +15,43 @@ import numpy as np
 import pytest
 
 import golden_checks as gc
+import recorded
 from pdb_eda_b200 import structure, synthetic
 
 pytestmark = pytest.mark.gpu
 
 
-def _pair(ref, st, n, cell, sg, seed):
-    """(reference DensityAnalysis, this package's) on the same synthetic inputs, identical float32-narrowed cutoffs."""
-    ref_ccp4, ref_da, ref_cutils, ref_pp = ref
+def _pair(ref, name, st, n, cell, sg, seed):
+    """(reference DensityAnalysis, this package's) on the same synthetic inputs, identical float32-narrowed cutoffs.  Without
+    the reference installed (ref None) the first is None and the tests compare with the recorded results (tests/recorded.py)."""
     from pdb_eda_b200 import densityAnalysis
     d1, d2 = synthetic.mapPair(st, n, cell, seed=seed)
     b1, b2 = synthetic.ccp4Bytes(d1, cell, n), synthetic.ccp4Bytes(d2, cell, n)
     text = structure.formatPDB(st, remark290=synthetic.cartesianOperators(sg, cell), cell=cell, spaceGroup=sg)
+    if ref is None:
+        densityAnalysis.setGlobals(densityAnalysis._loadDefaultParams())
+        m = densityAnalysis.fromFile(io.StringIO(text), io.BytesIO(b1), io.BytesIO(b2))
+        assert m != 0
+        (m1, s1), (m2, s2) = recorded.host_mean_std(m.densityObj), recorded.host_mean_std(m.diffDensityObj)
+        cuts = recorded.inputs(name, [m1 + 1.5 * s1, m2 + 3 * s2])
+        gc.close([m.densityObj.densityCutoff, m.diffDensityObj.diffDensityCutoff], cuts)
+        m.densityObj.densityCutoff, m.diffDensityObj.diffDensityCutoff = cuts
+        return None, m
+    ref_ccp4, ref_da, ref_cutils, ref_pp = ref
     densityAnalysis.setGlobals(ref_da.paramsGlobal)
     dens, diff = ref_ccp4.parse(io.BytesIO(b1), "t"), ref_ccp4.parse(io.BytesIO(b2), "t")
     dens.densityCutoff = dens.meanDensity + 1.5 * dens.stdDensity
     diff.diffDensityCutoff = diff.meanDensity + 3 * diff.stdDensity
+    recorded.inputs(name, [dens.densityCutoff, diff.diffDensityCutoff], live=True)
     r = ref_da.DensityAnalysis("t", dens, diff, st, ref_pp.readPDBfile(io.StringIO(text)))
     m = densityAnalysis.fromFile(io.StringIO(text), io.BytesIO(b1), io.BytesIO(b2))
     assert m != 0
     m.densityObj.densityCutoff, m.diffDensityObj.diffDensityCutoff = dens.densityCutoff, diff.diffDensityCutoff
     return r, m
+
+
+def _blobs(blobs):
+    return [[np.array(sorted(b.crsList), dtype=np.int64).reshape(-1, 3), b.totalDensity] for b in blobs]
 
 
 def _rows_close(mine, theirs, nExact):
@@ -50,12 +66,26 @@ def _rows_close(mine, theirs, nExact):
 
 
 @pytest.mark.timeout(900)
-def test_c1_full_size_against_the_live_reference(ref):
+def test_c1_full_size_against_the_live_reference():
     """BASELINE.json configs[0]: single-structure mode on a 96^3 P2(1)2(1)2(1) map pair with a 2,500-atom structure."""
     n, cell = (96, 96, 96), (48.0, 48.0, 48.0, 90, 90, 90)
     st = synthetic.polyAlaStructure(500, (0, 0, 0), cell[:3], seed=1, residuesPerChain=250)
-    r, m = _pair(ref, st, n, cell, "P 21 21 21", 7)
+    r, m = _pair(recorded.reference(), "test_c1_full_size", st, n, cell, "P 21 21 21", 7)
     assert len(list(m.biopdbObj.get_atoms())) == 2500
+    mask = {"ALA": ["N", "CA", "C"]}
+    if r is None:
+        m.aggregateCloud()
+        assert m.numVoxelsAggregated > 20000 and len(m.atomCloudDescriptions) > 2000
+        assert len(m.greenBlobList) > 100 and len(m.redBlobList) > 100 and len(m.symmetryAtoms) > 10000
+        recorded.check("test_c1_full_size-clouds", [m.numVoxelsAggregated, m.densityElectronRatio, m.totalAggregatedDensity, m.totalAggregatedElectrons,
+                                                    dict(m.atomTypeOverlapCompleteness), dict(m.atomTypeOverlapIncompleteness),
+                                                    m.residueCloudDescriptions, m.domainCloudDescriptions, m.atomCloudDescriptions["num_voxels"],
+                                                    m.medians, _blobs(m.greenBlobList), _blobs(m.redBlobList),
+                                                    [row[:10] for row in m.calculateAtomSpecificBlobStatistics(m.greenBlobList + m.redBlobList)],
+                                                    m.calculateResidueRegionDensity(3.5, 1.5, "", mask)[:120],
+                                                    m.calculateResidueRegionDiscrepancies(3.5, 3.0, "ALA", mask)[:120]])
+        recorded.check("test_c1_full_size-symmetry", [[a.symmetry for a in m.symmetryAtoms], m.symmetryAtomCoords], rtol=1e-12, atol=1e-10)
+        return
     r.aggregateCloud()
     m.aggregateCloud()
     assert r.numVoxelsAggregated == m.numVoxelsAggregated > 20000
@@ -79,7 +109,6 @@ def test_c1_full_size_against_the_live_reference(ref):
     blobs_r, blobs_m = r.greenBlobList + r.redBlobList, m.greenBlobList + m.redBlobList
     _rows_close([row[:10] for row in m.calculateAtomSpecificBlobStatistics(blobs_m)],
                 [row[:10] for row in r.calculateAtomSpecificBlobStatistics(blobs_r)], 0)
-    mask = {"ALA": ["N", "CA", "C"]}
     # the reference needs ~0.17 s per residue at 3.5 A: the first 120 residues through the public method via its type-free path
     sub = lambda an: [res for k, res in enumerate(an.biopdbObj.get_residues()) if k < 120]
     _rows_close(m.calculateResidueRegionDensity(3.5, 1.5, "", mask)[:120], _residue_density(r, sub(r), 3.5, 1.5, mask), 4)
@@ -110,7 +139,7 @@ def _residue_discrepancy(an, residues, radius, numSD, atomMask):
 
 
 @pytest.mark.timeout(900)
-def test_c5_symmetry_heavy_hexagonal_cell(ref):
+def test_c5_symmetry_heavy_hexagonal_cell():
     """BASELINE.json configs[4]: P6(5)22, cell 60 x 60 x 120 A (gamma = 120), 120 x 120 x 240 intervals, 2,000 atoms:
     324 images per atom, atom-mask density around the residues, blob distances over the generated symmetry atoms."""
     n, cell = (120, 120, 240), (60.0, 60.0, 120.0, 90, 90, 120)
@@ -118,7 +147,22 @@ def test_c5_symmetry_heavy_hexagonal_cell(ref):
     lo, hi = omat @ np.array([0.3, 0.3, 0.1]), omat @ np.array([0.6, 0.7, 0.9])
     lo, hi = np.minimum(lo, hi), np.maximum(lo, hi)
     st = synthetic.polyAlaStructure(400, lo - 3, hi + 3, seed=9, residuesPerChain=100)
-    r, m = _pair(ref, st, n, cell, "P 65 2 2", 13)
+    r, m = _pair(recorded.reference(), "test_c5_hexagonal", st, n, cell, "P 65 2 2", 13)
+    mask = {"ALA": ["N", "CA", "C"]}
+    if r is None:
+        assert len(m.pdbObj.header.rotationMats) == 12 and len(m.symmetryAtoms) > 20000
+        recorded.check("test_c5_hexagonal-symmetry", [[a.symmetry for a in m.symmetryAtoms], [(a.name, a.parent.id) for a in m.symmetryAtoms],
+                                                      m.symmetryAtomCoords], rtol=1e-12, atol=1e-10)
+        m.aggregateCloud()
+        blobs = m.greenBlobList + m.redBlobList
+        assert len(blobs) > 1000
+        mine = m.calculateSymmetryAtomRegionDensity(2.0, 1.5, "CA")[:150]
+        recorded.check("test_c5_hexagonal-regions", [m.numVoxelsAggregated, m.densityElectronRatio, _blobs(blobs),
+                                                     [row[:10] for row in m.calculateAtomSpecificBlobStatistics(blobs)],
+                                                     m.calculateResidueRegionDensity(3.5, 1.5, "", mask)[:80],
+                                                     [row[:6] + row[7:] for row in mine]])
+        recorded.check("test_c5_hexagonal-symmetry-coords", [np.asarray(row[6], dtype=np.float64) for row in mine], rtol=1e-12, atol=1e-10)
+        return
     assert len(r.pdbObj.header.rotationMats) == 12
     rs, ms = r.symmetryAtoms, m.symmetryAtoms
     assert len(rs) == len(ms) > 20000
@@ -134,7 +178,6 @@ def test_c5_symmetry_heavy_hexagonal_cell(ref):
     assert all(p.crsList == q.crsList for p, q in zip(blobs_r, blobs_m))
     _rows_close([row[:10] for row in m.calculateAtomSpecificBlobStatistics(blobs_m)],
                 [row[:10] for row in r.calculateAtomSpecificBlobStatistics(blobs_r)], 0)
-    mask = {"ALA": ["N", "CA", "C"]}
     sub = [res for k, res in enumerate(r.biopdbObj.get_residues()) if k < 80]
     _rows_close(m.calculateResidueRegionDensity(3.5, 1.5, "", mask)[:80], _residue_density(r, sub, 3.5, 1.5, mask), 4)
     # symmetry-atom variant (fully-within-map flag, testValidXyzList) on the first images

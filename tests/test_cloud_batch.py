@@ -3,7 +3,8 @@
 CPU tier: the batch-wide statistics block against the per-structure restatement of pdb_eda/densityAnalysis.py:734-766
 (``DensityAnalysis._atomTypeStatistics``, itself checked against the live reference in test_analysis_vs_reference.py).
 GPU tier: ``CloudBatch`` over several structures in ONE batch against the REAL reference's ``aggregateCloud`` run on each
-structure (oracle/_ref on the host CPU): every number ``analyzePDBID`` (pdb_eda/multipleStructures.py:320-356) reads.
+structure (oracle/_ref on the host CPU; without it, against the recorded results of tests/recorded.py): every number
+``analyzePDBID`` (pdb_eda/multipleStructures.py:320-356) reads.
 """
 import io
 
@@ -85,17 +86,28 @@ def test_segmented_median_and_std():
 
 
 @pytest.mark.gpu
-def test_cloud_batch_matches_the_reference(ref):
+def test_cloud_batch_matches_the_reference():
+    """Without the reference installed: against the recorded results (tests/recorded.py)."""
+    import recorded
     import test_analysis_vs_reference as tar
     from pdb_eda_b200 import cloudBatch, densityAnalysis, pdbParser
-    ref_ccp4, ref_da, ref_cutils, ref_pp = ref
-    densityAnalysis.setGlobals(ref_da.paramsGlobal)
-    params = ref_da.paramsGlobal
+    ref = recorded.reference()
+    params = ref[1].paramsGlobal if ref else densityAnalysis._loadDefaultParams()
+    densityAnalysis.setGlobals(params)
     refs, items = [], []
     for name in tar.CASES:
         st, d1, d2, pdb_text = tar._build(name)
+        if ref is None:
+            m = densityAnalysis.fromFile(io.StringIO(pdb_text), io.BytesIO(d1), io.BytesIO(d2))
+            mean, std = recorded.host_mean_std(m.densityObj)
+            m.densityObj.densityCutoff = recorded.inputs("cloud_batch-" + name, [mean + 1.5 * std])[0]
+            items.append((m.densityObj, cloudBatch.AtomTable.fromStructure(m.biopdbObj, params)))
+            assert items[-1][1].supported
+            continue
+        ref_ccp4, ref_da, ref_cutils, ref_pp = ref
         r_dens = ref_ccp4.parse(io.BytesIO(d1), "t")
         r_dens.densityCutoff = r_dens.meanDensity + 1.5 * r_dens.stdDensity
+        recorded.inputs("cloud_batch-" + name, [r_dens.densityCutoff], live=True)
         r = ref_da.DensityAnalysis("t", r_dens, None, st, ref_pp.readPDBfile(io.StringIO(pdb_text)))
         r.aggregateCloud()
         assert r.densityElectronRatio is not None
@@ -113,6 +125,13 @@ def test_cloud_batch_matches_the_reference(ref):
     items.append((m.densityObj, cloudBatch.AtomTable.fromStructure(m.biopdbObj, params)))
     results = cloudBatch.CloudBatch(items, params).run()
     assert results[-1].densityElectronRatio is None
+    if ref is None:
+        assert all(res.densityElectronRatio is not None for res in results[:-1])
+        recorded.check("test_cloud_batch_matches_the_reference",
+                       [[res.numVoxelsAggregated, res.densityElectronRatio, res.totalAggregatedDensity, res.totalAggregatedElectrons,
+                         dict(res.atomTypeOverlapCompleteness), dict(res.atomTypeOverlapIncompleteness), res.numAtomsAnalyzed,
+                         res.numResidueClouds, res.numDomainClouds, res.medians] for res in results[:-1]])
+        return
     for r, res in zip(refs, results):
         assert res.numVoxelsAggregated == r.numVoxelsAggregated
         gc.close([res.densityElectronRatio, res.totalAggregatedDensity, res.totalAggregatedElectrons],
@@ -130,13 +149,12 @@ def test_cloud_batch_matches_the_reference(ref):
 
 
 @pytest.mark.gpu
-def test_cloud_batch_is_deterministic_and_order_independent(ref):
+def test_cloud_batch_is_deterministic_and_order_independent():
     """The same structures in another batch order / alone give identical numbers (no cross-structure leakage)."""
     import test_analysis_vs_reference as tar
     from pdb_eda_b200 import cloudBatch, densityAnalysis
-    ref_da = ref[1]
-    densityAnalysis.setGlobals(ref_da.paramsGlobal)
-    params = ref_da.paramsGlobal
+    params = densityAnalysis._loadDefaultParams()
+    densityAnalysis.setGlobals(params)
     items = []
     for name in ("p212121", "perm"):
         st, d1, d2, pdb_text = tar._build(name)
@@ -232,7 +250,7 @@ def test_statistics_kernel_matches_the_numpy_statement():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("radiusScale", [1.0, 1.8, 3.0])
-def test_pair_path_equals_the_hash_table_path(ref, radiusScale, monkeypatch):
+def test_pair_path_equals_the_hash_table_path(radiusScale, monkeypatch):
     """pe_cloud_aggregate merges clouds through the atom grid + pair kernel and keeps the voxel hash table as the fallback for
     batches the pair kernel's frame cannot hold (a DEVICE flag decides; PE_CLOUD_FORCE_HASH=1 forces the fallback).  Both must give
     the same per-atom records and per-structure totals, bit for bit -- at the atom-type radii (candidate boxes of <= 256 voxels: 8
@@ -242,8 +260,7 @@ def test_pair_path_equals_the_hash_table_path(ref, radiusScale, monkeypatch):
     import copy
     import test_analysis_vs_reference as tar
     from pdb_eda_b200 import cloudBatch, densityAnalysis
-    ref_da = ref[1]
-    params = copy.deepcopy(ref_da.paramsGlobal)
+    params = copy.deepcopy(densityAnalysis._loadDefaultParams())
     params["radii"] = {k: float(np.float32(v * radiusScale)) for k, v in params["radii"].items()}
     densityAnalysis.setGlobals(params)
     try:
@@ -274,7 +291,7 @@ def test_pair_path_equals_the_hash_table_path(ref, radiusScale, monkeypatch):
             assert np.array_equal(arr0["medians"][column], arr1["medians"][column], equal_nan=True), column
         assert arr0["numVoxels"].sum() > 0
     finally:
-        densityAnalysis.setGlobals(ref_da.paramsGlobal)
+        densityAnalysis.setGlobals(densityAnalysis._loadDefaultParams())
 
 
 @pytest.mark.gpu

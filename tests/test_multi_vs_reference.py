@@ -6,7 +6,8 @@ objects (oracle/_ref, Cython cutils, on the host CPU) through the statements of
   * ``processFunction``              pdb_eda/optimizeParams.py:434-436       (diffs / slopes: a missing or NaN type is omitted)
   * ``calculateMedianDiffsSlopes``   pdb_eda/optimizeParams.py:360-408       (gather over structures, medians, completeness)
 restated line by line below, and compare with this package's per-structure path (``multi.analyzeStructure``), its batched
-path (``multi.PoolShard`` -> ``packBatch`` -> ``gatherPacked``) and ``multi.OptimizeService``.
+path (``multi.PoolShard`` -> ``packBatch`` -> ``gatherPacked``) and ``multi.OptimizeService``.  Without the reference
+installed, the same paths are compared with each other and with the recorded results of tests/recorded.py.
 """
 import io
 
@@ -14,6 +15,7 @@ import numpy as np
 import pytest
 
 import golden_checks as gc
+import recorded
 from pdb_eda_b200 import structure, synthetic
 
 
@@ -106,9 +108,19 @@ def _tiny_entry():
 
 
 @pytest.fixture(scope="module")
-def both(ref):
-    ref_ccp4, ref_da, ref_cutils, ref_pp = ref
+def both():
+    """(parameters, reference analyzers or None without the reference installed, this package's analyzers)."""
     from pdb_eda_b200 import densityAnalysis
+    ref = recorded.reference()
+    if ref is None:
+        params = densityAnalysis._loadDefaultParams()
+        densityAnalysis.setGlobals(params)
+        mine = [densityAnalysis.fromFile(io.StringIO(text), io.BytesIO(d1), io.BytesIO(d2)) for _, text, d1, d2 in _entries() + [_tiny_entry()]]
+        stats = [recorded.host_mean_std(m.densityObj) for m in mine]
+        for m, cut in zip(mine, recorded.inputs("multi", [mean + 1.5 * std for mean, std in stats])):
+            m.densityObj.densityCutoff = cut
+        return params, None, mine
+    ref_ccp4, ref_da, ref_cutils, ref_pp = ref
     params = ref_da.paramsGlobal
     densityAnalysis.setGlobals(params)
     refs, mine = [], []
@@ -121,6 +133,7 @@ def both(ref):
         m = densityAnalysis.fromFile(io.StringIO(text), io.BytesIO(d1), io.BytesIO(d2))
         m.densityObj.densityCutoff = dens.densityCutoff
         mine.append(m)
+    recorded.inputs("multi", [r.densityObj.densityCutoff for r in refs], live=True)
     assert refs[-1].densityElectronRatio is None and all(r.densityElectronRatio for r in refs[:-1])
     return params, refs, mine
 
@@ -138,6 +151,17 @@ def test_rows_of_analyzePDBID(both):
     assert rows[:, 0].tolist() == [0.0, 1.0, 2.0, 3.0]                      # the structure with too few electrons has no row
     ns = 1 + len(multi.STAT_COLUMNS)
     col = {c: 1 + k for k, c in enumerate(multi.STAT_COLUMNS)}
+    if refs is None:
+        singles = [multi.analyzeStructure(m, types) for m in mine[:-1]]
+        for k, single in enumerate(singles):
+            gc.close(rows[k, ns:ns + len(types)], [single["diffs"][t] for t in types], rtol=1e-9, atol=1e-12)
+            for name in multi.STAT_COLUMNS[:-1]:                               # all but execution_time
+                gc.close(rows[k, col[name]], single["stats"][name], rtol=1e-9)
+        assert multi.analyzeStructure(mine[-1], types) == 0
+        recorded.check("test_rows_of_analyzePDBID", [cumulative, np.delete(rows, col["execution_time"], axis=1),
+                                                     [[single["diffs"], [single["stats"][c] for c in multi.STAT_COLUMNS[:-1]]] for single in singles]],
+                       atol=1e-12)
+        return
     for k, (r, m) in enumerate(zip(refs[:-1], mine[:-1])):
         diffs, stats = ref_analyzePDBID(r, params["radii"])
         single = multi.analyzeStructure(m, types)
@@ -157,8 +181,15 @@ def test_calculateMedianDiffsSlopes(both, tmp_path):
     against the batched shard, the per-structure path and OptimizeService."""
     from pdb_eda_b200 import cloudBatch, multi
     params, refs, mine = both
-    want = ref_calculateMedianDiffsSlopes([ref_processFunction(r, params) if r.densityElectronRatio else 0 for r in refs], params)
     types = list(params["radii"])
+    if refs is None:
+        batched = multi.PoolShard([(k, m.densityObj, cloudBatch.AtomTable.fromStructure(m.biopdbObj, params)) for k, m in enumerate(mine)],
+                                  params).analyze(optimizer=True)
+        want = (batched["medianDiffs"], batched["meanDiffs"], batched["overallStdDevDiffs"], batched["medianSlopes"], batched["sizeDiffs"],
+                batched["atomTypeOverlapCompleteness"])
+        recorded.check("test_calculateMedianDiffsSlopes", list(want), atol=1e-12)
+    else:
+        want = ref_calculateMedianDiffsSlopes([ref_processFunction(r, params) if r.densityElectronRatio else 0 for r in refs], params)
     entries = [(k, m.densityObj, cloudBatch.AtomTable.fromStructure(m.biopdbObj, params)) for k, m in enumerate(mine)]
     batched = multi.PoolShard(entries, params).analyze(optimizer=True)
     single = multi.gatherResults({k: multi.analyzeStructure(m, types, optimizer=True) for k, m in enumerate(mine)}, list(range(len(mine))),

@@ -1,10 +1,16 @@
 """CPU tier: the restatement oracle against the REAL reference run live (oracle/_ref), on seeds the golden fixtures
-do not contain.  Skipped where the reference install is absent."""
+do not contain.  Where the reference install is absent, against the recorded results of tests/recorded.py."""
 import numpy as np
 import pytest
 
 import cases
+import recorded
 from impl_oracle import OracleImpl
+
+
+def _corners(h):
+    corners = [h.crs2xyzCoord([c, r, s]) for c in [0, h.ncrs[0] - 1] for r in [0, h.ncrs[1] - 1] for s in [0, h.ncrs[2] - 1]]
+    return [sorted(float(p[k]) for p in corners) for k in range(3)]
 
 
 class _Atom:
@@ -13,10 +19,27 @@ class _Atom:
 
 
 @pytest.mark.parametrize("name,seed", [("ortho", 23), ("perm", 29), ("hex", 31), ("tric", 37)])
-def test_oracle_matches_live_reference(ref, name, seed):
-    ref_ccp4, ref_da, ref_cutils, _ = ref
+def test_oracle_matches_live_reference(name, seed, request):
     from pdb_eda_b200 import ccp4 as my_ccp4, synthetic
     data, _ = cases.make_case(name, seed)
+    ref = recorded.reference()
+    if ref is None:
+        mdm = cases.parse_with(my_ccp4, data)
+        orc = OracleImpl(mdm)
+        rng = np.random.default_rng(seed)
+        atoms = cases.random_atoms(mdm, 8, seed=seed + 1)      # from the header, bit-identical to the reference's (test_oracle_golden)
+        radii = rng.uniform(0.5, 2.4, len(atoms))
+        mean, std = recorded.host_mean_std(mdm)
+        cut, bcut = recorded.inputs(request.node.name, [mean + 1.3 * std, mean + 2.4 * std])
+        out = [[orc.sphere_lists(atoms, radii, c) for c in (0.0, cut, -cut)], orc.sphere_sums(atoms[:4], np.full(4, 2.2), np.array([0, 4]), cut, -cut)[0],
+               orc.full_blobs(bcut, -bcut)]
+        ops = synthetic.cartesianOperators("P 21 21 21" if name != "hex" else "P 65 2 2", cases.GEOMETRIES[name]["cell"])
+        xs, ys, zs = _corners(mdm.header)
+        shift = np.array([np.dot(mdm.header.orthoMat, (i, j, k)) for i in (-1, 0, 1) for j in (-1, 0, 1) for k in (-1, 0, 1)])
+        out.append(orc.symmetry(atoms.astype(np.float64), ops, shift, [xs[0] - 5, ys[0] - 5, zs[0] - 5], [xs[-1] + 5, ys[-1] + 5, zs[-1] + 5]))
+        recorded.check(request.node.name, out, rtol=1e-12, atol=1e-10)
+        return
+    ref_ccp4, ref_da, ref_cutils, _ = ref
     rdm = cases.parse_with(ref_ccp4, data)
     mdm = cases.parse_with(my_ccp4, data)
     orc = OracleImpl(mdm)
@@ -24,6 +47,7 @@ def test_oracle_matches_live_reference(ref, name, seed):
     atoms = cases.random_atoms(rdm, 8, seed=seed + 1)
     radii = rng.uniform(0.5, 2.4, len(atoms))
     cut = float(rdm.meanDensity + 1.3 * rdm.stdDensity)
+    recorded.inputs(request.node.name, [cut, float(rdm.meanDensity + 2.4 * rdm.stdDensity)], live=True)
     for c in (0.0, cut, -cut):
         want = [rdm.getSphereCrsFromXyz(a, r, c) for a, r in zip(atoms, radii)]
         crs, off = orc.sphere_lists(atoms, radii, c)
@@ -56,11 +80,25 @@ def test_oracle_matches_live_reference(ref, name, seed):
 
 
 @pytest.mark.parametrize("seed", [1, 2, 5, 8])
-def test_oracle_matches_live_reference_on_random_geometries(ref, seed):
+def test_oracle_matches_live_reference_on_random_geometries(seed, request):
     """The geometries of the GPU fuzz test (tests/test_cuda_vs_oracle.py::test_fuzz_random_geometries), oracle vs reference."""
-    ref_ccp4, _, ref_cutils, _ = ref
     from pdb_eda_b200 import ccp4 as my_ccp4
     data, _ = cases.random_geometry(seed)
+    ref = recorded.reference()
+    if ref is None:
+        mdm = cases.parse_with(my_ccp4, data)
+        orc = OracleImpl(mdm)
+        rng = np.random.default_rng(seed)
+        atoms = cases.random_atoms(mdm, 6, seed=seed + 50, margin=4.0)
+        radii = rng.uniform(0.4, 2.6, len(atoms))
+        mean, std = recorded.host_mean_std(mdm)
+        cut, bcut = recorded.inputs(request.node.name, [mean + 1.1 * std, mean + 2.2 * std])
+        out = [[orc.sphere_lists(atoms, radii, c) for c in (0.0, cut, -cut)], orc.full_blobs(bcut, -bcut)]
+        pts = np.stack([rng.integers(-2 * mdm.header.crsInterval[k], 3 * mdm.header.crsInterval[k], 60) for k in range(3)], axis=1)
+        out.append(orc.point_density(pts))
+        recorded.check(request.node.name, out, rtol=0, atol=0)
+        return
+    ref_ccp4, _, ref_cutils, _ = ref
     rdm = cases.parse_with(ref_ccp4, data)
     mdm = cases.parse_with(my_ccp4, data)
     assert np.array_equal(np.asarray(rdm.header.origin, float), np.asarray(mdm.header.origin, float))
@@ -70,6 +108,7 @@ def test_oracle_matches_live_reference_on_random_geometries(ref, seed):
     atoms = cases.random_atoms(rdm, 6, seed=seed + 50, margin=4.0)
     radii = rng.uniform(0.4, 2.6, len(atoms))
     cut = float(rdm.meanDensity + 1.1 * rdm.stdDensity)
+    recorded.inputs(request.node.name, [cut, float(rdm.meanDensity + 2.2 * rdm.stdDensity)], live=True)
     for c in (0.0, cut, -cut):
         want = [rdm.getSphereCrsFromXyz(a, r, c) for a, r in zip(atoms, radii)]
         crs, off = orc.sphere_lists(atoms, radii, c)
