@@ -133,6 +133,19 @@ int pe_sphere_union_warp_cycles(unsigned long long *out5);
 int pe_sphere_sums(const pe_geom *g, const float *d_rho, int32_t n_atoms, const double *d_xyz,
                    const float *d_radius, int32_t n_groups, const int32_t *d_group_start, float cut_pos,
                    float cut_neg, double *d_out, void *d_ws, void *stream);
+/* The per-atom and the grouped sums of the same atoms in one call: the results equal those of
+ *   pe_sphere_sums(g, d_rho, n_atoms, d_xyz, d_atom_radius, n_atoms, NULL, cut_pos, cut_neg, d_out_atoms, d_ws, stream) and
+ *   pe_sphere_sums(g, d_rho, n_atoms, d_xyz, d_group_radius, n_groups, d_group_start, cut_pos, cut_neg, d_out_groups, d_ws, stream),
+ * bit for bit, with the same argument checks and status codes and the same workspace (pe_sphere_workspace_bytes(n_atoms)).
+ * When the cell is orthogonal and every per-atom box at max_atom_radius is at most 8 voxels wide (the atom-type radii of the
+ * cloud pass on a 0.5 A grid), the per-atom sums run as short work items at the end of the grouped kernel: one launch instead
+ * of two, and the per-atom work fills the SMs that the last groups leave idle.  Otherwise the call issues the two launches.
+ * max_atom_radius is the largest value of d_atom_radius (any larger bound also does; the host cannot read the device array
+ * without a synchronisation); an atom whose radius exceeds it gets NaN rows instead of sums. */
+int pe_sphere_sums_atoms_and_groups(const pe_geom *g, const float *d_rho, int32_t n_atoms, const double *d_xyz,
+                                    const float *d_atom_radius, float max_atom_radius, const float *d_group_radius,
+                                    int32_t n_groups, const int32_t *d_group_start, float cut_pos, float cut_neg,
+                                    double *d_out_atoms, double *d_out_groups, void *d_ws, void *stream);
 
 /* getSphereCrsFromXyz (pdb_eda/cutils.pyx:220-248), batched, as lists.  Two calls:
  *   pe_sphere_count: d_count[a] = len(getSphereCrsFromXyz(dm, xyz[a], radius[a], cutoff)), and

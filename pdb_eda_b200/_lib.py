@@ -63,6 +63,7 @@ SIGNATURES = {
     "pe_sphere_union_cycles": (ctypes.c_int, [ctypes.POINTER(ctypes.c_ulonglong)]),
     "pe_sphere_union_warp_cycles": (ctypes.c_int, [ctypes.POINTER(ctypes.c_ulonglong)]),
     "pe_sphere_sums": (ctypes.c_int, [_GEOM, _P, _I32, _P, _P, _I32, _P, _F32, _F32, _P, _P, _P]),
+    "pe_sphere_sums_atoms_and_groups": (ctypes.c_int, [_GEOM, _P, _I32, _P, _P, _F32, _P, _I32, _P, _F32, _F32, _P, _P, _P, _P]),
     "pe_sphere_count": (ctypes.c_int, [_GEOM, _P, _I32, _P, _P, _F32, _P, _P, _P]),
     "pe_sphere_fill": (ctypes.c_int, [_GEOM, _P, _I32, _P, _P, _F32, _P, _I32, _P, _P, _P, _P]),
     "pe_blob_workspace_bytes": (_I64, [_GEOM, _I64]),

@@ -23,7 +23,9 @@
 //   * warp-shuffle / fixed-order block reductions make the float64 sums run-to-run deterministic.
 // Skewed cells take generic passes that evaluate the reference's 3x3 mat-vec per candidate in the host BLAS's
 // accumulation order.
+#include <float.h>
 #include <limits.h>
+#include <math.h>
 #include <stdlib.h>
 #include <stddef.h>
 #include <type_traits>
@@ -34,7 +36,7 @@ namespace pe {
 
 int launch_union_warp(const pe_geom *g, const float *d_rho, int n_groups, const int32_t *d_group_start, const double *d_xyz,
                       const float *d_radius, int32_t *box, double *thr, float cut_pos, float cut_neg, int *d_counter, double *d_out,
-                      cudaStream_t st);  // pe_union.cu
+                      int n_quad_atoms, const float *d_atom_radius, double *d_out_atoms, cudaStream_t st);  // pe_union.cu
 
 // ------------------------------------------------------------------------------------------------ sums kernel
 // CASEB: the column axis carries z (the last term of the reference's sum), so fl(X2 + Y2) depends on (row, section).
@@ -138,19 +140,9 @@ __device__ __forceinline__ void sums_one_atom(const pe_geom &g, const float *__r
     __syncwarp();  // the tables are refilled for the warp's next atom
 }
 
-// Per-atom sums.  A warp takes kAtomsPerWarp = 4 consecutive atoms.  At the atom-type radii of the cloud pass
-// (0.6 - 1.3 A on a 0.5 A grid) a box is 4^3 or 6^3 candidates for ~15 in-sphere voxels, so when all four boxes are at
-// most 8 wide (orthogonal cell) each atom gets 8 lanes: a lane walks box rows (row, section), finds the row's in-sphere
-// columns exactly (row_chord) and gathers just those -- a fraction of the instructions of one warp per atom (49.7 -> 29.1 us on C2's
-// cloud pass, see DESIGN.md).  Otherwise the warp handles its atoms one after the other with all 32 lanes
-// (sums_one_atom).
-constexpr int kSmallDim = 8;
-constexpr int kAtomsPerWarp = 4;
-struct SmallTab {
-    double sq[3][kSmallDim];  // per crs axis: fl((coord - atom)^2) of the box's indices
-    int off[3][kSmallDim];    // wrapped element offsets, or kInvalidOff
-};
-
+// Per-atom sums.  A warp takes kAtomsPerWarp = 4 consecutive atoms: 8 lanes per atom (quad_sums, pe_sphere_dev.cuh) when all four
+// boxes are at most kSmallDim wide in an orthogonal cell; otherwise the warp handles its atoms one after the other with all
+// 32 lanes (sums_one_atom).
 template <int MODE>
 __global__ void __launch_bounds__(kSphereWarps * 32)
     sphere_sums_kernel(const __grid_constant__ pe_geom g, const float *__restrict__ rho, int n_atoms,
@@ -163,115 +155,9 @@ __global__ void __launch_bounds__(kSphereWarps * 32)
     if (a0 >= n_atoms) return;
     cp = eff_pos(cp);
     cn = eff_neg(cn);
-    const int sub = lane >> 3, l8 = lane & 7;
-    const int a = a0 + sub;
-    const bool live = a < n_atoms;
-    // box and distance threshold of this lane's atom (the 8 lanes of an atom compute the same values: SIMT makes that free,
-    // and a separate one-thread-per-atom launch in front of this kernel cost 9 us for C2's 40,000 atoms)
-    int lo[3] = {0, 0, 0}, dim[3] = {0, 0, 0};
-    double ax = 0.0, ay = 0.0, az = 0.0, T = -1.0;
-    if (live) {
-        ax = xyz[3 * a];
-        ay = xyz[3 * a + 1];
-        az = xyz[3 * a + 2];
-        AtomBox bb;
-        atom_box(g, ax, ay, az, radius[a], bb, T);
-#pragma unroll
-        for (int k = 0; k < 3; ++k) {
-            lo[k] = bb.lo[k];
-            dim[k] = bb.dim[k];
-        }
-    }
-    const bool small = g.orthogonal && dim[0] <= kSmallDim && dim[1] <= kSmallDim && dim[2] <= kSmallDim;
-    if (!__all_sync(kFull, small)) {
-        for (int q = 0; q < kAtomsPerWarp && a0 + q < n_atoms; ++q)
-            sums_one_atom<MODE>(g, rho, a0 + q, xyz, radius, cp, cn, tabs[warp], lane, out);
-        return;
-    }
-    SphereAcc acc;
-    if (live && dim[0] > 0 && dim[1] > 0 && dim[2] > 0) {
-        SmallTab &t = stab[warp][sub];
-#pragma unroll
-        for (int axis = 0; axis < 3; ++axis) {
-            if (l8 < dim[axis]) {
-                t.sq[axis][l8] = axis_sq(g, axis, lo[axis] + l8, ax, ay, az);
-                t.off[axis][l8] = axis_off(g, axis, lo[axis] + l8);
-            }
-        }
-        __syncwarp(0xffu << (8 * sub));  // the 8 lanes of this atom (they take this branch together)
-        const int ic = g.map2crs[0];  // xyz axis carried by the columns
-        const float inv_gl = (float)(1.0 / g.grid_length[ic]);
-        // the atom's fractional column inside the box: formed in float64 and rounded once, so that the guess stays within
-        // 1e-5 columns of the real chord ends whatever the size of the map (row_chord's proof needs that)
-        const float xc = (float)((sel3(ax, ay, az, ic) - g.origin[ic]) / g.grid_length[ic] - (double)lo[0]);
-        const int nC = dim[0];
-        const double *sqc = t.sq[0];
-        // the column nearest the atom: the box's centre column or, after rounding, one of its neighbours
-        int km = min(max(nC / 2, 0), nC - 1);
-        if (km > 0 && sqc[km - 1] < sqc[km]) --km;
-        else if (km + 1 < nC && sqc[km + 1] < sqc[km]) ++km;
-        const int rows = dim[1] * dim[2];
-        const unsigned div_d1 = (1024u + (unsigned)dim[1] - 1u) / (unsigned)dim[1];  // exact for row < 64, dim[1] <= 8
-        static_assert(kSmallDim * kSmallDim * kSmallDim <= 1024, "magic division by dim[1]");
-        for (int row = l8; row < rows; row += 8) {
-            const int is = (int)(((unsigned)row * div_d1) >> 10), ir = row - is * dim[1];  // row / dim[1]
-            const double sr = t.sq[1][ir], ss = t.sq[2][is];
-            const double A = (MODE == 0) ? ss : ((MODE == 1) ? sr : __dadd_rn(sr, ss));
-            const double B = (MODE == 0) ? sr : ss;
-            int kl, kh;
-            if (!row_chord<MODE>(sqc, nC, km, xc, inv_gl, A, B, T, kl, kh)) continue;
-            const int o1 = t.off[1][ir], o2 = t.off[2][is];
-            const int orr = o1 | o2;
-            const unsigned osum = (unsigned)o1 + (unsigned)o2;
-            // all loads of the chord first (a chord has at most kSmallDim columns), then the sums.  (Walking the rows of
-            // the four atoms in lock step, reconverged every iteration, is slower -- 31.2 against 29.1 us: left to
-            // themselves the four groups drift apart and hide each other's latency.)
-            float v[kSmallDim];
-#pragma unroll
-            for (int j = 0; j < kSmallDim; ++j) {
-                const int k = kl + j;
-                v[j] = 0.f;
-                if (k <= kh) {
-                    const int oc = t.off[0][k];
-                    const bool ok = (orr | oc) >= 0;
-                    if (ok) v[j] = __ldg(rho + (int)(osum + (unsigned)oc));
-                    acc.bad |= ok ? 0 : 1;
-                }
-            }
-            const bool has_neg = cn > __int_as_float(0xff800000);  // warp-uniform: the negative class is in use
-#pragma unroll
-            for (int j = 0; j < kSmallDim; ++j) {
-                if (kl + j > kh) break;  // chords are ~3 columns long: the sums are not worth issuing for empty slots
-                if (has_neg)
-                    acc.add(true, v[j], cp, cn);
-                else
-                    acc.add_pos(true, v[j], cp);
-            }
-        }
-    }
-    __syncwarp();
-    // sums over the 8 lanes of an atom
-#pragma unroll
-    for (int o = 4; o > 0; o >>= 1) {
-        acc.n_all += __shfl_xor_sync(kFull, acc.n_all, o);
-        acc.n_pos += __shfl_xor_sync(kFull, acc.n_pos, o);
-        acc.n_neg += __shfl_xor_sync(kFull, acc.n_neg, o);
-        acc.bad += __shfl_xor_sync(kFull, acc.bad, o);
-        acc.s_all += __shfl_xor_sync(kFull, acc.s_all, o);
-        acc.s_pos += __shfl_xor_sync(kFull, acc.s_pos, o);
-        acc.s_neg += __shfl_xor_sync(kFull, acc.s_neg, o);
-    }
-    if (live && l8 == 0) {
-        double *o = out + (int64_t)a * PE_SPHERE_NOUT;
-        o[0] = (double)acc.n_all;
-        o[1] = acc.s_all;
-        o[2] = (double)acc.n_pos;
-        o[3] = acc.s_pos;
-        o[4] = (double)acc.n_neg;
-        o[5] = acc.s_neg;
-        o[6] = acc.bad ? 0.0 : 1.0;
-        o[7] = (double)dim[0] * (double)dim[1] * (double)dim[2];
-    }
+    if (quad_sums<MODE>(g, rho, n_atoms, a0, xyz, radius, cp, cn, stab[warp], lane, out)) return;
+    for (int q = 0; q < kAtomsPerWarp && a0 + q < n_atoms; ++q)
+        sums_one_atom<MODE>(g, rho, a0 + q, xyz, radius, cp, cn, tabs[warp], lane, out);
 }
 
 // ------------------------------------------------------------------------------------------------ union kernel
@@ -841,6 +727,25 @@ __global__ void sphere_fill_kernel(const __grid_constant__ pe_geom g, const floa
 
 using namespace pe;
 
+// Round 1's CTA-per-group kernel instead of the warp-per-group one, kept for A/B measurements.
+static bool use_union_cta_kernel() {
+    static const bool on = getenv("PE_UNION_CTA") != nullptr;
+    return on;
+}
+
+// Whether every box of an atom whose radius is at most max_radius is at most kSmallDim wide, decided as atom_box decides a
+// box: dim = 2 * R + 2 along each crs axis, with R from xyz2crs(origin + r) -- in an orthogonal cell
+// rint(fl(fl(origin + r) - origin) / grid_length), which only grows with r.
+static bool boxes_are_small(const pe_geom *g, float max_radius) {
+    if (!g->orthogonal || !(max_radius <= FLT_MAX)) return false;  // skewed cell, NaN or infinite bound
+    const double r = (double)max_radius;
+    double R[3];
+    for (int i = 0; i < 3; ++i) R[i] = nearbyint(((g->origin[i] + r) - g->origin[i]) / g->grid_length[i]);
+    for (int k = 0; k < 3; ++k)
+        if (2.0 * R[g->map2crs[k]] + 2.0 > (double)kSmallDim) return false;
+    return true;
+}
+
 extern "C" {
 
 int pe_sphere_union_cycles(unsigned long long *out4) {
@@ -887,10 +792,10 @@ int pe_sphere_sums(const pe_geom *g, const float *d_rho, int32_t n_atoms, const 
         PE_LAUNCH_CHECK();
         return PE_OK;
     }
-    static const bool use_cta_kernel = getenv("PE_UNION_CTA") != nullptr;  // round 1's kernel, kept for A/B measurements
-    if (n_groups > 0 && !use_cta_kernel) {
+    if (n_groups > 0 && !use_union_cta_kernel()) {
         int *counter = (int *)ws;  // third region of the workspace
-        return launch_union_warp(g, d_rho, n_groups, d_group_start, d_xyz, d_radius, box, thr, cut_pos, cut_neg, counter, d_out, st);
+        return launch_union_warp(g, d_rho, n_groups, d_group_start, d_xyz, d_radius, box, thr, cut_pos, cut_neg, counter, d_out, 0,
+                                 nullptr, nullptr, st);
     }
     if (n_groups > 0) {
         const int mode = g->map2xyz[2] == 1 ? 0 : (g->map2xyz[2] == 2 ? 1 : 2);  // crs axis that carries z
@@ -909,6 +814,32 @@ int pe_sphere_sums(const pe_geom *g, const float *d_rho, int32_t n_atoms, const 
     }
     PE_LAUNCH_CHECK();
     return PE_OK;
+}
+
+int pe_sphere_sums_atoms_and_groups(const pe_geom *g, const float *d_rho, int32_t n_atoms, const double *d_xyz,
+                                    const float *d_atom_radius, float max_atom_radius, const float *d_group_radius, int32_t n_groups,
+                                    const int32_t *d_group_start, float cut_pos, float cut_neg, double *d_out_atoms,
+                                    double *d_out_groups, void *d_ws, void *stream) {
+    if (int rc = check_geom(g)) return rc;
+    PE_CHECK_ARG(n_atoms >= 0 && n_groups >= 0, "pe_sphere_sums_atoms_and_groups: negative size");
+    if (n_atoms == 0 && n_groups == 0) return PE_OK;
+    PE_CHECK_ARG(d_rho && d_xyz && d_atom_radius && d_group_radius && d_out_atoms && d_out_groups && d_ws,
+                 "pe_sphere_sums_atoms_and_groups: null pointer");
+    PE_CHECK_ARG(d_group_start || n_groups == n_atoms,
+                 "pe_sphere_sums_atoms_and_groups: n_groups must equal n_atoms without group offsets");
+    PE_CHECK_ARG(!(cut_pos < 0.f) && !(cut_neg > 0.f), "pe_sphere_sums_atoms_and_groups: cut_pos must be >= 0 and cut_neg <= 0");
+    if (n_atoms > 0 && n_groups > 0 && d_group_start && !use_union_cta_kernel() && boxes_are_small(g, max_atom_radius)) {
+        char *ws = (char *)d_ws;
+        int32_t *box = (int32_t *)ws;
+        ws += align_up((int64_t)n_atoms * 6 * 4, 256);
+        double *thr = (double *)ws;
+        ws += align_up((int64_t)n_atoms * 8, 256);
+        return launch_union_warp(g, d_rho, n_groups, d_group_start, d_xyz, d_group_radius, box, thr, cut_pos, cut_neg, (int *)ws,
+                                 d_out_groups, n_atoms, d_atom_radius, d_out_atoms, (cudaStream_t)stream);
+    }
+    if (int rc = pe_sphere_sums(g, d_rho, n_atoms, d_xyz, d_atom_radius, n_atoms, nullptr, cut_pos, cut_neg, d_out_atoms, d_ws, stream))
+        return rc;
+    return pe_sphere_sums(g, d_rho, n_atoms, d_xyz, d_group_radius, n_groups, d_group_start, cut_pos, cut_neg, d_out_groups, d_ws, stream);
 }
 
 int pe_sphere_count(const pe_geom *g, const float *d_rho, int32_t n_atoms, const double *d_xyz, const float *d_radius,

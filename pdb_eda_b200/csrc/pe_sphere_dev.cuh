@@ -264,4 +264,133 @@ __device__ __forceinline__ bool row_chord(const double *sqc, int nC, int km, flo
     return true;
 }
 
+// ------------------------------------------------------------------------------------------------ per-atom sums, 4 atoms per warp
+// At the atom-type radii of the cloud pass (0.6 - 1.3 A on a 0.5 A grid) a box is 4^3 or 6^3 candidates for ~15 in-sphere
+// voxels, so when all four boxes of a warp's quad are at most kSmallDim wide (orthogonal cell) each atom gets 8 lanes: a lane
+// walks box rows (row, section), finds the row's in-sphere columns exactly (row_chord) and gathers just those -- a fraction of
+// the instructions of one warp per atom (49.7 -> 29.1 us on C2's cloud pass, see DESIGN.md).  One copy of this code serves
+// sphere_sums_kernel (pe_sphere.cu) and the atom items of sphere_union_warp_kernel (pe_union.cu), so a per-atom result does
+// not depend on which kernel computed it.
+constexpr int kSmallDim = 8;
+constexpr int kAtomsPerWarp = 4;
+struct SmallTab {
+    double sq[3][kSmallDim];  // per crs axis: fl((coord - atom)^2) of the box's indices
+    int off[3][kSmallDim];    // wrapped element offsets, or kInvalidOff
+};
+
+// Sums of the atoms [a0, a0 + 4) (those below n_atoms) into out (PE_SPHERE_NOUT per atom).  cp / cn are the effective cutoffs
+// (eff_pos / eff_neg).  Returns false, warp-uniformly and with nothing written, unless the cell is orthogonal and every box of
+// the quad is at most kSmallDim wide.  Called by a whole warp; tab: kAtomsPerWarp tables of the warp's own.
+template <int MODE>
+__device__ __forceinline__ bool quad_sums(const pe_geom &g, const float *__restrict__ rho, int n_atoms, int a0,
+                                          const double *__restrict__ xyz, const float *__restrict__ radius, float cp, float cn,
+                                          SmallTab *tab, int lane, double *__restrict__ out) {
+    const int sub = lane >> 3, l8 = lane & 7;
+    const int a = a0 + sub;
+    const bool live = a < n_atoms;
+    // box and distance threshold of this lane's atom (the 8 lanes of an atom compute the same values: SIMT makes that free,
+    // and a separate one-thread-per-atom launch in front of this kernel cost 9 us for C2's 40,000 atoms)
+    int lo[3] = {0, 0, 0}, dim[3] = {0, 0, 0};
+    double ax = 0.0, ay = 0.0, az = 0.0, T = -1.0;
+    if (live) {
+        ax = xyz[3 * a];
+        ay = xyz[3 * a + 1];
+        az = xyz[3 * a + 2];
+        AtomBox bb;
+        atom_box(g, ax, ay, az, radius[a], bb, T);
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            lo[k] = bb.lo[k];
+            dim[k] = bb.dim[k];
+        }
+    }
+    const bool small = g.orthogonal && dim[0] <= kSmallDim && dim[1] <= kSmallDim && dim[2] <= kSmallDim;
+    if (!__all_sync(kFull, small)) return false;
+    SphereAcc acc;
+    if (live && dim[0] > 0 && dim[1] > 0 && dim[2] > 0) {
+        SmallTab &t = tab[sub];
+#pragma unroll
+        for (int axis = 0; axis < 3; ++axis) {
+            if (l8 < dim[axis]) {
+                t.sq[axis][l8] = axis_sq(g, axis, lo[axis] + l8, ax, ay, az);
+                t.off[axis][l8] = axis_off(g, axis, lo[axis] + l8);
+            }
+        }
+        __syncwarp(0xffu << (8 * sub));  // the 8 lanes of this atom (they take this branch together)
+        const int ic = g.map2crs[0];  // xyz axis carried by the columns
+        const float inv_gl = (float)(1.0 / g.grid_length[ic]);
+        // the atom's fractional column inside the box: formed in float64 and rounded once, so that the guess stays within
+        // 1e-5 columns of the real chord ends whatever the size of the map (row_chord's proof needs that)
+        const float xc = (float)((sel3(ax, ay, az, ic) - g.origin[ic]) / g.grid_length[ic] - (double)lo[0]);
+        const int nC = dim[0];
+        const double *sqc = t.sq[0];
+        // the column nearest the atom: the box's centre column or, after rounding, one of its neighbours
+        int km = min(max(nC / 2, 0), nC - 1);
+        if (km > 0 && sqc[km - 1] < sqc[km]) --km;
+        else if (km + 1 < nC && sqc[km + 1] < sqc[km]) ++km;
+        const int rows = dim[1] * dim[2];
+        const unsigned div_d1 = (1024u + (unsigned)dim[1] - 1u) / (unsigned)dim[1];  // exact for row < 64, dim[1] <= 8
+        static_assert(kSmallDim * kSmallDim * kSmallDim <= 1024, "magic division by dim[1]");
+        for (int row = l8; row < rows; row += 8) {
+            const int is = (int)(((unsigned)row * div_d1) >> 10), ir = row - is * dim[1];  // row / dim[1]
+            const double sr = t.sq[1][ir], ss = t.sq[2][is];
+            const double A = (MODE == 0) ? ss : ((MODE == 1) ? sr : __dadd_rn(sr, ss));
+            const double B = (MODE == 0) ? sr : ss;
+            int kl, kh;
+            if (!row_chord<MODE>(sqc, nC, km, xc, inv_gl, A, B, T, kl, kh)) continue;
+            const int o1 = t.off[1][ir], o2 = t.off[2][is];
+            const int orr = o1 | o2;
+            const unsigned osum = (unsigned)o1 + (unsigned)o2;
+            // all loads of the chord first (a chord has at most kSmallDim columns), then the sums.  (Walking the rows of
+            // the four atoms in lock step, reconverged every iteration, is slower -- 31.2 against 29.1 us: left to
+            // themselves the four groups drift apart and hide each other's latency.)
+            float v[kSmallDim];
+#pragma unroll
+            for (int j = 0; j < kSmallDim; ++j) {
+                const int k = kl + j;
+                v[j] = 0.f;
+                if (k <= kh) {
+                    const int oc = t.off[0][k];
+                    const bool ok = (orr | oc) >= 0;
+                    if (ok) v[j] = __ldg(rho + (int)(osum + (unsigned)oc));
+                    acc.bad |= ok ? 0 : 1;
+                }
+            }
+            const bool has_neg = cn > __int_as_float(0xff800000);  // warp-uniform: the negative class is in use
+#pragma unroll
+            for (int j = 0; j < kSmallDim; ++j) {
+                if (kl + j > kh) break;  // chords are ~3 columns long: the sums are not worth issuing for empty slots
+                if (has_neg)
+                    acc.add(true, v[j], cp, cn);
+                else
+                    acc.add_pos(true, v[j], cp);
+            }
+        }
+    }
+    __syncwarp();  // the tables are free for the warp's next use
+    // sums over the 8 lanes of an atom
+#pragma unroll
+    for (int o = 4; o > 0; o >>= 1) {
+        acc.n_all += __shfl_xor_sync(kFull, acc.n_all, o);
+        acc.n_pos += __shfl_xor_sync(kFull, acc.n_pos, o);
+        acc.n_neg += __shfl_xor_sync(kFull, acc.n_neg, o);
+        acc.bad += __shfl_xor_sync(kFull, acc.bad, o);
+        acc.s_all += __shfl_xor_sync(kFull, acc.s_all, o);
+        acc.s_pos += __shfl_xor_sync(kFull, acc.s_pos, o);
+        acc.s_neg += __shfl_xor_sync(kFull, acc.s_neg, o);
+    }
+    if (live && l8 == 0) {
+        double *o = out + (int64_t)a * PE_SPHERE_NOUT;
+        o[0] = (double)acc.n_all;
+        o[1] = acc.s_all;
+        o[2] = (double)acc.n_pos;
+        o[3] = acc.s_pos;
+        o[4] = (double)acc.n_neg;
+        o[5] = acc.s_neg;
+        o[6] = acc.bad ? 0.0 : 1.0;
+        o[7] = (double)dim[0] * (double)dim[1] * (double)dim[2];
+    }
+    return true;
+}
+
 }  // namespace pe

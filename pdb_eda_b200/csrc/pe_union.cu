@@ -20,6 +20,7 @@
 // Exactness, summation order (fixed) and outputs are those of the round-1 kernel; skewed cells and groups whose tile would
 // need more than 32 columns per bitmap word are handled by splitting the bounding box into more tiles (columns included).
 #include <limits.h>
+#include <stddef.h>
 #include "pe_sphere_dev.cuh"
 
 #ifndef PE_UNION_SWEEP
@@ -61,9 +62,15 @@ constexpr int kULoads = PE_UNION_LOADS;  // loads in flight per lane (4: 165 us,
 struct WarpUnion {
     uint32_t bits[kUT * kUT];     // [row][section]
     int list[kUList];
-    double sqC[kUT], sqR[kUT], sqS[kUT];
+    double sqC[kUT], sqR[kUT], sqS[kUT];  // an atom item keeps its quad's SmallTabs here (quad_tabs)
     int offC[kUT], offR[kUT], offS[kUT];
 };
+// At 7 CTAs per SM the shared memory has no room for more: an atom item's tables take the place of a residue item's per-atom
+// tables and tile offsets, which are dead between two items.
+static_assert(offsetof(WarpUnion, offS) + sizeof(WarpUnion::offS) - offsetof(WarpUnion, sqC) == kAtomsPerWarp * sizeof(SmallTab),
+              "the quad's tables fill the residue tables' bytes exactly");
+static_assert(offsetof(WarpUnion, sqC) % alignof(SmallTab) == 0, "SmallTab alignment");
+__device__ __forceinline__ SmallTab *quad_tabs(WarpUnion &w) { return reinterpret_cast<SmallTab *>(w.sqC); }
 
 // Membership of one atom in the warp's tile, exactly, without square roots: a lane takes one box row of the atom and one
 // direction along the section axis, starting at the section nearest the atom (isc) and walking away from it.  Along that walk
@@ -252,12 +259,17 @@ __device__ __forceinline__ int warp_max(int v) {
     return v;
 }
 
+// Work items, handed out in order through one counter: [0, n_groups) are groups (the long items), then, when n_quad_atoms > 0,
+// one item per quad of atoms [4q, 4q + 4) summed at atom_radius into out_atoms (quad_sums: the short items fill the SMs that
+// the last groups would leave idle).  The host hands atoms over only when every box at atom_radius is at most kSmallDim wide;
+// a quad that is not writes NaN rows, so that a wrong decision cannot pass for a result.
 template <int MODE>
 __global__ void __launch_bounds__(kUW * 32, kUCtas)
     sphere_union_warp_kernel(const __grid_constant__ pe_geom g, const float *__restrict__ rho, int n_groups,
                              const int32_t *__restrict__ group_start, const double *__restrict__ xyz, const float *__restrict__ radius,
                              int32_t *box, double *thr, float cp, float cn, int *__restrict__ counter,
-                             double *__restrict__ out /* n_groups x PE_SPHERE_NOUT */) {
+                             double *__restrict__ out /* n_groups x PE_SPHERE_NOUT */, int n_quad_atoms,
+                             const float *__restrict__ atom_radius, double *__restrict__ out_atoms /* n_quad_atoms x PE_SPHERE_NOUT */) {
     __shared__ WarpUnion wsh[kUW];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     WarpUnion &w = wsh[warp];
@@ -272,11 +284,20 @@ __global__ void __launch_bounds__(kUW * 32, kUCtas)
     long long t_mark = clock64();
     long long t_phase[5] = {0, 0, 0, 0, 0};
 #endif
+    const int n_items = n_groups + (n_quad_atoms + kAtomsPerWarp - 1) / kAtomsPerWarp;
     for (;;) {
-        int grp = 0;
-        if (lane == 0) grp = atomicAdd(counter, 1);
-        grp = __shfl_sync(kFull, grp, 0);
-        if (grp >= n_groups) break;
+        int item = 0;
+        if (lane == 0) item = atomicAdd(counter, 1);
+        item = __shfl_sync(kFull, item, 0);
+        if (item >= n_items) break;
+        if (item >= n_groups) {
+            const int a0 = (item - n_groups) * kAtomsPerWarp;
+            if (!quad_sums<MODE>(g, rho, n_quad_atoms, a0, xyz, atom_radius, cp, cn, quad_tabs(w), lane, out_atoms) &&
+                lane < min(kAtomsPerWarp, n_quad_atoms - a0) * PE_SPHERE_NOUT)
+                out_atoms[(int64_t)a0 * PE_SPHERE_NOUT + lane] = __longlong_as_double(0x7ff8000000000000ll);
+            continue;
+        }
+        const int grp = item;
         const int a0 = group_start[grp], a1 = group_start[grp + 1];
         // boxes and thresholds of the group's atoms (lanes over atoms), bounding box by warp reductions
         int ulo0 = INT_MAX, ulo1 = INT_MAX, ulo2 = INT_MAX, uhi0 = INT_MIN, uhi1 = INT_MIN, uhi2 = INT_MIN;
@@ -416,22 +437,25 @@ __global__ void __launch_bounds__(kUW * 32, kUCtas)
 
 int launch_union_warp(const pe_geom *g, const float *d_rho, int n_groups, const int32_t *d_group_start, const double *d_xyz,
                       const float *d_radius, int32_t *box, double *thr, float cut_pos, float cut_neg, int *d_counter, double *d_out,
-                      cudaStream_t st) {
+                      int n_quad_atoms, const float *d_atom_radius, double *d_out_atoms, cudaStream_t st) {
     const int mode = g->map2xyz[2] == 1 ? 0 : (g->map2xyz[2] == 2 ? 1 : 2);  // crs axis that carries z
     PE_CUDA(cudaMemsetAsync(d_counter, 0, sizeof(int), st));
-    const int warps_needed = n_groups;
+    const int warps_needed = n_groups + (n_quad_atoms + kAtomsPerWarp - 1) / kAtomsPerWarp;
     int grid = (warps_needed + kUW - 1) / kUW;
     const int max_grid = sm_count() * kUCtas;
     if (grid > max_grid) grid = max_grid;
     if (mode == 0)
         PE_LAUNCH("sphere_union_kernel", st, sphere_union_warp_kernel<0><<<grid, kUW * 32, 0, st>>>(
-            *g, d_rho, n_groups, d_group_start, d_xyz, d_radius, box, thr, cut_pos, cut_neg, d_counter, d_out));
+            *g, d_rho, n_groups, d_group_start, d_xyz, d_radius, box, thr, cut_pos, cut_neg, d_counter, d_out,
+            n_quad_atoms, d_atom_radius, d_out_atoms));
     else if (mode == 1)
         PE_LAUNCH("sphere_union_kernel", st, sphere_union_warp_kernel<1><<<grid, kUW * 32, 0, st>>>(
-            *g, d_rho, n_groups, d_group_start, d_xyz, d_radius, box, thr, cut_pos, cut_neg, d_counter, d_out));
+            *g, d_rho, n_groups, d_group_start, d_xyz, d_radius, box, thr, cut_pos, cut_neg, d_counter, d_out,
+            n_quad_atoms, d_atom_radius, d_out_atoms));
     else
         PE_LAUNCH("sphere_union_kernel", st, sphere_union_warp_kernel<2><<<grid, kUW * 32, 0, st>>>(
-            *g, d_rho, n_groups, d_group_start, d_xyz, d_radius, box, thr, cut_pos, cut_neg, d_counter, d_out));
+            *g, d_rho, n_groups, d_group_start, d_xyz, d_radius, box, thr, cut_pos, cut_neg, d_counter, d_out,
+            n_quad_atoms, d_atom_radius, d_out_atoms));
     PE_LAUNCH_CHECK();
     return PE_OK;
 }
