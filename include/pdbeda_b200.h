@@ -123,12 +123,9 @@ int pe_crs2xyz(const pe_geom *g, int64_t n, const int32_t *d_crs, double *d_xyz,
  * d_ws: >= pe_sphere_workspace_bytes(n_atoms) bytes. */
 #define PE_SPHERE_NOUT 8
 int64_t pe_sphere_workspace_bytes(int64_t n_atoms);
-/* Diagnostic: SM cycles of the grouped (union) kernel by phase -- prologue, membership, gather, epilogue -- summed
- * over all CTAs since the last call; synchronises and resets.  All zeros unless the library was built with
- * -DPE_UNION_PHASE_CYCLES=1 (the counters cost the kernel registers). */
-int pe_sphere_union_cycles(unsigned long long *out4);
-/* The same for the warp-per-group kernel (the default): boxes + bounding box, tile offsets + per-atom tables, membership,
- * gather, reduction + output; zeros unless built with -DPE_UNION_PHASE_CYCLES=1. */
+/* Diagnostic: warp cycles of the grouped (union) kernel by phase -- boxes + bounding box, tile offsets + per-atom tables,
+ * membership, gather, reduction + output -- summed over all warps since the last call; synchronises and resets.  All zeros
+ * unless the library was built with -DPE_UNION_PHASE_CYCLES=1 (the counters cost the kernel registers). */
 int pe_sphere_union_warp_cycles(unsigned long long *out5);
 int pe_sphere_sums(const pe_geom *g, const float *d_rho, int32_t n_atoms, const double *d_xyz,
                    const float *d_radius, int32_t n_groups, const int32_t *d_group_start, float cut_pos,

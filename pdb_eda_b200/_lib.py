@@ -60,7 +60,6 @@ SIGNATURES = {
     "pe_xyz2crs": (ctypes.c_int, [_GEOM, _I64, _P, _P, _P]),
     "pe_crs2xyz": (ctypes.c_int, [_GEOM, _I64, _P, _P, _P]),
     "pe_sphere_workspace_bytes": (_I64, [_I64]),
-    "pe_sphere_union_cycles": (ctypes.c_int, [ctypes.POINTER(ctypes.c_ulonglong)]),
     "pe_sphere_union_warp_cycles": (ctypes.c_int, [ctypes.POINTER(ctypes.c_ulonglong)]),
     "pe_sphere_sums": (ctypes.c_int, [_GEOM, _P, _I32, _P, _P, _I32, _P, _F32, _F32, _P, _P, _P]),
     "pe_sphere_sums_atoms_and_groups": (ctypes.c_int, [_GEOM, _P, _I32, _P, _P, _F32, _P, _I32, _P, _F32, _F32, _P, _P, _P, _P]),

@@ -190,6 +190,8 @@ struct SphereAcc {
 
 // ------------------------------------------------------------------------------------------------ exact chords
 // MODE 0: z is carried by the row axis, 1: by the section axis, 2: by the column axis.
+inline int z_axis_mode(const pe_geom *g) { return g->map2xyz[2] == 1 ? 0 : (g->map2xyz[2] == 2 ? 1 : 2); }
+
 // Squared distance of column k of a box row exactly as the reference adds it: fl(fl(X2 + Y2) + Z2).
 template <int MODE>
 __device__ __forceinline__ bool row_pred(const double *sqc, int k, double A, double B, double T) {
@@ -244,7 +246,7 @@ __device__ __forceinline__ bool row_chord(const double *sqc, int nC, int km, flo
     if (!row_pred<MODE>(sqc, km, A, B, T)) return false;  // the row misses the sphere
     int lo = 0, hi = km;  // smallest k in [0, km] inside
     while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
+        const int mid = (int)((unsigned)(lo + hi) >> 1);  // lo + hi >= 0, which the compiler does not always prove
         if (row_pred<MODE>(sqc, mid, A, B, T))
             hi = mid;
         else

@@ -3,12 +3,9 @@
 // Replaces getSphereCrsFromXyzList (pdb_eda/cutils.pyx:250-271) + the sums of calculateRegionDensity / calculateRegionDiscrepancy
 // (pdb_eda/densityAnalysis.py:1037-1068, :1160-1211) for every residue (group) of a structure at once.
 //
-// Round 1's kernel (sphere_union_kernel, pe_sphere.cu) gave a group to a CTA of four warps and separated table building,
-// membership and gather by block barriers; its phase split on C2 was 16 % prologue, 37 % membership, 41 % gather, 7 %
-// epilogue (profiles/r02_union_phases.md) with the warps of a block waiting on each other at every barrier.  Here a warp owns
-// a group from start to finish -- boxes, bounding box, per-atom tables, membership bitmap, compaction, gather, reduction all
-// stay inside the warp (shuffles and __syncwarp only), groups are handed out through one atomic counter, and the four warps
-// of a CTA only share the SM:
+// A warp owns a group from start to finish -- boxes, bounding box, per-atom tables, membership bitmap, compaction, gather,
+// reduction all stay inside the warp (shuffles and __syncwarp only, no block barriers), groups are handed out through one
+// atomic counter, and the four warps of a CTA only share the SM:
 //   * tile = 32 columns x 32 rows x 32 sections of the group's bounding box (a residue at the default 3.5 A radius on a 0.5 A
 //     grid is one tile), one 32-bit bitmap word per (row, section): 4 KB per warp;
 //   * atoms are taken one after the other: the warp tabulates the atom's squares along the three axes (one entry per lane),
@@ -17,15 +14,13 @@
 //   * gather: the bitmap rows are taken 32 at a time (one per lane); a row's bits are almost always ONE run, which is written
 //     to the warp's list of map offsets with a counted loop (runs with holes fall back to bit scanning); the list is then
 //     walked densely with 8 independent loads in flight per lane, each voxel of the union read exactly once.
-// Exactness, summation order (fixed) and outputs are those of the round-1 kernel; skewed cells and groups whose tile would
-// need more than 32 columns per bitmap word are handled by splitting the bounding box into more tiles (columns included).
+// The float64 summation order is fixed, so results are run-to-run deterministic.  Skewed cells test every candidate voxel of a
+// box with the reference's distance instead of tabulated squares; a bounding box larger than one tile is split into more tiles
+// (columns included).
 #include <limits.h>
 #include <stddef.h>
 #include "pe_sphere_dev.cuh"
 
-#ifndef PE_UNION_SWEEP
-#define PE_UNION_SWEEP 0
-#endif
 #ifndef PE_UNION_PHASE_CYCLES
 #define PE_UNION_PHASE_CYCLES 0
 #endif
@@ -33,7 +28,7 @@
 namespace pe {
 
 // Diagnostic (compiled in with -DPE_UNION_PHASE_CYCLES=1 only): warp cycles by phase, summed over all warps since the last
-// read through pe_sphere_union_cycles(): 0 boxes + bounding box, 1 tile offsets + per-atom tables, 2 membership, 3 gather,
+// read through pe_sphere_union_warp_cycles(): 0 boxes + bounding box, 1 tile offsets + per-atom tables, 2 membership, 3 gather,
 // 4 reduction + output.
 __device__ unsigned long long g_union_warp_cycles[5];
 #if PE_UNION_PHASE_CYCLES
@@ -47,17 +42,11 @@ __device__ unsigned long long g_union_warp_cycles[5];
 #define PHASE_MARK(k) do { } while (0)
 #endif
 
-constexpr int kUW = 4;            // warps per CTA
-constexpr int kUT = 32;           // tile edge
-#ifndef PE_UNION_CTAS
-#define PE_UNION_CTAS 7
-#endif
-constexpr int kUCtas = PE_UNION_CTAS;                                   // resident CTAs per SM the kernel is shaped for
-constexpr int kUList = kUCtas >= 9 ? 256 : (kUCtas >= 8 ? 448 : 704);    // list entries per warp
-#ifndef PE_UNION_LOADS
-#define PE_UNION_LOADS 8
-#endif
-constexpr int kULoads = PE_UNION_LOADS;  // loads in flight per lane (4: 165 us, 8: 144 us, 12 / 16: 149-153 us on C2's region pass)
+constexpr int kUW = 4;        // warps per CTA
+constexpr int kUT = 32;       // tile edge
+constexpr int kUCtas = 7;     // resident CTAs per SM (6 / 7 / 8 / 9: 165 / 144 / 146-148 / 174 us; spills at 64 registers)
+constexpr int kUList = 704;   // list entries per warp: what 7 CTAs per SM leave (448 at 8, 256 at 9)
+constexpr int kULoads = 8;    // loads in flight per lane (4: 165 us, 8: 144 us, 12 / 16: 149-153 us on C2's region pass)
 
 struct WarpUnion {
     uint32_t bits[kUT * kUT];     // [row][section]
@@ -65,6 +54,8 @@ struct WarpUnion {
     double sqC[kUT], sqR[kUT], sqS[kUT];  // an atom item keeps its quad's SmallTabs here (quad_tabs)
     int offC[kUT], offR[kUT], offS[kUT];
 };
+// 228 KB of shared memory per SM, of which every CTA also takes 1 KB for the system: kUList is as long as kUCtas CTAs allow.
+static_assert(kUCtas * (kUW * sizeof(WarpUnion) + 1024) <= 228 * 1024, "kUCtas CTAs per SM do not fit the shared memory");
 // At 7 CTAs per SM the shared memory has no room for more: an atom item's tables take the place of a residue item's per-atom
 // tables and tile offsets, which are dead between two items.
 static_assert(offsetof(WarpUnion, offS) + sizeof(WarpUnion::offS) - offsetof(WarpUnion, sqC) == kAtomsPerWarp * sizeof(SmallTab),
@@ -72,49 +63,15 @@ static_assert(offsetof(WarpUnion, offS) + sizeof(WarpUnion::offS) - offsetof(War
 static_assert(offsetof(WarpUnion, sqC) % alignof(SmallTab) == 0, "SmallTab alignment");
 __device__ __forceinline__ SmallTab *quad_tabs(WarpUnion &w) { return reinterpret_cast<SmallTab *>(w.sqC); }
 
-// Membership of one atom in the warp's tile, exactly, without square roots: a lane takes one box row of the atom and one
-// direction along the section axis, starting at the section nearest the atom (isc) and walking away from it.  Along that walk
-// the squared distance of every column only grows (each rounding step of fl(fl(X2 + Y2) + Z2) is monotone in the section
-// term), and inside a (row, section) line the in-sphere columns are one interval around the column nearest the atom (km), so
-// the interval [kl, kh] can only SHRINK from one section to the next: the lane keeps it and re-tests just its two ends with
-// the reference's float64 predicate (row_pred), stepping an end inwards while it is outside.  About two tests per line
-// instead of a chord guess with four (round 1) -- and no floating-point guess at all.
+// Membership of one atom in the warp's tile, exactly: a lane takes (row, section) lines of the atom's box, each on its own --
+// row_chord finds the line's in-sphere columns and the lane ORs the run into the line's word.  (A sweep along the
+// sections that narrows one interval from line to line needs fewer tests per line, but chains every line to the previous one
+// and was slower: profiles/r02_union_phases.md.)
 template <int MODE>
-__device__ __forceinline__ void v2_mark_atom(WarpUnion &w, int lane, int cl, int nC, int rl, int nR, int sl, int nS, double T, int kmin,
-                                             int smin) {
+__device__ __forceinline__ void mark_atom(WarpUnion &w, int lane, int cl, int nC, int rl, int nR, int sl, int nS, double T, float xc,
+                                          float inv_gl, int kmin) {
     const double *sqc = w.sqC;
     int km = kmin;  // the column nearest the atom: the box's centre column or, after rounding, one of its neighbours
-    if (km > 0 && sqc[km - 1] < sqc[km]) --km;
-    else if (km + 1 < nC && sqc[km + 1] < sqc[km]) ++km;
-    int isc = smin;  // likewise the section nearest the atom
-    if (isc > 0 && w.sqS[isc - 1] < w.sqS[isc]) --isc;
-    else if (isc + 1 < nS && w.sqS[isc + 1] < w.sqS[isc]) ++isc;
-    for (int item = lane; item < 2 * nR; item += 32) {
-        const int ir = item >> 1, dir = item & 1;          // dir 0: isc, isc + 1, ...; dir 1: isc - 1, isc - 2, ...
-        const double sr = w.sqR[ir];
-        int kl = 0, kh = nC - 1;
-        uint32_t *words = w.bits + (rl + ir) * kUT + sl;
-        for (int is = dir ? isc - 1 : isc; dir ? is >= 0 : is < nS; is += dir ? -1 : 1) {
-            const double ss = w.sqS[is];
-            const double A = (MODE == 0) ? ss : ((MODE == 1) ? sr : __dadd_rn(sr, ss));
-            const double B = (MODE == 0) ? sr : ss;
-            if (!row_pred<MODE>(sqc, km, A, B, T)) break;  // the line misses the sphere, and so do all lines further out
-            while (!row_pred<MODE>(sqc, kl, A, B, T)) ++kl;  // stops at km at the latest
-            while (!row_pred<MODE>(sqc, kh, A, B, T)) --kh;
-            const int count = kh - kl + 1;
-            const uint32_t run = count >= 32 ? ~0u : ((1u << count) - 1u);
-            words[is] |= run << (cl + kl);  // within an atom this word belongs to this lane alone
-        }
-    }
-}
-
-// The same with round 1's chord guess (row_chord): every (row, section) line on its own -- more instructions per line than
-// the sweep, but the lines are independent (no chain from one section to the next).  Selected with -DPE_UNION_SWEEP=0.
-template <int MODE>
-__device__ __forceinline__ void v2_mark_atom_chord(WarpUnion &w, int lane, int cl, int nC, int rl, int nR, int sl, int nS, double T, float xc,
-                                                   float inv_gl, int kmin) {
-    const double *sqc = w.sqC;
-    int km = kmin;
     if (km > 0 && sqc[km - 1] < sqc[km]) --km;
     else if (km + 1 < nC && sqc[km + 1] < sqc[km]) ++km;
     const int shift = nS > 1 ? 32 - __clz(nS - 1) : 0;
@@ -170,12 +127,12 @@ __device__ __forceinline__ void step_sum(const float *v, SphereAcc &acc, float c
 // almost always ONE run, written with a counted loop; rows with holes are bit-scanned), and the list is walked densely, 8
 // (or, for short lists, 4) independent loads per lane and step.
 // Measured and dropped (profiles/r02_union_phases.md): keeping a batch's loads in flight across the compaction of the next one,
-// in registers (146.3 us) or as cp.async copies into the list itself (147.9 us) against 144.4 us for this plain form; 6 / 7 / 8 / 9
-// CTAs per SM 165 / 144 / 146-148 (spills at 64 registers) / 174 us.  No single pipe limits the kernel (issue slots 64 % busy; ALU
-// 38 %, LSU 32 %, XU 20 %, FP64 12 %): it is the length of each warp's dependent instruction chains at 28 warps per SM.
+// in registers (146.3 us) or as cp.async copies into the list itself (147.9 us) against 144.4 us for this plain form.  No single
+// pipe limits the kernel (issue slots 64 % busy; ALU 38 %, LSU 32 %, XU 20 %, FP64 12 %): it is the length of each warp's
+// dependent instruction chains at 28 warps per SM.
 template <bool CHECKED, bool HASNEG>
-__device__ __forceinline__ void v2_gather(WarpUnion &w, const float *__restrict__ rho, SphereAcc &acc, float cp, float cn, int lane,
-                                          int tR, int tS) {
+__device__ __forceinline__ void gather_tile(WarpUnion &w, const float *__restrict__ rho, SphereAcc &acc, float cp, float cn, int lane,
+                                            int tR, int tS) {
     int *list = w.list;
     const int oc0 = w.offC[0];
     for (int r0 = 0; r0 < tR; ++r0) {  // one tile row = tS (<= 32) words = one batch
@@ -371,13 +328,8 @@ __global__ void __launch_bounds__(kUW * 32, kUCtas)
                                 PHASE_MARK(1);
                                 // centre column of the box (range(c - R - 1, c + R + 1): c = lo + dim / 2), clamped into the tile part
                                 const int kmin = min(max(b0 + d0 / 2 - cl, 0), nC - 1);
-#if PE_UNION_SWEEP
-                                const int smin = min(max(b2 + d2 / 2 - sl, 0), nS - 1);
-                                v2_mark_atom<MODE>(w, lane, cl - tc0, nC, rl - tr0, nR, sl - ts0, nS, T, kmin, smin);
-#else
                                 const float xc = (float)((sel3(ax, ay, az, icx) - g.origin[icx]) / g.grid_length[icx] - (double)cl);
-                                v2_mark_atom_chord<MODE>(w, lane, cl - tc0, nC, rl - tr0, nR, sl - ts0, nS, T, xc, inv_gl, kmin);
-#endif
+                                mark_atom<MODE>(w, lane, cl - tc0, nC, rl - tr0, nR, sl - ts0, nS, T, xc, inv_gl, kmin);
                                 __syncwarp();  // tables are rewritten by the next atom; its rows may share words with this one
                                 PHASE_MARK(2);
                             } else {
@@ -398,14 +350,14 @@ __global__ void __launch_bounds__(kUW * 32, kUCtas)
                         PHASE_MARK(1);
                         if (checked) {
                             if (has_neg)
-                                v2_gather<true, true>(w, rho, acc, cp, cn, lane, tR, tS);
+                                gather_tile<true, true>(w, rho, acc, cp, cn, lane, tR, tS);
                             else
-                                v2_gather<true, false>(w, rho, acc, cp, cn, lane, tR, tS);
+                                gather_tile<true, false>(w, rho, acc, cp, cn, lane, tR, tS);
                         } else {
                             if (has_neg)
-                                v2_gather<false, true>(w, rho, acc, cp, cn, lane, tR, tS);
+                                gather_tile<false, true>(w, rho, acc, cp, cn, lane, tR, tS);
                             else
-                                v2_gather<false, false>(w, rho, acc, cp, cn, lane, tR, tS);
+                                gather_tile<false, false>(w, rho, acc, cp, cn, lane, tR, tS);
                         }
                         __syncwarp();
                         PHASE_MARK(3);
@@ -438,7 +390,7 @@ __global__ void __launch_bounds__(kUW * 32, kUCtas)
 int launch_union_warp(const pe_geom *g, const float *d_rho, int n_groups, const int32_t *d_group_start, const double *d_xyz,
                       const float *d_radius, int32_t *box, double *thr, float cut_pos, float cut_neg, int *d_counter, double *d_out,
                       int n_quad_atoms, const float *d_atom_radius, double *d_out_atoms, cudaStream_t st) {
-    const int mode = g->map2xyz[2] == 1 ? 0 : (g->map2xyz[2] == 2 ? 1 : 2);  // crs axis that carries z
+    const int mode = z_axis_mode(g);
     PE_CUDA(cudaMemsetAsync(d_counter, 0, sizeof(int), st));
     const int warps_needed = n_groups + (n_quad_atoms + kAtomsPerWarp - 1) / kAtomsPerWarp;
     int grid = (warps_needed + kUW - 1) / kUW;

@@ -57,11 +57,6 @@ t = (ctypes.c_ulonglong * 12)()
 _lib.load().pe_blob_stage_times(t)
 t = list(t)
 print("blob sparse phases P1..P4 (us):", [round((t[i + 1] - t[i]) / 1e3, 1) for i in range(4)])
-u = (ctypes.c_ulonglong * 4)()
-_lib.load().pe_sphere_union_cycles(u)
-tot = float(sum(u)) or 1.0
-if sum(u):  # only when the library was built with -DPE_UNION_PHASE_CYCLES=1
-    print("union kernel cycles by phase (prologue, membership, gather, epilogue): %s" % [round(x / tot, 3) for x in u])
 u = (ctypes.c_ulonglong * 5)()
 _lib.load().pe_sphere_union_warp_cycles(u)
 if sum(u):

@@ -126,6 +126,19 @@ def test_a_radius_above_the_bound_gives_nan_rows():
     assert np.array_equal(got_g, dm.sphere_sums(xyz, group_r, start, 0.5, 0.0).cpu().numpy())
 
 
+def test_workspace_holds_what_the_entry_points_carve():
+    """The atoms' boxes (6 int32 each) and distance thresholds (float64) in 256-byte aligned regions, then the grouped kernel's
+    work-item counter (one int), which a grouped call writes even when it has no atoms."""
+    lib = _lib.load()
+
+    def aligned(nbytes):
+        return (nbytes + 255) // 256 * 256
+
+    assert lib.pe_sphere_workspace_bytes(0) >= 4
+    for n in (1, 5, 40_000):
+        assert lib.pe_sphere_workspace_bytes(n) >= aligned(24 * n) + aligned(8 * n) + 4, n
+
+
 def test_argument_errors_match_pe_sphere_sums():
     """Checked on the host before anything is launched: the same status codes as pe_sphere_sums."""
     lib = _lib.load()
