@@ -227,7 +227,8 @@ int pe_slab_status(const void *d_ws, void *stream, int32_t *bad);
 /* createCrsLists (pdb_eda/cutils.pyx:41-70) on an arbitrary list of n un-wrapped voxels (d_crs n x 3 int32):
  * d_label[i] = cluster number in the reference's creation order (by first unused input index).
  * d_nclusters: TWO int64: [0] = number of clusters, [1] = non-zero when an index was outside the key range
- * (|index| < 2^20 without groups; |index| < 2^13 and group < 2^22 with groups) and the result is invalid.
+ * (|index| < 2^20, i.e. -1048575 .. 1048575, without groups; |index| < 2^13, i.e. -8191 .. 8191, and
+ * 0 <= group < 2^22 with groups) and the result is invalid.
  * The grouped form clusters every group (d_group[i] >= 0, e.g. the residue a cloud voxel belongs to) on its own
  * -- the residue-cloud merging of aggregateCloud (pdb_eda/densityAnalysis.py:646-677) -- and tolerates repeated
  * voxels: d_first[i] (optional) = 1 iff i is the first entry holding its (group, voxel), which is what turns the
@@ -257,7 +258,9 @@ int pe_pair_metrics(const pe_geom *g, const float *d_rho_fo, const float *d_rho_
  * blobs overlap iff some voxel of one is identical or 26-adjacent to some voxel of the other (same group when
  * d_group is given).  Writes each overlapping unordered pair once as (smaller owner, larger owner) to d_pairs
  * (cap_pairs x 2 int32, unordered); d_npairs: TWO int64: [0] = number of pairs found (re-run with a larger
- * cap_pairs when it exceeds it), [1] = key-range overflow flag as above.
+ * cap_pairs when it exceeds it), [1] = key-range overflow flag as above.  d_pairs is complete only when
+ * d_npairs[0] <= cap_pairs; otherwise [0] is an upper bound and d_pairs holds some true pairs (possibly none, and
+ * not necessarily in its first rows).
  * This is the overlap matrix of pdb_eda/densityAnalysis.py:646-649 and :689-692 in sparse form.
  * d_ws: >= pe_overlap_workspace_bytes(n, cap_pairs). */
 int64_t pe_overlap_workspace_bytes(int64_t n, int64_t cap_pairs);

@@ -329,6 +329,24 @@ __device__ __forceinline__ void fill_box_record(const FillArgs &A, int a, int ma
                 ((unsigned long long)(d1 & 15) << 4) | (unsigned long long)(d2 & 15);
 }
 
+// Shift masks of the flood fill for box positions 32 w .. 32 w + 31 (p = (ic*D1 + ir)*D2 + is): nfs / nls = positions that may
+// move -1 / +1 along sections, nfr / nlr = -1 / +1 along rows.  They cover EVERY position, member or not: one dilation step moves
+// along sections and then along rows, and a diagonal neighbour is reached through a position that may hold no voxel.  Built row
+// by row (a row = D2 consecutive positions), so a word costs at most 32 / D2 + 2 steps.
+__device__ __forceinline__ void shift_masks(int w, int vol, int D1, int D2, uint32_t &nfs, uint32_t &nls, uint32_t &nfr, uint32_t &nlr) {
+    nfs = nls = nfr = nlr = 0u;
+    const int p0 = 32 * w, p1 = min(p0 + 32, vol);
+    for (int t = p0 / D2; t * D2 < p1; ++t) {
+        const int a = max(t * D2, p0) - p0, e = min((t + 1) * D2, p1) - p0;  // the row's bits a .. e-1 in this word
+        const uint32_t row = (e - a >= 32 ? 0xffffffffu : (1u << (e - a)) - 1u) << a;
+        const int ir = t % D1;
+        if (ir != 0) nfr |= row;
+        if (ir != D1 - 1) nlr |= row;
+        nfs |= t * D2 >= p0 ? row & ~(1u << a) : row;               // not the row's first position (is = 0)
+        nls |= (t + 1) * D2 <= p1 ? row & ~(1u << (e - 1)) : row;    // not its last (is = D2 - 1)
+    }
+}
+
 // One atom by one warp (boxes of more than 256 candidates, or no bitmap from the count pass).
 __device__ __forceinline__ void fill_one_atom(const FillArgs &A, int a, unsigned char *base, AxisTab *tab, pe_geom *gs, int lane) {
     const pe_batch_map *__restrict__ maps = A.maps;
@@ -424,22 +442,8 @@ __device__ __forceinline__ void fill_one_atom(const FillArgs &A, int a, unsigned
         // masks that stop a shift from wrapping into the next row / plane -- intersected with the unlabelled voxels, until it stops
         // growing; clusters therefore come out in the order of their first member.  (The min-label propagation this replaces was
         // 56 % of the kernel's instructions: 27 bit tests and label look-ups per voxel and round.)
-        uint32_t nfs = 0u, nls = 0u, nfr = 0u, nlr = 0u;  // source voxels that may move -1 / +1 along sections, -1 / +1 along rows
-        {
-            // only the lane's own voxels ever move, so the masks are formed for its set bits only (the loop over all 32 positions
-            // of every lane was 27 % of the kernel's instructions); p / D by multiplication: exact for p < 1,024, D <= 32
-            const uint32_t m2 = (65536u + (uint32_t)D2 - 1u) / (uint32_t)D2, m1 = (65536u + (uint32_t)D1 - 1u) / (uint32_t)D1;
-            for (uint32_t c = lane < nw ? bits[lane] : 0u; c; c &= c - 1u) {
-                const int j = __ffs((int)c) - 1;
-                const uint32_t p = 32u * (uint32_t)lane + (uint32_t)j;
-                const uint32_t q = D2 <= 32 ? (p * m2) >> 16 : p / (uint32_t)D2;
-                const int is = (int)(p - q * (uint32_t)D2), ir = (int)(D1 <= 32 ? q - ((q * m1) >> 16) * (uint32_t)D1 : q % (uint32_t)D1);
-                nfs |= (is != 0 ? 1u : 0u) << j;
-                nls |= (is != D2 - 1 ? 1u : 0u) << j;
-                nfr |= (ir != 0 ? 1u : 0u) << j;
-                nlr |= (ir != D1 - 1 ? 1u : 0u) << j;
-            }
-        }
+        uint32_t nfs, nls, nfr, nlr;  // positions that may move -1 / +1 along sections, -1 / +1 along rows
+        shift_masks(lane, vol, D1, D2, nfs, nls, nfr, nlr);
         auto shl = [&](uint32_t v, int k) {  // the bit string moved k positions up
             const int q = k >> 5, r = k & 31;
             uint32_t a = __shfl_up_sync(kFull, v, q), c = __shfl_up_sync(kFull, v, q + 1);
@@ -694,17 +698,8 @@ __global__ void __launch_bounds__(kSphereWarps * 32) cloud_fill_kernel(const Fil
     // 4 + 5. 26-connected clusters by bit-parallel flood fill, numbered by their first member (createCrsLists order)
     // p / D by multiplication: exact for p < 256, D <= 256
     const uint32_t m2 = (65536u + (uint32_t)max(D2, 1) - 1u) / (uint32_t)max(D2, 1), m1 = (65536u + (uint32_t)max(D1, 1) - 1u) / (uint32_t)max(D1, 1);
-    uint32_t nfs = 0u, nls = 0u, nfr = 0u, nlr = 0u;  // own voxels that may move -1 / +1 along sections, -1 / +1 along rows
-    for (uint32_t c = mine; c; c &= c - 1u) {
-        const int j = __ffs((int)c) - 1;
-        const uint32_t p = 32u * (uint32_t)l8 + (uint32_t)j;
-        const uint32_t q = (p * m2) >> 16;
-        const int is = (int)(p - q * (uint32_t)D2), ir = (int)(q - ((q * m1) >> 16) * (uint32_t)D1);
-        nfs |= (is != 0 ? 1u : 0u) << j;
-        nls |= (is != D2 - 1 ? 1u : 0u) << j;
-        nfr |= (ir != 0 ? 1u : 0u) << j;
-        nlr |= (ir != D1 - 1 ? 1u : 0u) << j;
-    }
+    uint32_t nfs, nls, nfr, nlr;  // positions that may move -1 / +1 along sections, -1 / +1 along rows
+    shift_masks(l8, vol, D1, D2, nfs, nls, nfr, nlr);
     auto shl = [&](uint32_t v, int k) {  // the group's bit string moved k positions up
         const int q = k >> 5, r = k & 31;
         uint32_t x = __shfl_up_sync(gmask, v, q, 8), y = __shfl_up_sync(gmask, v, q + 1, 8);

@@ -17,8 +17,9 @@
 // then ranking the roots), which is the order createCrsLists creates them in.
 //
 // Entries may carry a group id (e.g. the residue a cloud voxel belongs to): voxels only see voxels of their own
-// group.  Key layout: without groups 3 x 21 bits (|index| < 2^20); with groups 22 bits of group + 3 x 14 bits
-// (|index| < 2^13, group < 2^22) -- checked on the device, violations raise the overflow flag.
+// group.  Key layout: without groups 3 x 21 bits (|index| < 2^20, i.e. -1048575 .. 1048575); with groups 22 bits of
+// group + 3 x 14 bits (|index| < 2^13, i.e. -8191 .. 8191, and 0 <= group < 2^22) -- checked on the device, anything
+// else (including -2^20 / -2^13 and a negative group) raises the overflow flag.
 #include "pe_common.cuh"
 
 namespace pe {
@@ -27,16 +28,20 @@ constexpr int kClThreads = 256;
 constexpr uint64_t kEmptyKey = ~0ull;
 constexpr uint32_t kNil = 0xffffffffu;
 
+// An axis field holds index + (2^(bits-1) - 1), i.e. 0 .. 2^bits - 2 for |index| < 2^(bits-1): the all-ones field is never
+// used, so no valid key equals kEmptyKey (with groups the key fills all 64 bits).
 __device__ __forceinline__ bool pack_crs(int c, int r, int s, int group, bool grouped, uint64_t &key) {
     if (grouped) {
-        const int off = 1 << 13;
+        const int off = (1 << 13) - 1;
+        const unsigned top = (1u << 14) - 2u;
         const unsigned uc = (unsigned)(c + off), ur = (unsigned)(r + off), us = (unsigned)(s + off);
-        if ((uc | ur | us) >> 14 || (unsigned)group >> 22) return false;
+        if (uc > top || ur > top || us > top || (unsigned)group >> 22) return false;
         key = ((uint64_t)(unsigned)group << 42) | ((uint64_t)uc << 28) | ((uint64_t)ur << 14) | (uint64_t)us;
     } else {
-        const int off = 1 << 20;
+        const int off = (1 << 20) - 1;
+        const unsigned top = (1u << 21) - 2u;
         const unsigned uc = (unsigned)(c + off), ur = (unsigned)(r + off), us = (unsigned)(s + off);
-        if ((uc | ur | us) >> 21) return false;
+        if (uc > top || ur > top || us > top) return false;
         key = ((uint64_t)uc << 42) | ((uint64_t)ur << 21) | (uint64_t)us;
     }
     return true;
