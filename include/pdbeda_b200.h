@@ -254,6 +254,28 @@ int pe_crs_stats(const pe_geom *g, const float *d_rho, int64_t n, const int32_t 
 int pe_pair_metrics(const pe_geom *g, const float *d_rho_fo, const float *d_rho_diff, int64_t n, const int32_t *d_crs,
                     const int32_t *d_label, const uint8_t *d_take, int64_t n_groups, double *d_out, void *stream);
 
+/* calculateRsccRsrMetrics over the set-union of a group's atom spheres (getSphereCrsFromXyzList, pdb_eda/cutils.pyx:250-271:
+ * the reference's box and predicate, float32 radius, un-wrapped indices, a repeated voxel counted once) for the groups of many
+ * structures at once -- residueMetrics / atomMetrics (pdb_eda/densityAnalysis.py:803-858) of a whole batch.
+ * d_maps (device array, n_maps entries): per structure the geometry and the device pointers of its 2Fo-Fc map (d_fo) and its
+ * Fo-Fc map (d_diff) on the same grid; fewer than 2^31 stored voxels per map.  Group g is made of the atoms
+ * d_group_start[g] .. d_group_start[g+1] (d_xyz n x 3 float64, d_radius n float32) on map d_group_map[g].
+ * d_out[g*8 ..] = the eight sums of pe_pair_metrics over the group's voxel set: n, sum fo, sum fc, sum |fo - fc|,
+ * sum |fo + fc|, sum (fo-mean)^2, sum (fc-mean)^2, sum (fo-mean)(fc-mean), with fc = fo - 2 * diff in float64, voxels the map
+ * does not cover counted with fo = fc = 0 and the moments centred on the group's own means (two passes).  An empty group
+ * gives a zero row, a group whose d_group_map entry is outside [0, n_maps) a NaN row.  The summation order is fixed:
+ * results are bit-identical from run to run and do not depend on the other groups of the call.
+ * d_ws: >= pe_pair_union_workspace_bytes(n_atoms). */
+typedef struct pe_pair_map {
+    pe_geom geom;
+    const float *d_fo;
+    const float *d_diff;
+} pe_pair_map;
+int64_t pe_pair_union_workspace_bytes(int32_t n_atoms);
+int pe_pair_union_metrics(int32_t n_maps, const pe_pair_map *d_maps, int32_t n_groups, const int32_t *d_group_map,
+                          const int32_t *d_group_start, const double *d_xyz, const float *d_radius, double *d_out, void *d_ws,
+                          void *stream);
+
 /* testOverlap (pdb_eda/cutils.pyx:8-25), all pairs at once: every entry is a voxel of the blob d_owner[i]; two
  * blobs overlap iff some voxel of one is identical or 26-adjacent to some voxel of the other (same group when
  * d_group is given).  Writes each overlapping unordered pair once as (smaller owner, larger owner) to d_pairs

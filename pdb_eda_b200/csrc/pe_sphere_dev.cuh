@@ -266,6 +266,48 @@ __device__ __forceinline__ bool row_chord(const double *sqc, int nC, int km, flo
     return true;
 }
 
+// ------------------------------------------------------------------------------------------------ tile membership
+// Shared by the grouped kernels (pe_union.cu, pe_metrics.cu): a warp owns a 32^3 tile, bits holds one 32-bit word per
+// (row, section) (row-major, 32 sections per row).  sqc / sqR / sqS: the atom's squares along the tile part's columns,
+// rows and sections.
+// Membership of one atom in the warp's tile, exactly: a lane takes (row, section) lines of the atom's box, each on its own --
+// row_chord finds the line's in-sphere columns and the lane ORs the run into the line's word.  (A sweep along the
+// sections that narrows one interval from line to line needs fewer tests per line, but chains every line to the previous one
+// and was slower: profiles/r02_union_phases.md.)
+template <int MODE>
+__device__ __forceinline__ void mark_atom(uint32_t *bits, const double *sqc, const double *sqR, const double *sqS, int lane, int cl,
+                                          int nC, int rl, int nR, int sl, int nS, double T, float xc, float inv_gl, int kmin) {
+    int km = kmin;  // the column nearest the atom: the box's centre column or, after rounding, one of its neighbours
+    if (km > 0 && sqc[km - 1] < sqc[km]) --km;
+    else if (km + 1 < nC && sqc[km + 1] < sqc[km]) ++km;
+    const int shift = nS > 1 ? 32 - __clz(nS - 1) : 0;
+    const int total = nR << shift;
+#pragma unroll 2
+    for (int li = lane; li < total; li += 32) {
+        const int is = li & ((1 << shift) - 1), ir = li >> shift;
+        if (is >= nS) continue;
+        const double sr = sqR[ir], ss = sqS[is];
+        const double A = (MODE == 0) ? ss : ((MODE == 1) ? sr : __dadd_rn(sr, ss));
+        const double B = (MODE == 0) ? sr : ss;
+        int kl, kh;
+        if (!row_chord<MODE>(sqc, nC, km, xc, inv_gl, A, B, T, kl, kh)) continue;  // the row misses the sphere
+        const int count = kh - kl + 1;
+        const uint32_t run = count >= 32 ? ~0u : ((1u << count) - 1u);
+        bits[(rl + ir) * 32 + (sl + is)] |= run << (cl + kl);  // within an atom this word belongs to this lane alone
+    }
+}
+
+__device__ __forceinline__ int warp_min(int v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = min(v, __shfl_xor_sync(kFull, v, o));
+    return v;
+}
+__device__ __forceinline__ int warp_max(int v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = max(v, __shfl_xor_sync(kFull, v, o));
+    return v;
+}
+
 // ------------------------------------------------------------------------------------------------ per-atom sums, 4 atoms per warp
 // At the atom-type radii of the cloud pass (0.6 - 1.3 A on a 0.5 A grid) a box is 4^3 or 6^3 candidates for ~15 in-sphere
 // voxels, so when all four boxes of a warp's quad are at most kSmallDim wide (orthogonal cell) each atom gets 8 lanes: a lane

@@ -63,34 +63,6 @@ static_assert(offsetof(WarpUnion, offS) + sizeof(WarpUnion::offS) - offsetof(War
 static_assert(offsetof(WarpUnion, sqC) % alignof(SmallTab) == 0, "SmallTab alignment");
 __device__ __forceinline__ SmallTab *quad_tabs(WarpUnion &w) { return reinterpret_cast<SmallTab *>(w.sqC); }
 
-// Membership of one atom in the warp's tile, exactly: a lane takes (row, section) lines of the atom's box, each on its own --
-// row_chord finds the line's in-sphere columns and the lane ORs the run into the line's word.  (A sweep along the
-// sections that narrows one interval from line to line needs fewer tests per line, but chains every line to the previous one
-// and was slower: profiles/r02_union_phases.md.)
-template <int MODE>
-__device__ __forceinline__ void mark_atom(WarpUnion &w, int lane, int cl, int nC, int rl, int nR, int sl, int nS, double T, float xc,
-                                          float inv_gl, int kmin) {
-    const double *sqc = w.sqC;
-    int km = kmin;  // the column nearest the atom: the box's centre column or, after rounding, one of its neighbours
-    if (km > 0 && sqc[km - 1] < sqc[km]) --km;
-    else if (km + 1 < nC && sqc[km + 1] < sqc[km]) ++km;
-    const int shift = nS > 1 ? 32 - __clz(nS - 1) : 0;
-    const int total = nR << shift;
-#pragma unroll 2
-    for (int li = lane; li < total; li += 32) {
-        const int is = li & ((1 << shift) - 1), ir = li >> shift;
-        if (is >= nS) continue;
-        const double sr = w.sqR[ir], ss = w.sqS[is];
-        const double A = (MODE == 0) ? ss : ((MODE == 1) ? sr : __dadd_rn(sr, ss));
-        const double B = (MODE == 0) ? sr : ss;
-        int kl, kh;
-        if (!row_chord<MODE>(sqc, nC, km, xc, inv_gl, A, B, T, kl, kh)) continue;  // the row misses the sphere
-        const int count = kh - kl + 1;
-        const uint32_t run = count >= 32 ? ~0u : ((1u << count) - 1u);
-        w.bits[(rl + ir) * kUT + (sl + is)] |= run << (cl + kl);  // within an atom this word belongs to this lane alone
-    }
-}
-
 // Sums of one step of the gather: kULoads values per lane; the float64 additions form a small tree (fixed shape:
 // deterministic) so that no accumulator carries a chain of eight dependent additions.
 template <bool HASNEG, int N>
@@ -203,17 +175,6 @@ __device__ __forceinline__ void gather_tile(WarpUnion &w, const float *__restric
             if (!__any_sync(kFull, pending)) break;
         }
     }
-}
-
-__device__ __forceinline__ int warp_min(int v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = min(v, __shfl_xor_sync(kFull, v, o));
-    return v;
-}
-__device__ __forceinline__ int warp_max(int v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = max(v, __shfl_xor_sync(kFull, v, o));
-    return v;
 }
 
 // Work items, handed out in order through one counter: [0, n_groups) are groups (the long items), then, when n_quad_atoms > 0,
@@ -329,7 +290,8 @@ __global__ void __launch_bounds__(kUW * 32, kUCtas)
                                 // centre column of the box (range(c - R - 1, c + R + 1): c = lo + dim / 2), clamped into the tile part
                                 const int kmin = min(max(b0 + d0 / 2 - cl, 0), nC - 1);
                                 const float xc = (float)((sel3(ax, ay, az, icx) - g.origin[icx]) / g.grid_length[icx] - (double)cl);
-                                mark_atom<MODE>(w, lane, cl - tc0, nC, rl - tr0, nR, sl - ts0, nS, T, xc, inv_gl, kmin);
+                                mark_atom<MODE>(w.bits, w.sqC, w.sqR, w.sqS, lane, cl - tc0, nC, rl - tr0, nR, sl - ts0, nS, T, xc, inv_gl,
+                                                kmin);
                                 __syncwarp();  // tables are rewritten by the next atom; its rows may share words with this one
                                 PHASE_MARK(2);
                             } else {

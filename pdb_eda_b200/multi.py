@@ -367,3 +367,47 @@ class PoolShard:
         if device is None:
             device = torch.device("cuda", torch.cuda.current_device()) if torch.cuda.is_available() else torch.device("cpu")
         return gatherPacked(cumulative, rows, self.atomTypes, device, group, local)
+
+
+def summarizeMetrics(ok, failed, rows, device="cpu", group=None):
+    """(entries ok, entries failed, rows) summed over the ranks with ONE all_reduce; the same dict on every rank."""
+    counts = np.array([ok, failed, rows], dtype=np.float64)
+    if dist.is_initialized() and dist.get_world_size(group) > 1:
+        t = torch.from_numpy(counts).to(device)
+        dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
+        counts = t.cpu().numpy()
+    return {"ok": int(counts[0]), "failed": int(counts[1]), "rows": int(counts[2])}
+
+
+def runMultipleMetrics(items, loader, level, costs=None, write=None, device=None, group=None, maxBytes=8 << 30):
+    """RSCC / RSR rows (``residueMetrics()`` or ``atomMetrics()``, ``level`` "residue" / "atom") of many entries:
+    ``loader(item)`` returns a DensityAnalysis (or 0); the entries are sharded over the ranks of the default process group
+    longest first, and every rank analyses its share in batches of at most ``maxBytes`` device bytes (both maps + atoms,
+    ``metricsBatch.MetricsBatch``).  Rows are ragged and large, so they are not gathered: ``write(index, rows)`` is called
+    on the owning rank for every entry that yields rows.  An entry that fails to load or on which the single-structure
+    call would raise is counted as failed.  Returns the all-reduced counts (``summarizeMetrics``) on every rank."""
+    from . import metricsBatch
+    rank = dist.get_rank(group) if dist.is_initialized() else 0
+    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    costs = [1.0] * len(items) if costs is None else costs
+    mine = shardStructures(costs, world)[rank]                 # longest first
+
+    def loaded():
+        for idx in mine:
+            try:
+                yield idx, loader(items[idx])
+            except Exception:
+                yield idx, 0                                   # a bad entry yields no rows; the run continues
+
+    ok = failed = nrows = 0
+    for idx, rows in metricsBatch.analyzeStream(loaded(), level, maxBytes, device):
+        if rows is None:
+            failed += 1
+            continue
+        ok += 1
+        nrows += len(rows)
+        if write is not None:
+            write(idx, rows)
+    if device is None:
+        device = torch.device("cuda", torch.cuda.current_device()) if torch.cuda.is_available() else torch.device("cpu")
+    return summarizeMetrics(ok, failed, nrows, device, group)

@@ -141,19 +141,34 @@ def analyze(args):
             header, rows = analyzer.residueMetricsHeaderList, analyzer.residueMetrics()
         else:
             header, rows = analyzer.atomMetricsHeaderList, analyzer.atomMetrics()
-            for info in rows:
-                info[4] = [x for x in info[4]]
-                info[5] = [float(x) for x in info[5]]
-        rows = [[numpyConverter(e) for e in row] for row in rows]
+        return statisticsResult(args, header, rows, analyzer.pdbid)
     if args.include_pdbid:
         header = ["pdbid"] + header
         rows = [[analyzer.pdbid] + row for row in rows]
     return header, rows
 
 
+def statisticsResult(args, header, rows, pdbid):
+    """(header, rows) of ``statistics`` from the rows of residueMetrics() / atomMetrics(), as written to the result file."""
+    if not args.residue:
+        for info in rows:
+            info[4] = [x for x in info[4]]
+            info[5] = [float(x) for x in info[5]]
+    rows = [[numpyConverter(e) for e in row] for row in rows]
+    if args.include_pdbid:
+        header = ["pdbid"] + header
+        rows = [[pdbid] + row for row in rows]
+    return header, rows
+
+
 def main(argv=None):
     args = buildParser().parse_args(argv)
     header, rows = analyze(args)
+    writeResult(args, header, rows)
+
+
+def writeResult(args, header, rows):
+    """Writes (header, rows) to ``args.out_file`` ("-": stdout) in ``args.out_format``."""
     with open(args.out_file, "w") if args.out_file != "-" else sys.stdout as out:
         if header is None:
             out.write(json.dumps(rows))
