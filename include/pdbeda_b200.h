@@ -144,6 +144,30 @@ int pe_sphere_sums_atoms_and_groups(const pe_geom *g, const float *d_rho, int32_
                                     int32_t n_groups, const int32_t *d_group_start, float cut_pos, float cut_neg,
                                     double *d_out_atoms, double *d_out_groups, void *d_ws, void *stream);
 
+/* pe_sphere_sums for the atoms of many structures, each on its own map, in one launch (the region density / discrepancy of a
+ * whole batch).  d_maps (device array, n_maps entries): per structure its geometry, the device pointer of its map and its own
+ * cutoffs (cut_pos >= 0 >= cut_neg; the caller checks them where it builds the table, an entry that breaks the rule gives NaN
+ * rows).  Structure k owns the atoms d_atom_start[k] .. d_atom_start[k+1] (n_maps + 1 offsets; d_xyz n_atoms x 3 float64,
+ * d_radius n_atoms float32).  Group g is summed on map d_group_map[g]:
+ *   grouped   (d_group_start given): group g is the set-union of the atoms d_group_start[g] .. d_group_start[g+1], one warp
+ *             per group as in pe_sphere_sums; d_atom_start may be NULL;
+ *   per atom  (d_group_start NULL, n_groups == n_atoms): group a is atom a; atoms are taken four at a time from each
+ *             structure's first atom, so a quad never spans two structures.
+ * d_out (n_groups x PE_SPHERE_NOUT) holds the values documented for pe_sphere_sums.  Every row is bit-identical to the row
+ * pe_sphere_sums gives for the same structure alone (its geometry, map, cutoffs, atoms and group offsets) when the atoms of
+ * each structure name one map; it does not depend on the other structures of the call.  A group whose map index is outside
+ * [0, n_maps) gives a NaN row.  d_ws: >= pe_batch_sphere_sums_workspace_bytes(n_atoms) bytes. */
+typedef struct pe_sums_map {
+    pe_geom geom;
+    const float *d_rho;
+    float cut_pos;
+    float cut_neg;
+} pe_sums_map;
+int64_t pe_batch_sphere_sums_workspace_bytes(int64_t n_atoms);
+int pe_batch_sphere_sums(int32_t n_maps, const pe_sums_map *d_maps, int32_t n_atoms, const double *d_xyz, const float *d_radius,
+                         int32_t n_groups, const int32_t *d_group_map, const int32_t *d_group_start, const int32_t *d_atom_start,
+                         double *d_out, void *d_ws, void *stream);
+
 /* getSphereCrsFromXyz (pdb_eda/cutils.pyx:220-248), batched, as lists.  Two calls:
  *   pe_sphere_count: d_count[a] = len(getSphereCrsFromXyz(dm, xyz[a], radius[a], cutoff)), and
  *                    d_box[a*6 ..] = box low corner (c, r, s) and box extents (nc, nr, ns);

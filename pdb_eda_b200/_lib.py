@@ -73,6 +73,8 @@ SIGNATURES = {
     "pe_cluster_crs_grouped": (ctypes.c_int, [_I64, _P, _P, _P, _P, _P, _P, _P]),
     "pe_crs_stats": (ctypes.c_int, [_GEOM, _P, _I64, _P, _P, _P, _I64, _P, _P]),
     "pe_pair_metrics": (ctypes.c_int, [_GEOM, _P, _P, _I64, _P, _P, _P, _I64, _P, _P]),
+    "pe_batch_sphere_sums_workspace_bytes": (_I64, [_I64]),
+    "pe_batch_sphere_sums": (ctypes.c_int, [_I32, _P, _I32, _P, _P, _I32, _P, _P, _P, _P, _P, _P]),
     "pe_pair_union_workspace_bytes": (_I64, [_I32]),
     "pe_pair_union_metrics": (ctypes.c_int, [_I32, _P, _I32, _P, _P, _P, _P, _P, _P, _P]),
     "pe_overlap_workspace_bytes": (_I64, [_I64, _I64]),

@@ -35,6 +35,9 @@ namespace pe {
 int launch_union_warp(const pe_geom *g, const float *d_rho, int n_groups, const int32_t *d_group_start, const double *d_xyz,
                       const float *d_radius, int32_t *box, double *thr, float cut_pos, float cut_neg, int *d_counter, double *d_out,
                       int n_quad_atoms, const float *d_atom_radius, double *d_out_atoms, cudaStream_t st);  // pe_union.cu
+int launch_batch_union(int n_maps, const pe_sums_map *d_maps, int n_groups, const int32_t *d_group_map, const int32_t *d_group_start,
+                       const double *d_xyz, const float *d_radius, int32_t *box, double *thr, int *d_counter, double *d_out,
+                       cudaStream_t st);  // pe_union.cu
 
 // ------------------------------------------------------------------------------------------------ sums kernel
 // CASEB: the column axis carries z (the last term of the reference's sum), so fl(X2 + Y2) depends on (row, section).
@@ -156,6 +159,78 @@ __global__ void __launch_bounds__(kSphereWarps * 32)
     if (quad_sums<MODE>(g, rho, n_atoms, a0, xyz, radius, cp, cn, stab[warp], lane, out)) return;
     for (int q = 0; q < kAtomsPerWarp && a0 + q < n_atoms; ++q)
         sums_one_atom<MODE>(g, rho, a0 + q, xyz, radius, cp, cn, tabs[warp], lane, out);
+}
+
+// Per-atom sums of many structures, each on its own map (pe_batch_sphere_sums without group offsets).  The work items are the
+// quads of sphere_sums_kernel counted from each structure's first atom, so that a quad never spans two structures and takes
+// the same atoms as it does in a launch for its structure alone; flattened over the structures, they are dealt out to the
+// warps in a fixed stride.  A quad whose atoms all name one valid map runs sphere_sums_kernel's code on it (quad_sums, or
+// sums_one_atom atom by atom); otherwise every atom is summed alone on its own map, or gets a NaN row when that map index or
+// its cutoffs are invalid.  The warp keeps the current map's pe_geom in shared memory.
+__device__ __forceinline__ void copy_geom(pe_geom &dst, const pe_geom &src, int lane) {
+    static_assert(sizeof(pe_geom) % 4 == 0, "pe_geom is copied as 32-bit words");
+    __syncwarp();  // the previous geometry is no longer read
+    for (int i = lane; i < (int)(sizeof(pe_geom) / 4); i += 32) reinterpret_cast<int *>(&dst)[i] = reinterpret_cast<const int *>(&src)[i];
+    __syncwarp();
+}
+
+__device__ __forceinline__ bool sums_map_ok(int m, int n_maps, const pe_sums_map *maps) {
+    return m >= 0 && m < n_maps && !(maps[m].cut_pos < 0.f) && !(maps[m].cut_neg > 0.f);
+}
+
+__global__ void __launch_bounds__(kSphereWarps * 32)
+    batch_sphere_sums_kernel(int n_maps, const pe_sums_map *__restrict__ maps, const int32_t *__restrict__ atom_start,
+                             const int32_t *__restrict__ group_map, const double *__restrict__ xyz, const float *__restrict__ radius,
+                             double *__restrict__ out /* n_atoms x PE_SPHERE_NOUT */) {
+    __shared__ AxisTab tabs[kSphereWarps][2];
+    __shared__ SmallTab stab[kSphereWarps][kAtomsPerWarp];
+    __shared__ pe_geom geoms[kSphereWarps];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t gw = (int64_t)blockIdx.x * kSphereWarps + warp, n_warps = (int64_t)gridDim.x * kSphereWarps;
+    pe_geom &g = geoms[warp];
+    int64_t q_base = 0;  // flattened index of structure k's first quad
+    for (int k = 0; k < n_maps; ++k) {
+        const int s0 = atom_start[k], s1 = atom_start[k + 1];
+        const int64_t nq = s1 > s0 ? (s1 - s0 + kAtomsPerWarp - 1) / kAtomsPerWarp : 0;
+        int64_t t = q_base + ((gw - q_base) % n_warps + n_warps) % n_warps;  // this warp's first quad at or after q_base
+        for (; t < q_base + nq; t += n_warps) {
+            const int a0 = s0 + (int)(t - q_base) * kAtomsPerWarp;
+            const int m = group_map[a0];
+            const int mq = (lane < kAtomsPerWarp && a0 + lane < s1) ? group_map[a0 + lane] : m;
+            if (__all_sync(kFull, mq == m) && sums_map_ok(m, n_maps, maps)) {
+                copy_geom(g, maps[m].geom, lane);
+                const float *rho = maps[m].d_rho;
+                const float cp = eff_pos(maps[m].cut_pos), cn = eff_neg(maps[m].cut_neg);
+                const int mode = g.map2xyz[2] == 1 ? 0 : (g.map2xyz[2] == 2 ? 1 : 2);  // z_axis_mode, warp-uniform
+                bool done;
+                if (mode == 0)
+                    done = quad_sums<0>(g, rho, s1, a0, xyz, radius, cp, cn, stab[warp], lane, out);
+                else if (mode == 1)
+                    done = quad_sums<1>(g, rho, s1, a0, xyz, radius, cp, cn, stab[warp], lane, out);
+                else
+                    done = quad_sums<2>(g, rho, s1, a0, xyz, radius, cp, cn, stab[warp], lane, out);
+                if (done) continue;
+            }
+            for (int a = a0; a < min(a0 + kAtomsPerWarp, s1); ++a) {
+                const int ma = group_map[a];
+                if (!sums_map_ok(ma, n_maps, maps)) {
+                    if (lane < PE_SPHERE_NOUT) out[(int64_t)a * PE_SPHERE_NOUT + lane] = __longlong_as_double(0x7ff8000000000000ll);
+                    continue;
+                }
+                copy_geom(g, maps[ma].geom, lane);
+                const float *rho = maps[ma].d_rho;
+                const float cp = eff_pos(maps[ma].cut_pos), cn = eff_neg(maps[ma].cut_neg);
+                const int mode = g.map2xyz[2] == 1 ? 0 : (g.map2xyz[2] == 2 ? 1 : 2);
+                if (mode == 0)
+                    sums_one_atom<0>(g, rho, a, xyz, radius, cp, cn, tabs[warp], lane, out);
+                else if (mode == 1)
+                    sums_one_atom<1>(g, rho, a, xyz, radius, cp, cn, tabs[warp], lane, out);
+                else
+                    sums_one_atom<2>(g, rho, a, xyz, radius, cp, cn, tabs[warp], lane, out);
+            }
+        }
+        q_base += nq;
+    }
 }
 
 // ------------------------------------------------------------------------------------------------ list kernels
@@ -393,6 +468,33 @@ int pe_sphere_sums_atoms_and_groups(const pe_geom *g, const float *d_rho, int32_
     if (int rc = pe_sphere_sums(g, d_rho, n_atoms, d_xyz, d_atom_radius, n_atoms, nullptr, cut_pos, cut_neg, d_out_atoms, d_ws, stream))
         return rc;
     return pe_sphere_sums(g, d_rho, n_atoms, d_xyz, d_group_radius, n_groups, d_group_start, cut_pos, cut_neg, d_out_groups, d_ws, stream);
+}
+
+int64_t pe_batch_sphere_sums_workspace_bytes(int64_t n_atoms) { return SphereWs::bytes(n_atoms < 0 ? 0 : n_atoms); }
+
+int pe_batch_sphere_sums(int32_t n_maps, const pe_sums_map *d_maps, int32_t n_atoms, const double *d_xyz, const float *d_radius,
+                         int32_t n_groups, const int32_t *d_group_map, const int32_t *d_group_start, const int32_t *d_atom_start,
+                         double *d_out, void *d_ws, void *stream) {
+    PE_CHECK_ARG(n_maps >= 0 && n_atoms >= 0 && n_groups >= 0, "pe_batch_sphere_sums: negative size");
+    if (n_groups == 0) return PE_OK;
+    PE_CHECK_ARG(n_maps > 0, "pe_batch_sphere_sums: groups without maps");
+    PE_CHECK_ARG(d_maps && d_xyz && d_radius && d_group_map && d_out && d_ws, "pe_batch_sphere_sums: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (d_group_start == nullptr) {
+        PE_CHECK_ARG(n_groups == n_atoms, "pe_batch_sphere_sums: n_groups must equal n_atoms without group offsets");
+        PE_CHECK_ARG(d_atom_start != nullptr, "pe_batch_sphere_sums: per-atom sums need d_atom_start");
+        // every structure adds at most one partial quad; the warps stride over the quads, so the grid only sets the parallelism
+        const int64_t quads = (int64_t)n_atoms / kAtomsPerWarp + n_maps;
+        int64_t blocks = (quads + kSphereWarps - 1) / kSphereWarps;
+        const int64_t max_blocks = (int64_t)sm_count() * 16;
+        if (blocks > max_blocks) blocks = max_blocks;
+        PE_LAUNCH("batch_sphere_sums_kernel", st, batch_sphere_sums_kernel<<<(int)blocks, kSphereWarps * 32, 0, st>>>(
+            n_maps, d_maps, d_atom_start, d_group_map, d_xyz, d_radius, d_out));
+        PE_LAUNCH_CHECK();
+        return PE_OK;
+    }
+    const SphereWs ws(d_ws, n_atoms);
+    return launch_batch_union(n_maps, d_maps, n_groups, d_group_map, d_group_start, d_xyz, d_radius, ws.box, ws.thr, ws.counter, d_out, st);
 }
 
 int pe_sphere_count(const pe_geom *g, const float *d_rho, int32_t n_atoms, const double *d_xyz, const float *d_radius,

@@ -31,16 +31,35 @@ namespace pe {
 // read through pe_sphere_union_warp_cycles(): 0 boxes + bounding box, 1 tile offsets + per-atom tables, 2 membership, 3 gather,
 // 4 reduction + output.
 __device__ unsigned long long g_union_warp_cycles[5];
+// The clock of one warp's phases, carried through the work items (every member is empty in the normal build).
+struct PhaseClock {
 #if PE_UNION_PHASE_CYCLES
-#define PHASE_MARK(k)                              \
-    do {                                           \
-        const long long now__ = clock64();         \
-        t_phase[k] += now__ - t_mark;              \
-        t_mark = now__;                            \
-    } while (0)
+    long long mark, t[5];
+    // clock64 only exists in the device pass; the host pass parses these bodies as well
+    __device__ __forceinline__ static long long now() {
+#ifdef __CUDA_ARCH__
+        return clock64();
 #else
-#define PHASE_MARK(k) do { } while (0)
+        return 0;
 #endif
+    }
+    __device__ __forceinline__ PhaseClock() : mark(now()), t{0, 0, 0, 0, 0} {}
+    __device__ __forceinline__ void lap(int k) {
+        const long long now = PhaseClock::now();
+        t[k] += now - mark;
+        mark = now;
+    }
+    __device__ __forceinline__ void flush(int lane) {
+        if (lane == 0) {
+#pragma unroll
+            for (int k = 0; k < 5; ++k) atomicAdd(g_union_warp_cycles + k, (unsigned long long)t[k]);
+        }
+    }
+#else
+    __device__ __forceinline__ void lap(int) {}
+    __device__ __forceinline__ void flush(int) {}
+#endif
+};
 
 constexpr int kUW = 4;        // warps per CTA
 constexpr int kUT = 32;       // tile edge
@@ -177,6 +196,139 @@ __device__ __forceinline__ void gather_tile(WarpUnion &w, const float *__restric
     }
 }
 
+// One group of atoms [a0, a1) by one warp, from the atom boxes to the output row o (PE_SPHERE_NOUT values, written by lane 0).
+// The list capacity kUList, kULoads and the short-list rule of gather_tile fix the summation order, so every kernel that calls
+// this gives a group the same bits.  Leaves w.bits clear.  cp / cn: effective cutoffs; icx / inv_gl: the column axis' xyz axis
+// and its inverse grid length.
+template <int MODE>
+__device__ __forceinline__ void union_group(WarpUnion &w, const pe_geom &g, const float *__restrict__ rho, int a0, int a1,
+                                            const double *__restrict__ xyz, const float *__restrict__ radius, int32_t *box,
+                                            double *thr, float cp, float cn, bool has_neg, int icx, float inv_gl, int lane,
+                                            double *__restrict__ o, PhaseClock &clk) {
+    // boxes and thresholds of the group's atoms (lanes over atoms), bounding box by warp reductions
+    int ulo0 = INT_MAX, ulo1 = INT_MAX, ulo2 = INT_MAX, uhi0 = INT_MIN, uhi1 = INT_MIN, uhi2 = INT_MIN;
+    double candidates = 0.0;
+    for (int a = a0 + lane; a < a1; a += 32) {
+        AtomBox bb;
+        double tt;
+        atom_box(g, xyz[3 * a], xyz[3 * a + 1], xyz[3 * a + 2], radius[a], bb, tt);
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            box[6 * a + k] = bb.lo[k];
+            box[6 * a + 3 + k] = bb.dim[k];
+        }
+        thr[a] = tt;
+        candidates += (double)bb.dim[0] * (double)bb.dim[1] * (double)bb.dim[2];
+        if (bb.dim[0] > 0 && bb.dim[1] > 0 && bb.dim[2] > 0) {
+            ulo0 = min(ulo0, bb.lo[0]);
+            ulo1 = min(ulo1, bb.lo[1]);
+            ulo2 = min(ulo2, bb.lo[2]);
+            uhi0 = max(uhi0, bb.lo[0] + bb.dim[0]);
+            uhi1 = max(uhi1, bb.lo[1] + bb.dim[1]);
+            uhi2 = max(uhi2, bb.lo[2] + bb.dim[2]);
+        }
+    }
+    __syncwarp();  // boxes visible to the whole warp
+    candidates = warp_sum(candidates);
+    ulo0 = warp_min(ulo0);
+    ulo1 = warp_min(ulo1);
+    ulo2 = warp_min(ulo2);
+    uhi0 = warp_max(uhi0);
+    uhi1 = warp_max(uhi1);
+    uhi2 = warp_max(uhi2);
+    SphereAcc acc;
+    clk.lap(0);
+    if (uhi0 > ulo0) {
+        for (int ts0 = ulo2; ts0 < uhi2; ts0 += kUT)
+            for (int tr0 = ulo1; tr0 < uhi1; tr0 += kUT)
+                for (int tc0 = ulo0; tc0 < uhi0; tc0 += kUT) {
+                    const int tC = min(kUT, uhi0 - tc0), tR = min(kUT, uhi1 - tr0), tS = min(kUT, uhi2 - ts0);
+                    // wrapped element offsets of the tile's indices; is every index stored and are the columns adjacent?
+                    int invalid = 0;
+                    {
+                        const int oc = lane < tC ? axis_off(g, 0, tc0 + lane) : 0;
+                        const int orw = lane < tR ? axis_off(g, 1, tr0 + lane) : 0;
+                        const int os = lane < tS ? axis_off(g, 2, ts0 + lane) : 0;
+                        w.offC[lane] = oc;
+                        w.offR[lane] = orw;
+                        w.offS[lane] = os;
+                        invalid = (oc | orw | os) < 0 ? 1 : 0;
+                        const int prev = __shfl_up_sync(kFull, oc, 1);
+                        if (lane > 0 && lane < tC && oc != prev + 1) invalid = 1;
+                    }
+                    const bool checked = __any_sync(kFull, invalid != 0);
+                    // membership, atom by atom
+                    for (int a = a0; a < a1; ++a) {
+                        const int32_t *bx = box + 6 * a;
+                        const int b0 = bx[0], b1 = bx[1], b2 = bx[2], d0 = bx[3], d1 = bx[4], d2 = bx[5];
+                        if (d0 <= 0 || d1 <= 0 || d2 <= 0) continue;
+                        const int cl = max(b0, tc0), ch = min(b0 + d0, tc0 + tC);
+                        const int rl = max(b1, tr0), rh = min(b1 + d1, tr0 + tR);
+                        const int sl = max(b2, ts0), sh = min(b2 + d2, ts0 + tS);
+                        if (cl >= ch || rl >= rh || sl >= sh) continue;
+                        const double ax = xyz[3 * a], ay = xyz[3 * a + 1], az = xyz[3 * a + 2];
+                        const double T = thr[a];
+                        if (g.orthogonal) {
+                            const int nC = ch - cl, nR = rh - rl, nS = sh - sl;
+                            if (lane < nC) w.sqC[lane] = axis_sq(g, 0, cl + lane, ax, ay, az);
+                            if (lane < nR) w.sqR[lane] = axis_sq(g, 1, rl + lane, ax, ay, az);
+                            if (lane < nS) w.sqS[lane] = axis_sq(g, 2, sl + lane, ax, ay, az);
+                            __syncwarp();
+                            clk.lap(1);
+                            // centre column of the box (range(c - R - 1, c + R + 1): c = lo + dim / 2), clamped into the tile part
+                            const int kmin = min(max(b0 + d0 / 2 - cl, 0), nC - 1);
+                            const float xc = (float)((sel3(ax, ay, az, icx) - g.origin[icx]) / g.grid_length[icx] - (double)cl);
+                            mark_atom<MODE>(w.bits, w.sqC, w.sqR, w.sqS, lane, cl - tc0, nC, rl - tr0, nR, sl - ts0, nS, T, xc, inv_gl,
+                                            kmin);
+                            __syncwarp();  // tables are rewritten by the next atom; its rows may share words with this one
+                            clk.lap(2);
+                        } else {
+                            const int nc = ch - cl, n1 = rh - rl;
+                            const int vol = nc * n1 * (sh - sl);
+                            for (int m = lane; m < vol; m += 32) {
+                                const int ic = m % nc, t = m / nc;
+                                const int c = cl + ic, r = rl + t % n1, s = sl + t / n1;
+                                double vx, vy, vz;
+                                crs2xyz(g, c, r, s, vx, vy, vz);
+                                if (!(dist2(ax, ay, az, vx, vy, vz) <= T)) continue;
+                                atomicOr(&w.bits[(r - tr0) * kUT + (s - ts0)], 1u << (c - tc0));
+                            }
+                            __syncwarp();
+                        }
+                    }
+                    // gather every voxel of the union once
+                    clk.lap(1);
+                    if (checked) {
+                        if (has_neg)
+                            gather_tile<true, true>(w, rho, acc, cp, cn, lane, tR, tS);
+                        else
+                            gather_tile<true, false>(w, rho, acc, cp, cn, lane, tR, tS);
+                    } else {
+                        if (has_neg)
+                            gather_tile<false, true>(w, rho, acc, cp, cn, lane, tR, tS);
+                        else
+                            gather_tile<false, false>(w, rho, acc, cp, cn, lane, tR, tS);
+                    }
+                    __syncwarp();
+                    clk.lap(3);
+                }
+    }
+    const int n_all = warp_sum(acc.n_all), n_pos = warp_sum(acc.n_pos), n_neg = warp_sum(acc.n_neg);
+    const int bad = warp_sum(acc.bad);
+    const double s_all = warp_sum(acc.s_all), s_pos = warp_sum(acc.s_pos), s_neg = warp_sum(acc.s_neg);
+    if (lane == 0) {
+        o[0] = (double)n_all;
+        o[1] = s_all;
+        o[2] = (double)n_pos;
+        o[3] = s_pos;
+        o[4] = (double)n_neg;
+        o[5] = s_neg;
+        o[6] = bad ? 0.0 : 1.0;
+        o[7] = candidates;
+    }
+    clk.lap(4);
+}
+
 // Work items, handed out in order through one counter: [0, n_groups) are groups (the long items), then, when n_quad_atoms > 0,
 // one item per quad of atoms [4q, 4q + 4) summed at atom_radius into out_atoms (quad_sums: the short items fill the SMs that
 // the last groups would leave idle).  The host hands atoms over only when every box at atom_radius is at most kSmallDim wide;
@@ -198,10 +350,7 @@ __global__ void __launch_bounds__(kUW * 32, kUCtas)
     const float inv_gl = (float)(1.0 / g.grid_length[icx]);
     for (int i = lane; i < kUT * kUT; i += 32) w.bits[i] = 0u;  // cleared once: the gather leaves it clear
     __syncwarp();
-#if PE_UNION_PHASE_CYCLES
-    long long t_mark = clock64();
-    long long t_phase[5] = {0, 0, 0, 0, 0};
-#endif
+    PhaseClock clk;
     const int n_items = n_groups + (n_quad_atoms + kAtomsPerWarp - 1) / kAtomsPerWarp;
     for (;;) {
         int item = 0;
@@ -216,137 +365,10 @@ __global__ void __launch_bounds__(kUW * 32, kUCtas)
             continue;
         }
         const int grp = item;
-        const int a0 = group_start[grp], a1 = group_start[grp + 1];
-        // boxes and thresholds of the group's atoms (lanes over atoms), bounding box by warp reductions
-        int ulo0 = INT_MAX, ulo1 = INT_MAX, ulo2 = INT_MAX, uhi0 = INT_MIN, uhi1 = INT_MIN, uhi2 = INT_MIN;
-        double candidates = 0.0;
-        for (int a = a0 + lane; a < a1; a += 32) {
-            AtomBox bb;
-            double tt;
-            atom_box(g, xyz[3 * a], xyz[3 * a + 1], xyz[3 * a + 2], radius[a], bb, tt);
-#pragma unroll
-            for (int k = 0; k < 3; ++k) {
-                box[6 * a + k] = bb.lo[k];
-                box[6 * a + 3 + k] = bb.dim[k];
-            }
-            thr[a] = tt;
-            candidates += (double)bb.dim[0] * (double)bb.dim[1] * (double)bb.dim[2];
-            if (bb.dim[0] > 0 && bb.dim[1] > 0 && bb.dim[2] > 0) {
-                ulo0 = min(ulo0, bb.lo[0]);
-                ulo1 = min(ulo1, bb.lo[1]);
-                ulo2 = min(ulo2, bb.lo[2]);
-                uhi0 = max(uhi0, bb.lo[0] + bb.dim[0]);
-                uhi1 = max(uhi1, bb.lo[1] + bb.dim[1]);
-                uhi2 = max(uhi2, bb.lo[2] + bb.dim[2]);
-            }
-        }
-        __syncwarp();  // boxes visible to the whole warp
-        candidates = warp_sum(candidates);
-        ulo0 = warp_min(ulo0);
-        ulo1 = warp_min(ulo1);
-        ulo2 = warp_min(ulo2);
-        uhi0 = warp_max(uhi0);
-        uhi1 = warp_max(uhi1);
-        uhi2 = warp_max(uhi2);
-        SphereAcc acc;
-        PHASE_MARK(0);
-        if (uhi0 > ulo0) {
-            for (int ts0 = ulo2; ts0 < uhi2; ts0 += kUT)
-                for (int tr0 = ulo1; tr0 < uhi1; tr0 += kUT)
-                    for (int tc0 = ulo0; tc0 < uhi0; tc0 += kUT) {
-                        const int tC = min(kUT, uhi0 - tc0), tR = min(kUT, uhi1 - tr0), tS = min(kUT, uhi2 - ts0);
-                        // wrapped element offsets of the tile's indices; is every index stored and are the columns adjacent?
-                        int invalid = 0;
-                        {
-                            const int oc = lane < tC ? axis_off(g, 0, tc0 + lane) : 0;
-                            const int orw = lane < tR ? axis_off(g, 1, tr0 + lane) : 0;
-                            const int os = lane < tS ? axis_off(g, 2, ts0 + lane) : 0;
-                            w.offC[lane] = oc;
-                            w.offR[lane] = orw;
-                            w.offS[lane] = os;
-                            invalid = (oc | orw | os) < 0 ? 1 : 0;
-                            const int prev = __shfl_up_sync(kFull, oc, 1);
-                            if (lane > 0 && lane < tC && oc != prev + 1) invalid = 1;
-                        }
-                        const bool checked = __any_sync(kFull, invalid != 0);
-                        // membership, atom by atom
-                        for (int a = a0; a < a1; ++a) {
-                            const int32_t *bx = box + 6 * a;
-                            const int b0 = bx[0], b1 = bx[1], b2 = bx[2], d0 = bx[3], d1 = bx[4], d2 = bx[5];
-                            if (d0 <= 0 || d1 <= 0 || d2 <= 0) continue;
-                            const int cl = max(b0, tc0), ch = min(b0 + d0, tc0 + tC);
-                            const int rl = max(b1, tr0), rh = min(b1 + d1, tr0 + tR);
-                            const int sl = max(b2, ts0), sh = min(b2 + d2, ts0 + tS);
-                            if (cl >= ch || rl >= rh || sl >= sh) continue;
-                            const double ax = xyz[3 * a], ay = xyz[3 * a + 1], az = xyz[3 * a + 2];
-                            const double T = thr[a];
-                            if (g.orthogonal) {
-                                const int nC = ch - cl, nR = rh - rl, nS = sh - sl;
-                                if (lane < nC) w.sqC[lane] = axis_sq(g, 0, cl + lane, ax, ay, az);
-                                if (lane < nR) w.sqR[lane] = axis_sq(g, 1, rl + lane, ax, ay, az);
-                                if (lane < nS) w.sqS[lane] = axis_sq(g, 2, sl + lane, ax, ay, az);
-                                __syncwarp();
-                                PHASE_MARK(1);
-                                // centre column of the box (range(c - R - 1, c + R + 1): c = lo + dim / 2), clamped into the tile part
-                                const int kmin = min(max(b0 + d0 / 2 - cl, 0), nC - 1);
-                                const float xc = (float)((sel3(ax, ay, az, icx) - g.origin[icx]) / g.grid_length[icx] - (double)cl);
-                                mark_atom<MODE>(w.bits, w.sqC, w.sqR, w.sqS, lane, cl - tc0, nC, rl - tr0, nR, sl - ts0, nS, T, xc, inv_gl,
-                                                kmin);
-                                __syncwarp();  // tables are rewritten by the next atom; its rows may share words with this one
-                                PHASE_MARK(2);
-                            } else {
-                                const int nc = ch - cl, n1 = rh - rl;
-                                const int vol = nc * n1 * (sh - sl);
-                                for (int m = lane; m < vol; m += 32) {
-                                    const int ic = m % nc, t = m / nc;
-                                    const int c = cl + ic, r = rl + t % n1, s = sl + t / n1;
-                                    double vx, vy, vz;
-                                    crs2xyz(g, c, r, s, vx, vy, vz);
-                                    if (!(dist2(ax, ay, az, vx, vy, vz) <= T)) continue;
-                                    atomicOr(&w.bits[(r - tr0) * kUT + (s - ts0)], 1u << (c - tc0));
-                                }
-                                __syncwarp();
-                            }
-                        }
-                        // gather every voxel of the union once
-                        PHASE_MARK(1);
-                        if (checked) {
-                            if (has_neg)
-                                gather_tile<true, true>(w, rho, acc, cp, cn, lane, tR, tS);
-                            else
-                                gather_tile<true, false>(w, rho, acc, cp, cn, lane, tR, tS);
-                        } else {
-                            if (has_neg)
-                                gather_tile<false, true>(w, rho, acc, cp, cn, lane, tR, tS);
-                            else
-                                gather_tile<false, false>(w, rho, acc, cp, cn, lane, tR, tS);
-                        }
-                        __syncwarp();
-                        PHASE_MARK(3);
-                    }
-        }
-        const int n_all = warp_sum(acc.n_all), n_pos = warp_sum(acc.n_pos), n_neg = warp_sum(acc.n_neg);
-        const int bad = warp_sum(acc.bad);
-        const double s_all = warp_sum(acc.s_all), s_pos = warp_sum(acc.s_pos), s_neg = warp_sum(acc.s_neg);
-        if (lane == 0) {
-            double *o = out + (int64_t)grp * PE_SPHERE_NOUT;
-            o[0] = (double)n_all;
-            o[1] = s_all;
-            o[2] = (double)n_pos;
-            o[3] = s_pos;
-            o[4] = (double)n_neg;
-            o[5] = s_neg;
-            o[6] = bad ? 0.0 : 1.0;
-            o[7] = candidates;
-        }
-        PHASE_MARK(4);
+        union_group<MODE>(w, g, rho, group_start[grp], group_start[grp + 1], xyz, radius, box, thr, cp, cn, has_neg, icx, inv_gl, lane,
+                          out + (int64_t)grp * PE_SPHERE_NOUT, clk);
     }
-#if PE_UNION_PHASE_CYCLES
-    if (lane == 0) {
-#pragma unroll
-        for (int k = 0; k < 5; ++k) atomicAdd(g_union_warp_cycles + k, (unsigned long long)t_phase[k]);
-    }
-#endif
+    clk.flush(lane);
 }
 
 int launch_union_warp(const pe_geom *g, const float *d_rho, int n_groups, const int32_t *d_group_start, const double *d_xyz,
@@ -370,6 +392,79 @@ int launch_union_warp(const pe_geom *g, const float *d_rho, int n_groups, const 
         PE_LAUNCH("sphere_union_kernel", st, sphere_union_warp_kernel<2><<<grid, kUW * 32, 0, st>>>(
             *g, d_rho, n_groups, d_group_start, d_xyz, d_radius, box, thr, cut_pos, cut_neg, d_counter, d_out,
             n_quad_atoms, d_atom_radius, d_out_atoms));
+    PE_LAUNCH_CHECK();
+    return PE_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ groups of many structures
+// The groups of a whole batch, each on its own map (pe_batch_sphere_sums, grouped form): the work item of
+// sphere_union_warp_kernel (union_group) with the geometry, map and cutoffs read from the group's table entry.  A warp keeps
+// its group's pe_geom in shared memory next to its WarpUnion, which leaves room for 6 CTAs per SM instead of 7; the order of
+// the sums does not depend on the occupancy, so a group's row is the bits sphere_union_warp_kernel gives it.
+constexpr int kUBatchCtas = 6;
+struct WarpUnionGeom {
+    WarpUnion u;
+    pe_geom geom;  // the current group's map geometry
+};
+static_assert(kUBatchCtas * (kUW * sizeof(WarpUnionGeom) + 1024) <= 228 * 1024, "kUBatchCtas CTAs per SM do not fit the shared memory");
+
+__global__ void __launch_bounds__(kUW * 32, kUBatchCtas)
+    batch_union_kernel(int n_maps, const pe_sums_map *__restrict__ maps, int n_groups, const int32_t *__restrict__ group_map,
+                       const int32_t *__restrict__ group_start, const double *__restrict__ xyz, const float *__restrict__ radius,
+                       int32_t *box, double *thr, int *__restrict__ counter, double *__restrict__ out /* n_groups x PE_SPHERE_NOUT */) {
+    __shared__ WarpUnionGeom wsh[kUW];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    WarpUnion &w = wsh[warp].u;
+    for (int i = lane; i < kUT * kUT; i += 32) w.bits[i] = 0u;  // cleared once: the gather leaves it clear
+    __syncwarp();
+    PhaseClock clk;
+    for (;;) {
+        int item = 0;
+        if (lane == 0) item = atomicAdd(counter, 1);
+        item = __shfl_sync(kFull, item, 0);
+        if (item >= n_groups) break;
+        const int grp = item;
+        double *o = out + (int64_t)grp * PE_SPHERE_NOUT;
+        const int m = group_map[grp];
+        const bool bad_map = m < 0 || m >= n_maps;
+        float cp = bad_map ? 0.f : maps[m].cut_pos, cn = bad_map ? 0.f : maps[m].cut_neg;
+        if (bad_map || cp < 0.f || cn > 0.f) {  // a group on no valid entry of the table: NaN, so that it cannot pass for a result
+            if (lane < PE_SPHERE_NOUT) o[lane] = __longlong_as_double(0x7ff8000000000000ll);
+            continue;
+        }
+        static_assert(sizeof(pe_geom) % 4 == 0, "pe_geom is copied as 32-bit words");
+        for (int i = lane; i < (int)(sizeof(pe_geom) / 4); i += 32)
+            reinterpret_cast<int *>(&wsh[warp].geom)[i] = reinterpret_cast<const int *>(&maps[m].geom)[i];
+        __syncwarp();
+        const pe_geom &g = wsh[warp].geom;
+        const float *rho = maps[m].d_rho;
+        cp = eff_pos(cp);
+        cn = eff_neg(cn);
+        const bool has_neg = cn > __int_as_float(0xff800000);
+        const int icx = g.map2crs[0];
+        const float inv_gl = (float)(1.0 / g.grid_length[icx]);
+        const int a0 = group_start[grp], a1 = group_start[grp + 1];
+        const int mode = g.map2xyz[2] == 1 ? 0 : (g.map2xyz[2] == 2 ? 1 : 2);  // z_axis_mode, warp-uniform
+        if (mode == 0)
+            union_group<0>(w, g, rho, a0, a1, xyz, radius, box, thr, cp, cn, has_neg, icx, inv_gl, lane, o, clk);
+        else if (mode == 1)
+            union_group<1>(w, g, rho, a0, a1, xyz, radius, box, thr, cp, cn, has_neg, icx, inv_gl, lane, o, clk);
+        else
+            union_group<2>(w, g, rho, a0, a1, xyz, radius, box, thr, cp, cn, has_neg, icx, inv_gl, lane, o, clk);
+        __syncwarp();  // the geometry is rewritten by the next group
+    }
+    clk.flush(lane);
+}
+
+int launch_batch_union(int n_maps, const pe_sums_map *d_maps, int n_groups, const int32_t *d_group_map, const int32_t *d_group_start,
+                       const double *d_xyz, const float *d_radius, int32_t *box, double *thr, int *d_counter, double *d_out,
+                       cudaStream_t st) {
+    PE_CUDA(cudaMemsetAsync(d_counter, 0, sizeof(int), st));
+    int grid = (n_groups + kUW - 1) / kUW;
+    const int max_grid = sm_count() * kUBatchCtas;
+    if (grid > max_grid) grid = max_grid;
+    PE_LAUNCH("batch_union_kernel", st, batch_union_kernel<<<grid, kUW * 32, 0, st>>>(
+        n_maps, d_maps, n_groups, d_group_map, d_group_start, d_xyz, d_radius, box, thr, d_counter, d_out));
     PE_LAUNCH_CHECK();
     return PE_OK;
 }

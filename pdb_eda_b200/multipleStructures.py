@@ -12,8 +12,9 @@ DIR/pdb<id>.ent(.gz) instead of downloading.  Result: per-entry ``stats`` and ``
 --single-mode runs a ``single`` submode on every entry (the reference's ``multiple --single-mode``): "<single options>" are
 the options of ``single`` after <pdbid> <out-file>, e.g. "statistics --residue --out-format csv --include-pdbid", and every
 entry's result goes to <out-dir>/<pdbid>.result in the schema ``single`` writes.  ``statistics --residue`` / ``--atom`` runs
-batched on the device (``multi.runMultipleMetrics``; with --print-validation, entry by entry); every other submode runs
-``single`` entry by entry on the rank that owns the entry.  Entries are sharded over the ranks and every rank writes the
+batched on the device (``multi.runMultipleMetrics``; with --print-validation, entry by entry), and so do ``density`` and
+``difference`` with --atom / --residue / --symmetry-atom and all their options (``regionBatch``: the region sums of a batch in
+one launch); ``map``, ``cloud`` and ``blob`` run ``single`` entry by entry on the rank that owns the entry.  Entries are sharded over the ranks and every rank writes the
 files of its own entries; the summary line (entries ok / failed, rows) is printed by rank 0.
 """
 import argparse
@@ -126,13 +127,59 @@ def _entryArgs(single, pdbid, outDir, dataDir):
     return a
 
 
+def batchedPath(single):
+    """Which batched path runs the ``--single-mode`` options ``single`` on the device: "metrics" (``statistics --residue`` /
+    ``--atom`` without --print-validation), "region" (``density`` / ``difference``), or None (``single`` entry by entry)."""
+    if single.submode == "statistics" and not single.print_validation:
+        return "metrics"
+    if single.submode in ("density", "difference"):
+        return "region"
+    return None
+
+
+_regionHeaders = {("density", "atom"): "atomRegionDensityHeader", ("density", "residue"): "residueRegionDensityHeader",
+                  ("density", "symmetry-atom"): "symmetryAtomRegionDensityHeader",
+                  ("difference", "atom"): "atomRegionDiscrepancyHeader", ("difference", "residue"): "residueRegionDiscrepancyHeader",
+                  ("difference", "symmetry-atom"): "symmetryAtomRegionDiscrepancyHeader"}
+
+
+def _runRegions(ids, outDir, single, dataDir, costs, group):
+    """``density`` / ``difference`` of every entry through ``regionBatch`` (the rows, options and failures of ``single``)."""
+    from . import regionBatch
+    level = "atom" if single.atom else ("residue" if single.residue else "symmetry-atom")
+    loader = makeLoader(dataDir)
+    atomMask = None
+    try:
+        if single.params:
+            densityAnalysis.setGlobals(singleStructure._loadJson(single.params, "params"))
+        if single.atom_mask:
+            atomMask = singleStructure._loadJson(single.atom_mask, "atom mask")
+    except RuntimeError:
+        loader = lambda pdbid: 0                 # single fails on every entry: so does every entry here
+    options = dict(radius=single.radius, numSD=singleStructure.numSDOf(single), type=single.type, atomMask=atomMask,
+                   useOptimizedRadii=single.optimized_radii)
+    header = getattr(densityAnalysis.DensityAnalysis, _regionHeaders[(single.submode, level)])
+
+    def stream(pairs, maxBytes, device):
+        return regionBatch.analyzeStream(pairs, single.submode, level, maxBytes, device, **options)
+
+    def write(idx, rows):
+        a = _entryArgs(single, ids[idx], outDir, dataDir)
+        singleStructure.writeResult(a, *singleStructure.regionResult(a, header, rows, ids[idx]))
+
+    return multi.runMultipleMetrics(ids, loader, None, costs=costs, write=write, group=group, stream=stream)
+
+
 def runSingleMode(ids, outDir, single, dataDir="", group=None):
     """``single`` with the options ``single`` (``parseSingleMode``) on every entry of ``ids``; this rank writes the result files
     of its own entries.  Returns the all-reduced counts of ``multi.summarizeMetrics`` (entries ok / failed, rows)."""
     os.makedirs(outDir, exist_ok=True)
     sizeOf = lambda path: os.path.getsize(path) if os.path.isfile(path) else 0
     costs = [sizeOf(os.path.join(dataDir, i + ".ccp4")) + 1 for i in ids] if dataDir else None     # longest first
-    if single.submode == "statistics" and not single.print_validation:
+    batched = batchedPath(single)
+    if batched == "region":
+        return _runRegions(ids, outDir, single, dataDir, costs, group)
+    if batched == "metrics":
         level = "residue" if single.residue else "atom"
 
         def write(idx, rows):

@@ -65,9 +65,7 @@ def _loadJson(path, what):
 
 def analyze(args):
     """Returns (headerList, rows) of the requested submode."""
-    numSD = args.num_sd
-    if numSD is None:
-        numSD = 3.0 if (args.green or args.red or args.submode == "difference") else 1.5
+    numSD = numSDOf(args)
     if args.params:
         densityAnalysis.setGlobals(_loadJson(args.params, "params"))
     atomMask = _loadJson(args.atom_mask, "atom mask") if args.atom_mask else None
@@ -98,7 +96,6 @@ def analyze(args):
         else:
             header, rows = DA.domainCloudHeader + ['density_electron_ratio'], [list(i) + [ratio] for i in analyzer.domainCloudDescriptions]
     elif sub in ("density", "difference"):
-        symmetry = args.symmetry_atom
         if sub == "density":
             if args.atom:
                 header, rows = DA.atomRegionDensityHeader, analyzer.calculateAtomRegionDensity(args.radius, numSD, args.type, args.optimized_radii)
@@ -113,10 +110,7 @@ def analyze(args):
                 header, rows = DA.residueRegionDiscrepancyHeader, analyzer.calculateResidueRegionDiscrepancies(args.radius, numSD, args.type, atomMask)
             else:
                 header, rows = DA.symmetryAtomRegionDiscrepancyHeader, analyzer.calculateSymmetryAtomRegionDiscrepancies(args.radius, numSD, args.type)
-        if symmetry:
-            for info in rows:
-                info[5] = [val for val in info[5]]
-                info[6] = [float(val) for val in info[6]]
+        return regionResult(args, header, rows, analyzer.pdbid)
     elif sub == "blob":
         header, rows = DA.blobStatisticsHeader, []
         diff, dens = analyzer.diffDensityObj, analyzer.densityObj
@@ -145,6 +139,26 @@ def analyze(args):
     if args.include_pdbid:
         header = ["pdbid"] + header
         rows = [[analyzer.pdbid] + row for row in rows]
+    return header, rows
+
+
+def numSDOf(args):
+    """--num-sd, or its default: 3.0 for green / red blobs and ``difference``, else 1.5."""
+    if args.num_sd is not None:
+        return args.num_sd
+    return 3.0 if (args.green or args.red or args.submode == "difference") else 1.5
+
+
+def regionResult(args, header, rows, pdbid):
+    """(header, rows) of ``density`` / ``difference`` from the rows of the calculate*Region* calls, as written to the result
+    file."""
+    if args.symmetry_atom:
+        for info in rows:
+            info[5] = [val for val in info[5]]
+            info[6] = [float(val) for val in info[6]]
+    if args.include_pdbid:
+        header = ["pdbid"] + header
+        rows = [[pdbid] + row for row in rows]
     return header, rows
 
 
