@@ -31,6 +31,22 @@ class PeGeom(ctypes.Structure):
     ]
 
 
+class PeBatchMap(ctypes.Structure):
+    """Mirror of ``struct pe_batch_map`` (include/pdbeda_b200.h)."""
+    _fields_ = [("geom", PeGeom), ("d_rho", ctypes.c_void_p), ("cutoff", ctypes.c_float), ("atom_begin", ctypes.c_int32),
+                ("atom_end", ctypes.c_int32), ("reserved", ctypes.c_int32)]
+
+
+class PeSumsMap(ctypes.Structure):
+    """Mirror of ``struct pe_sums_map`` (include/pdbeda_b200.h)."""
+    _fields_ = [("geom", PeGeom), ("d_rho", ctypes.c_void_p), ("cut_pos", ctypes.c_float), ("cut_neg", ctypes.c_float)]
+
+
+class PePairMap(ctypes.Structure):
+    """Mirror of ``struct pe_pair_map`` (include/pdbeda_b200.h)."""
+    _fields_ = [("geom", PeGeom), ("d_fo", ctypes.c_void_p), ("d_diff", ctypes.c_void_p)]
+
+
 class PdbEdaLibError(RuntimeError):
     pass
 

@@ -27,17 +27,11 @@ from scipy import special
 from . import _device
 from . import _lib
 from ._device import _ptr, _stream
-from ._lib import PeGeom, check
+from ._lib import PeBatchMap, check
 from ._gc import pausedGC
 
 MEDIAN_COLUMNS = ("num_voxels", "density_electron_ratio", "centroid_distance", "adj_density_electron_ratio", "volume", "bfactor",
                   "slopes", "domain_fraction", "corrected_fraction", "corrected_density_electron_ratio")
-
-
-class PeBatchMap(ctypes.Structure):
-    """Mirror of ``struct pe_batch_map`` (include/pdbeda_b200.h)."""
-    _fields_ = [("geom", PeGeom), ("d_rho", ctypes.c_void_p), ("cutoff", ctypes.c_float), ("atom_begin", ctypes.c_int32),
-                ("atom_end", ctypes.c_int32), ("reserved", ctypes.c_int32)]
 
 
 class AtomTable:

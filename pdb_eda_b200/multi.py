@@ -379,18 +379,14 @@ def summarizeMetrics(ok, failed, rows, device="cpu", group=None):
     return {"ok": int(counts[0]), "failed": int(counts[1]), "rows": int(counts[2])}
 
 
-def runMultipleMetrics(items, loader, level, costs=None, write=None, device=None, group=None, maxBytes=8 << 30, stream=None):
-    """RSCC / RSR rows (``residueMetrics()`` or ``atomMetrics()``, ``level`` "residue" / "atom") of many entries:
-    ``loader(item)`` returns a DensityAnalysis (or 0); the entries are sharded over the ranks of the default process group
-    longest first, and every rank analyses its share in batches of at most ``maxBytes`` device bytes (both maps + atoms,
-    ``metricsBatch.MetricsBatch``).  Rows are ragged and large, so they are not gathered: ``write(index, rows)`` is called
-    on the owning rank for every entry that yields rows.  An entry that fails to load or on which the single-structure
-    call would raise is counted as failed.  Returns the all-reduced counts (``summarizeMetrics``) on every rank.
-    ``stream(pairs, maxBytes, device)``, when given, replaces the RSCC / RSR batches (``level`` is then not read): it yields
-    (key, rows or None) for every (key, DensityAnalysis) of ``pairs`` in order, e.g. ``regionBatch.analyzeStream``."""
-    from . import metricsBatch
-    if stream is None:
-        stream = lambda pairs, mb, dev: metricsBatch.analyzeStream(pairs, level, mb, dev)
+def runMultipleRows(items, loader, stream, costs=None, write=None, device=None, group=None, maxBytes=8 << 30):
+    """The rows of one single-structure call on many entries: ``loader(item)`` returns a DensityAnalysis (or 0); the entries
+    are sharded over the ranks of the default process group longest first, and every rank takes its share through
+    ``stream(pairs, maxBytes, device)``, which yields (key, rows or None) for every (key, DensityAnalysis) of ``pairs`` in
+    order, in batches of at most ``maxBytes`` device bytes (e.g. ``metricsBatch.analyzeStream``, ``regionBatch.analyzeStream``
+    with the call bound).  Rows are ragged and large, so they are not gathered: ``write(index, rows)`` is called on the
+    owning rank for every entry that yields rows.  An entry that fails to load or on which the single-structure call would
+    raise is counted as failed.  Returns the all-reduced counts (``summarizeMetrics``) on every rank."""
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     costs = [1.0] * len(items) if costs is None else costs

@@ -11,11 +11,12 @@ DIR/pdb<id>.ent(.gz) instead of downloading.  Result: per-entry ``stats`` and ``
 
 --single-mode runs a ``single`` submode on every entry (the reference's ``multiple --single-mode``): "<single options>" are
 the options of ``single`` after <pdbid> <out-file>, e.g. "statistics --residue --out-format csv --include-pdbid", and every
-entry's result goes to <out-dir>/<pdbid>.result in the schema ``single`` writes.  ``statistics --residue`` / ``--atom`` runs
-batched on the device (``multi.runMultipleMetrics``; with --print-validation, entry by entry), and so do ``density`` and
-``difference`` with --atom / --residue / --symmetry-atom and all their options (``regionBatch``: the region sums of a batch in
-one launch); ``map``, ``cloud`` and ``blob`` run ``single`` entry by entry on the rank that owns the entry.  Entries are sharded over the ranks and every rank writes the
-files of its own entries; the summary line (entries ok / failed, rows) is printed by rank 0.
+entry's result goes to <out-dir>/<pdbid>.result in the schema ``single`` writes.  ``statistics --residue`` / ``--atom``
+(``metricsBatch``; with --print-validation, entry by entry) and ``density`` / ``difference`` with --atom / --residue /
+--symmetry-atom and all their options (``regionBatch``) run batched on the device through ``multi.runMultipleRows``: the
+groups of a batch of entries in one launch, with the rows, options and failures of ``single``.  ``map``, ``cloud`` and
+``blob`` run ``single`` entry by entry on the rank that owns the entry.  Entries are sharded over the ranks and every rank
+writes the files of its own entries; the summary line (entries ok / failed, rows) is printed by rank 0.
 """
 import argparse
 import csv
@@ -29,7 +30,7 @@ import sys
 import torch
 import torch.distributed as dist
 
-from . import densityAnalysis, multi, singleStructure
+from . import densityAnalysis, metricsBatch, multi, regionBatch, singleStructure
 
 statsHeaders = ['density_electron_ratio', 'voxel_volume', 'num_voxels_aggregated', 'total_aggregated_electrons', 'num_atoms_analyzed',
                 'num_residue_clouds_analyzed', 'num_domain_clouds_analyzed', 'atom_overlap_completeness']
@@ -143,31 +144,41 @@ _regionHeaders = {("density", "atom"): "atomRegionDensityHeader", ("density", "r
                   ("difference", "symmetry-atom"): "symmetryAtomRegionDiscrepancyHeader"}
 
 
-def _runRegions(ids, outDir, single, dataDir, costs, group):
-    """``density`` / ``difference`` of every entry through ``regionBatch`` (the rows, options and failures of ``single``)."""
-    from . import regionBatch
-    level = "atom" if single.atom else ("residue" if single.residue else "symmetry-atom")
+def _runBatched(ids, outDir, single, dataDir, costs, group):
+    """``single`` of every entry through the batched path of ``batchedPath(single)``: the rows, options and failures of
+    ``single``, written as ``single`` writes them."""
     loader = makeLoader(dataDir)
     atomMask = None
-    try:
+    try:                                         # what singleStructure.analyze loads before it reads the entry
         if single.params:
             densityAnalysis.setGlobals(singleStructure._loadJson(single.params, "params"))
         if single.atom_mask:
             atomMask = singleStructure._loadJson(single.atom_mask, "atom mask")
     except RuntimeError:
         loader = lambda pdbid: 0                 # single fails on every entry: so does every entry here
-    options = dict(radius=single.radius, numSD=singleStructure.numSDOf(single), type=single.type, atomMask=atomMask,
-                   useOptimizedRadii=single.optimized_radii)
-    header = getattr(densityAnalysis.DensityAnalysis, _regionHeaders[(single.submode, level)])
+    DA = densityAnalysis.DensityAnalysis
+    if batchedPath(single) == "metrics":
+        level = "residue" if single.residue else "atom"
+        header = DA.residueMetricsHeaderList if single.residue else DA.atomMetricsHeaderList
+        result = singleStructure.statisticsResult
 
-    def stream(pairs, maxBytes, device):
-        return regionBatch.analyzeStream(pairs, single.submode, level, maxBytes, device, **options)
+        def stream(pairs, maxBytes, device):
+            return metricsBatch.analyzeStream(pairs, level, maxBytes, device)
+    else:
+        level = "atom" if single.atom else ("residue" if single.residue else "symmetry-atom")
+        header = getattr(DA, _regionHeaders[(single.submode, level)])
+        result = singleStructure.regionResult
+        options = dict(radius=single.radius, numSD=singleStructure.numSDOf(single), type=single.type, atomMask=atomMask,
+                       useOptimizedRadii=single.optimized_radii)
+
+        def stream(pairs, maxBytes, device):
+            return regionBatch.analyzeStream(pairs, single.submode, level, maxBytes, device, **options)
 
     def write(idx, rows):
         a = _entryArgs(single, ids[idx], outDir, dataDir)
-        singleStructure.writeResult(a, *singleStructure.regionResult(a, header, rows, ids[idx]))
+        singleStructure.writeResult(a, *result(a, header, rows, ids[idx]))
 
-    return multi.runMultipleMetrics(ids, loader, None, costs=costs, write=write, group=group, stream=stream)
+    return multi.runMultipleRows(ids, loader, stream, costs=costs, write=write, group=group)
 
 
 def runSingleMode(ids, outDir, single, dataDir="", group=None):
@@ -176,19 +187,8 @@ def runSingleMode(ids, outDir, single, dataDir="", group=None):
     os.makedirs(outDir, exist_ok=True)
     sizeOf = lambda path: os.path.getsize(path) if os.path.isfile(path) else 0
     costs = [sizeOf(os.path.join(dataDir, i + ".ccp4")) + 1 for i in ids] if dataDir else None     # longest first
-    batched = batchedPath(single)
-    if batched == "region":
-        return _runRegions(ids, outDir, single, dataDir, costs, group)
-    if batched == "metrics":
-        level = "residue" if single.residue else "atom"
-
-        def write(idx, rows):
-            header = (densityAnalysis.DensityAnalysis.residueMetricsHeaderList if level == "residue"
-                      else densityAnalysis.DensityAnalysis.atomMetricsHeaderList)
-            a = _entryArgs(single, ids[idx], outDir, dataDir)
-            singleStructure.writeResult(a, *singleStructure.statisticsResult(a, header, rows, ids[idx]))
-
-        return multi.runMultipleMetrics(ids, makeLoader(dataDir), level, costs=costs, write=write, group=group)
+    if batchedPath(single) is not None:
+        return _runBatched(ids, outDir, single, dataDir, costs, group)
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     ok = failed = nrows = 0

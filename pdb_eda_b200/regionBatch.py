@@ -1,49 +1,52 @@
-"""Region density and region discrepancy per atom, residue or symmetry atom for a batch of structures -- ``density`` /
-``difference`` with ``--atom`` / ``--residue`` / ``--symmetry-atom`` of many entries.
+"""Region density and region discrepancy per atom, residue or symmetry atom -- ``density`` / ``difference`` with ``--atom`` /
+``--residue`` / ``--symmetry-atom`` -- of one structure or of a batch of structures.
 
-``DensityAnalysis.calculate*RegionDensity`` / ``calculate*RegionDiscrepancies`` (pdb_eda/densityAnalysis.py:948-1211) analyse
-one structure: the density-electron ratio of its cloud aggregation, one ``pe_sphere_sums`` launch and one read-back.  Here the
-atoms of MANY structures are laid out as one set of arrays (groups -- residues, or single atoms -- in CSR form across
-structures), every structure's map stays where it is in HBM with its own cutoffs (only pointers are gathered into one
-``pe_sums_map`` table), the ratios of the batch come from one ``CloudBatch``, and one launch of ``pe_batch_sphere_sums``
-(csrc/pe_union.cu, csrc/pe_sphere.cu) yields the sums of every group; every row of it is bit-identical to the row
-``pe_sphere_sums`` gives for that structure alone.  The rows are then built with numpy and are the rows, in the order and
-with the types, that the single-structure calls return.
+``makeEntry`` states what the six ``DensityAnalysis.calculate*RegionDensity`` / ``calculate*RegionDiscrepancies`` calls
+(pdb_eda/densityAnalysis.py:948-1211) select and return: the atoms or residues, the ``type`` filter and atom mask, the radii,
+the cutoffs and the row prefixes; ``finish`` turns the sums of its groups into the rows, built with numpy.  Those calls run
+their entry through one ``pe_sphere_sums`` launch.  ``RegionBatch`` runs the entries of MANY structures: their groups laid
+out across structures (``groupBatch``), every structure's map where it is in HBM with its own cutoffs (only pointers are
+gathered into one ``pe_sums_map`` table), the ratios of the batch from one ``CloudBatch``, and one launch of
+``pe_batch_sphere_sums`` (csrc/pe_union.cu, csrc/pe_sphere.cu) for the sums of every group; every row of it is bit-identical
+to the row ``pe_sphere_sums`` gives for that structure alone, so the rows equal those of the single-structure calls in
+value, type and order.
 """
-import ctypes
-
 import numpy as np
 import torch
 
-from . import _device
-from . import _lib
-from . import densityAnalysis
+from . import groupBatch
 from ._device import _ptr, _stream
-from ._lib import PE_SPHERE_NOUT, PeGeom, check
+from ._lib import PE_SPHERE_NOUT, PeSumsMap, check
 
 KINDS = ("density", "difference")
 LEVELS = ("atom", "residue", "symmetry-atom")
-
-
-class PeSumsMap(ctypes.Structure):
-    """Mirror of ``struct pe_sums_map`` (include/pdbeda_b200.h)."""
-    _fields_ = [("geom", PeGeom), ("d_rho", ctypes.c_void_p), ("cut_pos", ctypes.c_float), ("cut_neg", ctypes.c_float)]
 
 
 def _f32(x):
     return float(np.float32(x))
 
 
+def _meanOccupancy(atoms, cache):
+    """np.mean of the atoms' occupancies (pdb_eda/densityAnalysis.py:1031), computed once per distinct occupancy tuple: most
+    residues are all 1.0, and 8,000 np.mean calls on five-element lists cost more than the kernel that follows."""
+    occupancies = tuple([atom.get_occupancy() for atom in atoms])
+    mean = cache.get(occupancies)
+    if mean is None:
+        mean = cache[occupancies] = np.mean(occupancies)
+    return mean
+
+
 # ---------------------------------------------------------------------------------------------------- rows from sums
 def densityRows(sums, ratio):
-    """``_regionDensityRows`` of (n, 8) sums: [sum of rho > cutoff, / ratio] per group, as np.float64 scalars."""
+    """Region density rows of (n, 8) sums: [sum of rho > cutoff, / ratio] per group, as np.float64 scalars."""
     pos = np.asarray(sums, dtype=np.float64).reshape(-1, PE_SPHERE_NOUT)[:, 3]
     return [list(r) for r in zip(pos, pos / ratio)]
 
 
 def discrepancyRows(sums, ratio, avgAbsVoxel):
-    """``_regionDiscrepancyRows`` of (n, 8) sums: the ten values per group.  ``avgAbsVoxel``: getTotalAbsDensity(cutoff) /
-    number of voxels.  The expected columns are Python floats (a float times ``int(n)``), the others np.float64, as there."""
+    """Region discrepancy rows of (n, 8) sums: the ten values per group.  ``avgAbsVoxel``: getTotalAbsDensity(cutoff) /
+    number of voxels.  The expected columns are Python floats (the reference's float times ``int(n)``), the others
+    np.float64."""
     sums = np.asarray(sums, dtype=np.float64).reshape(-1, PE_SPHERE_NOUT)
     pos, neg = sums[:, 3], sums[:, 5]
     actual = pos + neg
@@ -125,7 +128,7 @@ def makeEntry(analyzer, kind, level, radius=3.5, numSD=None, type="", atomMask=N
                 if not atoms:
                     raise IndexError("list index out of range")  # the reference fails on a residue left without atoms
             kept.append([residue.parent.parent.id, residue.parent.id, residue.id[1], residue.resname,
-                         densityAnalysis._meanOccupancy(atoms, meanOf)])
+                         _meanOccupancy(atoms, meanOf)])
             xyz.extend([atom.coord for atom in atoms])
             if density and useOptimizedRadii:
                 radii.extend([analyzer._testRadius(atom, radius, True) for atom in atoms])
@@ -164,54 +167,19 @@ def makeEntry(analyzer, kind, level, radius=3.5, numSD=None, type="", atomMask=N
 
 
 # ---------------------------------------------------------------------------------------------------- the batch
-class RegionBatch:
+class RegionBatch(groupBatch.GroupBatch):
     """A batch of ``RegionEntry`` laid out for one ``pe_batch_sphere_sums`` launch, plus one ``CloudBatch`` for the ratios of
     the entries that need one.  All entries are grouped, or none is."""
 
     def __init__(self, entries, device=None):
-        self.entries = list(entries)
-        self.lib = _lib.load()
-        _device.require_cuda()
-        if device is None:
-            device = torch.device("cuda", torch.cuda.current_device())
-        self.device = device
-        nS = len(self.entries)
-        grouped = {e.groupStart is not None for e in self.entries}
-        if len(grouped) > 1:
-            raise ValueError("a batch is all grouped or all per atom")
-        self.grouped = grouped.pop() if grouped else False
-        atomCounts = np.array([len(e.xyz) for e in self.entries], dtype=np.int64)
-        groupCounts = np.array([e.nGroups for e in self.entries], dtype=np.int64)
-        self.atomStart = np.concatenate(([0], np.cumsum(atomCounts)))
-        self.groupBase = np.concatenate(([0], np.cumsum(groupCounts)))
-        self.nAtoms, self.nGroups = int(self.atomStart[-1]), int(self.groupBase[-1])
-        if self.nAtoms >= 2 ** 31 or self.nGroups >= 2 ** 31:
-            raise ValueError("a batch holds fewer than 2^31 atoms and groups")
-        xyz = np.concatenate([e.xyz for e in self.entries]) if nS else np.zeros((0, 3))
-        radius = np.concatenate([e.radius for e in self.entries]) if nS else np.zeros(0, dtype=np.float32)
-        groupMap = np.repeat(np.arange(nS, dtype=np.int32), groupCounts)
-        maps = (PeSumsMap * max(nS, 1))()
-        for k, e in enumerate(self.entries):
-            maps[k].geom = e.map.geom
-            maps[k].d_rho = e.map.rho.data_ptr()
-            maps[k].cut_pos, maps[k].cut_neg = e.cutPos, e.cutNeg
-        up = lambda arr: torch.from_numpy(np.ascontiguousarray(arr)).to(device)
-        self.d_maps = torch.frombuffer(bytearray(bytes(maps)), dtype=torch.uint8).to(device)
-        self.d_xyz = up(xyz if self.nAtoms else np.zeros((1, 3)))
-        self.d_radius = up(radius if self.nAtoms else np.zeros(1, dtype=np.float32))
-        self.d_groupMap = up(groupMap if self.nGroups else np.zeros(1, dtype=np.int32))
-        self.d_atomStart = up(self.atomStart.astype(np.int32))
-        self.d_groupStart = None
-        if self.grouped:
-            groupStart = np.empty(self.nGroups + 1, dtype=np.int32)
-            groupStart[-1] = self.nAtoms
-            for k, e in enumerate(self.entries):
-                groupStart[self.groupBase[k]:self.groupBase[k + 1]] = e.groupStart[:-1] + self.atomStart[k]
-            self.d_groupStart = up(groupStart)
-        self.d_out = torch.empty((max(self.nGroups, 1), PE_SPHERE_NOUT), dtype=torch.float64, device=device)
-        self.h_out = torch.empty(self.d_out.shape, dtype=torch.float64).pin_memory()
+        entries = list(entries)
+        maps = (PeSumsMap * max(len(entries), 1))()
+        for m, e in zip(maps, entries):
+            m.geom, m.d_rho = e.map.geom, e.map.rho.data_ptr()
+            m.cut_pos, m.cut_neg = e.cutPos, e.cutNeg
+        super().__init__(entries, maps, device)
         self.ws = torch.empty(max(int(self.lib.pe_batch_sphere_sums_workspace_bytes(self.nAtoms)), 256), dtype=torch.uint8,
-                              device=device)
+                              device=self.device)
         self.cloud, self.cloudOf = None, {}
 
     def launchSums(self):
@@ -225,6 +193,7 @@ class RegionBatch:
         """Enqueues the cloud aggregation of the entries whose ratio is not known yet (the defaults of ``aggregateCloud``), then
         the sums.  Entries whose structure the batched cloud layout cannot express, or every entry when
         PDB_EDA_B200_FULL_CLOUD is set, take ``densityElectronRatio`` (the per-structure pipeline) in ``collect``."""
+        from . import densityAnalysis
         items = []
         if densityAnalysis.BATCHED_CLOUD:
             from .cloudBatch import AtomTable, CloudBatch
@@ -244,8 +213,7 @@ class RegionBatch:
     def collect(self):
         """Synchronises; (ratio, (nGroups_k, 8) sums) of every entry."""
         arr = self.cloud.collectArrays() if self.cloud is not None else None
-        torch.cuda.current_stream().synchronize()
-        out = self.h_out.numpy()[:self.nGroups]
+        sums = super().collect()
         res = []
         for k, e in enumerate(self.entries):
             j = self.cloudOf.get(k)
@@ -256,51 +224,15 @@ class RegionBatch:
                     ratio = None                            # the single-structure call raises here too
             else:
                 ratio = float(arr["ratio"][j]) if arr["ok"][j] and len(self.cloud.items[j][1]) else None
-            res.append((ratio, out[self.groupBase[k]:self.groupBase[k + 1]].copy()))
+            res.append((ratio, sums[k]))
         return res
-
-    def run(self):
-        self.launch()
-        return self.collect()
 
 
 def analyzeStream(pairs, kind, level, maxBytes=8 << 30, device=None, **options):
-    """Yields (key, rows) for every (key, DensityAnalysis) of ``pairs``, in order: the rows of the single-structure call
-    ``kind`` x ``level`` with ``options`` (``makeEntry``), or None for an analyzer that is missing (falsy) or on which that call
-    would raise.  Analyzers are taken in batches of at most ``maxBytes`` device bytes (a larger entry forms a batch alone),
-    so that only one batch of them is held at a time."""
-    pending, used = [], 0                                   # (key, entry or None)
-
-    def flush():
-        entries = [e for _, e in pending if e is not None]
-        results = iter(RegionBatch(entries, device).run() if entries else [])
-        out = []
-        for key, e in pending:
-            rows = None
-            if e is not None:
-                ratio, sums = next(results)
-                try:
-                    rows = e.finish(ratio, sums)
-                except Exception:
-                    rows = None
-            out.append((key, rows))
-        pending.clear()
-        return out
-
-    for key, analyzer in pairs:
-        entry = None
-        if analyzer:
-            try:
-                entry = makeEntry(analyzer, kind, level, **options)
-            except Exception:
-                entry = None
-        b = entry.deviceBytes() if entry is not None else 0
-        if entry is not None and used and used + b > maxBytes:
-            yield from flush()
-            used = 0
-        pending.append((key, entry))
-        used += b
-    yield from flush()
+    """``groupBatch.stream`` of the single-structure call ``kind`` x ``level`` with ``options`` (``makeEntry``): (key, rows or
+    None) for every (key, DensityAnalysis) of ``pairs``, in order; None where that call would raise."""
+    return groupBatch.stream(pairs, lambda analyzer: makeEntry(analyzer, kind, level, **options),
+                             lambda entries: RegionBatch(entries, device).run(), maxBytes)
 
 
 def analyzeRegions(analyzers, kind, level, maxBytes=8 << 30, device=None, **options):

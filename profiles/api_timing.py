@@ -58,6 +58,10 @@ def run(name):
     timed("calculateAtomRegionDensity (3.5 A)", lambda: an.calculateAtomRegionDensity(3.5))
     if name != "c2":
         timed("calculateSymmetryAtomRegionDensity (3.5 A)", lambda: an.calculateSymmetryAtomRegionDensity(3.5))
+    for k in range(3):                                      # the first call includes one-time set-up
+        timed("residueMetrics (call %d)" % (k + 1), an.residueMetrics)
+    for k in range(3):
+        timed("atomMetrics (call %d)" % (k + 1), an.atomMetrics)
 
 
 if __name__ == "__main__":

@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Per-residue RSCC / RSR of the synthetic config-3 pool: the batched kernel (pe_pair_union_metrics, one launch for the whole
-pool) against the per-structure chain of DensityAnalysis.residueMetrics (sphere lists -> grouped de-duplication ->
-pe_pair_metrics), on the same structures, in one run.
+pool) against the per-structure voxel-list chain (sphere lists -> grouped de-duplication -> pe_pair_metrics), on the same
+structures, in one run.
 
 Pool: synthetic.poolSpec (grid sizes 64-256 on a 0.5 A grid, five space groups), a 2Fo-Fc map (synthetic.densityMapDevice)
 and a Fo-Fc map (smoothed noise at 0.1 x the 2Fo-Fc sigma) resident in HBM per structure, resolutions drawn in 0.6-3.0 A so
@@ -55,9 +55,9 @@ def build_pool(n, seed):
 
 
 def chain(entry):
-    """DensityAnalysis._groupMetrics on one structure."""
+    """The voxel-list chain on one structure: sphere lists -> grouped de-duplication -> pe_pair_metrics."""
     fo, diff = _Dm(entry.foMap), _Dm(entry.diffMap)
-    lists = cutils.sphereLists(fo, entry.coords32, entry.radius, 0.0)
+    lists = cutils.sphereLists(fo, entry.xyz, entry.radius, 0.0)
     group = torch.from_numpy(np.repeat(np.arange(entry.nGroups, dtype=np.int32), np.diff(entry.groupStart))).cuda()[lists["atom"].long()]
     _, first, _ = cutils.clusterCrs(lists["crs"], group, wantFirst=True)
     return cutils.pairMetrics(fo, diff, lists["crs"], group, first, entry.nGroups)
@@ -134,7 +134,7 @@ def main():
     rec = {
         "device": gpu, "structures": len(entries), "residues": b.nGroups, "atoms": b.nAtoms, "union_voxels": voxels,
         "map_bytes_resident": int(sum(4 * (e.foMap.rho.numel() + e.diffMap.rho.numel()) for e in entries)),
-        "radius_range": [float(min(e.radius for e in entries)), float(max(e.radius for e in entries))],
+        "radius_range": [float(min(e.radius[0] for e in entries)), float(max(e.radius[0] for e in entries))],
         "batched_ms": {"median": med, "min": float(min(times)), "max": float(max(times)), "repeats": len(times), "warmup": args.warmup},
         "chain_ms": chain_ms, "speedup": chain_ms / med,
         "batched_structures_per_s": len(entries) / (med / 1e3), "batched_residues_per_s": b.nGroups / (med / 1e3),

@@ -202,7 +202,7 @@ def test_statistics_kernel_matches_the_numpy_statement():
     recs, static = np.array(recs), np.array(static)
     nS, nA = len(sizes), len(atomMap)
     start = np.concatenate(([0], np.cumsum(sizes)))
-    maps = (cloudBatch.PeBatchMap * nS)()
+    maps = (_lib.PeBatchMap * nS)()
     for k in range(nS):
         maps[k].atom_begin, maps[k].atom_end = int(start[k]), int(start[k + 1])
     mapOut = np.zeros((nS, 8))

@@ -43,7 +43,7 @@ def _run_statistics(segments, nTypes=None, minTotalElectrons=400.0):
     segment.  Returns seg_out (n_segments x 14) and map_stats (n_segments x 4)."""
     import ctypes
     import torch
-    from pdb_eda_b200 import _lib, cloudBatch
+    from pdb_eda_b200 import _lib
     from pdb_eda_b200._device import _ptr, _stream
     lib = _lib.load()
     nS = len(segments)
@@ -56,7 +56,7 @@ def _run_statistics(segments, nTypes=None, minTotalElectrons=400.0):
         a = slice(int(start[k]), int(start[k + 1]))
         recs[a, 0], recs[a, 1], recs[a, 2], recs[a, 3], recs[a, 7] = 1.0, s["nv"], s["cd"], s["td"], s["flags"]
         static[a, 2] = s["bf"]
-    maps = (cloudBatch.PeBatchMap * nS)()
+    maps = (_lib.PeBatchMap * nS)()
     for k in range(nS):
         maps[k].atom_begin, maps[k].atom_end = int(start[k]), int(start[k + 1])
     mapOut = np.zeros((nS, 8))

@@ -1,6 +1,6 @@
 """CPU tier of the batched RSCC / RSR path (pdb_eda_b200/metricsBatch.py, pe_pair_union_metrics): argument errors without a
-device, the ``--single-mode`` surface of ``multiple``, the numpy row builder against a per-residue loop, and the all-reduced
-summary over two gloo ranks."""
+device, the ``--single-mode`` surface of ``multiple`` (including an unreadable --params / --atom-mask file), the numpy row
+builder against a per-residue loop, and the all-reduced summary over two gloo ranks."""
 import ctypes
 import os
 import socket
@@ -73,19 +73,20 @@ def _structure(seed):
     return st
 
 
-def test_residue_rows_against_a_per_residue_loop():
+def test_residue_entry_rows_against_the_reference_loop():
     from pdb_eda_b200 import metricsBatch
     st = _structure(5)
     entry = metricsBatch.residueEntry(_Analyzer(st))
     residues = list(st.get_residues())
-    assert entry.nGroups == len(residues) and entry.radius == metricsBatch.metricsRadius(2.0)
+    assert entry.nGroups == len(residues) and (entry.radius == np.float32(metricsBatch.metricsRadius(2.0))).all()
     assert entry.groupStart.tolist() == np.cumsum([0] + [len(r.child_list) for r in residues]).tolist()
-    np.testing.assert_array_equal(entry.coords32, np.asarray([a.coord for r in residues for a in r.child_list], dtype=np.float32))
+    assert entry.xyz.dtype == np.float64 and len(entry.radius) == len(entry.xyz)
+    np.testing.assert_array_equal(entry.xyz, np.asarray([a.coord for r in residues for a in r.child_list], dtype=np.float32))
     rng = np.random.default_rng(3)
     rscc, rsr = rng.uniform(-1, 1, len(residues)), rng.uniform(0, 1, len(residues))
     rscc[2] = np.nan
     got = entry.finish(rscc, rsr)
-    for k, residue in enumerate(residues):          # residueMetrics()'s loop (pdb_eda_b200/densityAnalysis.py)
+    for k, residue in enumerate(residues):          # the reference's per-residue loop (pdb_eda/densityAnalysis.py:815-829)
         bfactorWeightedSum = occupancySum = 0.0
         for atom in residue.child_list:
             bfactorWeightedSum += atom.get_bfactor() * atom.get_occupancy()
@@ -114,15 +115,30 @@ def test_entries_that_fail_like_the_single_call():
     assert out == [None, None]
 
 
+@pytest.mark.parametrize("opts", ["statistics --residue --params missing.json", "statistics --atom --params missing.json",
+                                  "statistics --residue --atom-mask missing.json"])
+def test_unreadable_options_file_fails_every_entry_as_single_does(tmp_path, monkeypatch, opts):
+    from pdb_eda_b200 import multipleStructures, singleStructure
+    monkeypatch.chdir(tmp_path)
+    single = multipleStructures.parseSingleMode(opts)
+    with pytest.raises(RuntimeError):
+        singleStructure.analyze(multipleStructures._entryArgs(single, "1abc", str(tmp_path / "out"), str(tmp_path)))
+    loads = []
+    monkeypatch.setattr(multipleStructures, "makeLoader", lambda dataDir: lambda pdbid: loads.append(pdbid) or 0)
+    summary = multipleStructures.runSingleMode(["1abc", "2bcd", "3cde"], str(tmp_path / "out"), single, str(tmp_path))
+    assert summary == {"ok": 0, "failed": 3, "rows": 0}
+    assert loads == [] and os.listdir(tmp_path / "out") == []         # no entry is read, no file is written
+
+
 def _worker(rank, world, port, out):
     import torch.distributed as dist
-    from pdb_eda_b200 import multi
+    from pdb_eda_b200 import metricsBatch, multi
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
     loads = []
-    run = multi.runMultipleMetrics(list(range(7)), lambda i: loads.append(i) or 0, "residue", costs=[3, 1, 4, 1, 5, 9, 2],
-                                   device="cpu")
+    stream = lambda pairs, maxBytes, device: metricsBatch.analyzeStream(pairs, "residue", maxBytes, device)
+    run = multi.runMultipleRows(list(range(7)), lambda i: loads.append(i) or 0, stream, costs=[3, 1, 4, 1, 5, 9, 2], device="cpu")
     summary = multi.summarizeMetrics(rank + 1, 2 * rank, 10 * rank + 5, "cpu")
     out[rank] = (run, summary, loads)
     dist.destroy_process_group()
@@ -137,7 +153,7 @@ def _free_port():
 
 
 @pytest.mark.timeout(120)
-def test_two_rank_summary_over_gloo():
+def test_two_rank_rows_summary_over_gloo():
     manager = mp.Manager()
     out = manager.dict()
     mp.spawn(_worker, args=(2, _free_port(), out), nprocs=2, join=True)

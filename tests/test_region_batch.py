@@ -58,7 +58,7 @@ def _batch_sums(items, which, mapIndex=None):
     lib = _lib.load()
     n = len(items)
     grouped = items[0][3] is not None
-    maps = (regionBatch.PeSumsMap * n)()
+    maps = (_lib.PeSumsMap * n)()
     atomStart, groupStart, groupMap, nG = [0], [], [], []
     for k, (dm, xyz, r, gs) in enumerate(items):
         maps[k].geom, maps[k].d_rho = dm.geom, dm.rho.data_ptr()

@@ -1,12 +1,12 @@
 """CPU tier of the batched region density / discrepancy path (pdb_eda_b200/regionBatch.py, pe_batch_sphere_sums): argument
 errors without a device, which ``--single-mode`` options run batched, and the numpy row builders against the per-row
-arithmetic of the single-structure calls."""
+arithmetic of the reference (pdb_eda/densityAnalysis.py:1037-1068, :1160-1211)."""
 import types
 
 import numpy as np
 import pytest
 
-from pdb_eda_b200 import _lib, densityAnalysis, multipleStructures, regionBatch
+from pdb_eda_b200 import _lib, multipleStructures, regionBatch
 
 
 def test_argument_errors_without_a_device():
@@ -46,19 +46,6 @@ def test_which_single_mode_options_run_batched(opts, path):
     assert multipleStructures.batchedPath(multipleStructures.parseSingleMode(opts)) == path
 
 
-class _Fake:
-    """What ``_regionDensityRows`` / ``_regionDiscrepancyRows`` read of a DensityAnalysis."""
-
-    def __init__(self, ratio, totalAbs, nVoxels):
-        dm = types.SimpleNamespace(meanDensity=0.1, stdDensity=0.5, getTotalAbsDensity=lambda c: totalAbs,
-                                   deviceMap=types.SimpleNamespace(n_voxels=nVoxels))
-        self.densityObj = self.diffDensityObj = dm
-        self._ratio = ratio
-
-    def _requireRatio(self):
-        return self._ratio
-
-
 def _random_sums(rng, n):
     s = rng.standard_normal((n, 8)) * 10.0 ** rng.integers(-3, 6, (n, 1))
     s[:, 0] = rng.integers(0, 5000, n)
@@ -67,17 +54,34 @@ def _random_sums(rng, n):
     return s
 
 
+def _density_rows(sums, ratio):
+    """The reference's region density per row: [sum of rho > cutoff, / ratio]."""
+    return [[row[3], row[3] / ratio] for row in sums]
+
+
+def _discrepancy_rows(sums, ratio, avg_abs_vox):
+    """The reference's region discrepancy per row: the ten values, the expected count as a float times ``int(n)``."""
+    rows = []
+    for row in sums:
+        pos, neg = row[3], row[5]
+        actual = pos + neg
+        actual_abs = abs(pos) + abs(neg)
+        expected = avg_abs_vox * int(row[0])
+        rows.append([actual_abs, actual_abs / ratio, expected, expected / ratio, actual, actual / ratio, pos, pos / ratio, neg, neg / ratio])
+    return rows
+
+
 @pytest.mark.parametrize("seed", [0, 1, 2])
-def test_row_builders_equal_the_per_row_arithmetic(monkeypatch, seed):
+def test_row_builders_equal_the_reference_row_arithmetic(seed):
     rng = np.random.default_rng(seed)
     sums = _random_sums(rng, 400)
     ratio = float(rng.uniform(0.05, 3.0))
-    fake = _Fake(ratio, float(rng.uniform(1e3, 1e6)), int(rng.integers(10 ** 4, 10 ** 7)))
-    monkeypatch.setattr(densityAnalysis.utils, "sphereSums", lambda *a, **k: sums)
-    want, _ = densityAnalysis.DensityAnalysis._regionDensityRows(fake, np.zeros((400, 3)), np.ones(400), None, 1.5)
+    avg_abs_vox = float(rng.uniform(1e3, 1e6)) / int(rng.integers(10 ** 4, 10 ** 7))
+    want = _density_rows(sums, ratio)
     got = regionBatch.densityRows(sums, ratio)
-    want2, _ = densityAnalysis.DensityAnalysis._regionDiscrepancyRows(fake, np.zeros((400, 3)), 3.5, None, 3.0)
-    got2 = regionBatch.discrepancyRows(sums, ratio, fake.diffDensityObj.getTotalAbsDensity(0) / fake.diffDensityObj.deviceMap.n_voxels)
+    want2 = _discrepancy_rows(sums, ratio, avg_abs_vox)
+    got2 = regionBatch.discrepancyRows(sums, ratio, avg_abs_vox)
+    assert len(got) == len(want) and len(got2) == len(want2)
     for g, w in list(zip(got, want)) + list(zip(got2, want2)):
         assert len(g) == len(w)
         for x, y in zip(g, w):
