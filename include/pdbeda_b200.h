@@ -231,6 +231,10 @@ int pe_blob_label(const pe_geom *g, const float *d_rho, float cut_pos, float cut
  *                     all-reduces the table.
  * d_ws: >= pe_slab_workspace_bytes(world, cap_blobs, u0, u1), shared by the three calls; pe_slab_status reads its overflow
  * flag (synchronises).
+ * cap_blobs and cap_plane set the layout of the exchange buffers and must be the SAME on every rank (size them from the largest
+ * slab).  pe_slab_boundary stamps them into each buffer; pe_slab_merge sets the flag when any rank's buffer carries another
+ * stamp or counts beyond them (also when that rank's pe_blob_label or boundary overflowed), and then merges nothing, so every
+ * rank sees the failure.  cap_blobs < 2^31, cap_plane < 2^32.
  * Size limits: one SLAB holds fewer than 2^31 stored voxels (32-bit element offsets and keys inside a call); the WHOLE map may
  * be larger -- its keys are 64-bit and g_whole is used for index -> coordinate arithmetic only -- so maps beyond the 1290^3 that
  * one pe_blob_label call takes (1536^3, 2048^3 ...) are labelled slab by slab, on several GPUs or one after another on one. */

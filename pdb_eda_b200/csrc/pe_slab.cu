@@ -17,16 +17,23 @@
 //                     binary search per rank in the gathered (sorted) key arrays -- no global sort;
 //   pe_slab_relabel   re-numbers this rank's voxels and accumulates the per-blob sums from the voxels with the WHOLE map's
 //                     geometry (global section index), into a table the caller all-reduces.
-// No host round trip between the stages; capacities are fixed per call and overflows raise a flag.
+// No host round trip between the stages; capacities are fixed per call and the same on every rank (the buffer layout follows
+// them), overflows and buffers packed with other capacities raise a flag.
 #include "pe_common.cuh"
 
 namespace pe {
 
 constexpr int kSlabThreads = 256;
 
+// One sign's block: hdr[0] = local blobs, hdr[1] / hdr[2] = voxels of the first / last plane, hdr[3] = slab_stamp of the
+// capacities that laid the block out.  The merge reads every rank's block at the offsets ITS capacities give, so all ranks
+// must use the same ones; a block with another stamp sets the error flag and the merge leaves the buffers alone.
 struct SlabLayout {  // of one sign's block inside a rank's exchange buffer, in bytes
     int64_t hdr, minkey, first, last, size;
 };
+__host__ __device__ inline unsigned long long slab_stamp(int64_t cap_blobs, int64_t cap_plane) {  // cap_blobs < 2^31, cap_plane < 2^32
+    return ((unsigned long long)cap_blobs << 32) | (unsigned long long)cap_plane;
+}
 __host__ __device__ inline SlabLayout slab_layout(int64_t cap_blobs, int64_t cap_plane) {
     SlabLayout L;
     L.hdr = 0;
@@ -57,8 +64,13 @@ __global__ void __launch_bounds__(kSlabThreads)
     unsigned long long *minkey = (unsigned long long *)(base + L.minkey);
     int32_t *first = (int32_t *)(base + L.first), *last = (int32_t *)(base + L.last);
     const int64_t n = counts[2 * k], nb = counts[2 * k + 1];
-    if (blockIdx.x == 0 && threadIdx.x == 0) hdr[0] = (unsigned long long)nb;
-    if (nb > cap_blobs) {
+    // pe_blob_label failed (its counts may then exceed the capacities): no stamp, so that every rank's merge flags this block
+    const bool ok = counts[4] == 0 && n <= cap_voxels && nb <= cap_blobs;
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        hdr[0] = (unsigned long long)nb;
+        hdr[3] = ok ? slab_stamp(cap_blobs, cap_plane) : 0ull;
+    }
+    if (!ok) {
         if (blockIdx.x == 0 && threadIdx.x == 0) *d_bad = 1;
         return;
     }
@@ -105,6 +117,7 @@ struct MergeArgs {
     uint32_t *parent;      // 2 x world x cap_blobs
     unsigned long long *compkey;
     uint32_t *absorbed, *absorbed_scan;
+    int *bad;              // the error flag (first word of the workspace): set -> the later merge kernels do nothing
 };
 
 __device__ __forceinline__ const char *sign_block(const MergeArgs &a, int rank, int k) {
@@ -114,9 +127,18 @@ __device__ __forceinline__ int64_t blob_count(const MergeArgs &a, int rank, int 
     return (int64_t)((const unsigned long long *)sign_block(a, rank, k))[0];
 }
 
+// also checks the header of every rank's blocks before any kernel reads their contents: the stamp of this call's capacities,
+// counts within them.  Every rank flags the same blocks, so a failure on one rank stops all ranks before the all-reduce.
 __global__ void __launch_bounds__(kSlabThreads) slab_init_kernel(MergeArgs a) {
     const int64_t total = 2ll * a.world * a.cap_blobs;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    if (blockIdx.x == 0)
+        for (int slot = threadIdx.x; slot < 2 * a.world; slot += blockDim.x) {
+            const unsigned long long *hdr = (const unsigned long long *)sign_block(a, slot % a.world, slot / a.world);
+            if (hdr[3] != slab_stamp(a.cap_blobs, a.cap_plane) || hdr[0] > (unsigned long long)a.cap_blobs ||
+                hdr[1] > (unsigned long long)a.cap_plane || hdr[2] > (unsigned long long)a.cap_plane)
+                *a.bad = 1;
+        }
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
         a.parent[i] = (uint32_t)i;
         a.compkey[i] = ~0ull;
@@ -126,6 +148,7 @@ __global__ void __launch_bounds__(kSlabThreads) slab_init_kernel(MergeArgs a) {
 
 // blockIdx.y = sign * (world - 1) + cut: paints the first plane of rank cut + 1
 __global__ void __launch_bounds__(kSlabThreads) slab_paint_kernel(MergeArgs a) {
+    if (*a.bad) return;
     const int k = blockIdx.y / (a.world - 1), cut = blockIdx.y % (a.world - 1);
     const SlabLayout L = slab_layout(a.cap_blobs, a.cap_plane);
     const char *blk = sign_block(a, cut + 1, k);
@@ -140,6 +163,7 @@ __global__ void __launch_bounds__(kSlabThreads) slab_paint_kernel(MergeArgs a) {
 
 // the last plane of rank `cut` against the painted plane: 26-adjacency across the cut = the 9 (column, row) neighbours
 __global__ void __launch_bounds__(kSlabThreads) slab_union_kernel(MergeArgs a) {
+    if (*a.bad) return;
     const int k = blockIdx.y / (a.world - 1), cut = blockIdx.y % (a.world - 1);
     const SlabLayout L = slab_layout(a.cap_blobs, a.cap_plane);
     const char *blk = sign_block(a, cut, k);
@@ -166,6 +190,7 @@ __global__ void __launch_bounds__(kSlabThreads) slab_union_kernel(MergeArgs a) {
 
 // smallest key of every merged blob (at its union-find root)
 __global__ void __launch_bounds__(kSlabThreads) slab_compkey_kernel(MergeArgs a) {
+    if (*a.bad) return;
     const int slot = blockIdx.y;  // sign * world + rank
     const int k = slot / a.world, rank = slot % a.world;
     const char *blk = sign_block(a, rank, k);
@@ -181,6 +206,7 @@ __global__ void __launch_bounds__(kSlabThreads) slab_compkey_kernel(MergeArgs a)
 
 // a blob is absorbed when it is not the member of its merged blob that carries the smallest key
 __global__ void __launch_bounds__(kSlabThreads) slab_absorbed_kernel(MergeArgs a) {
+    if (*a.bad) return;
     const int slot = blockIdx.y;
     const int k = slot / a.world, rank = slot % a.world;
     const char *blk = sign_block(a, rank, k);
@@ -196,6 +222,7 @@ __global__ void __launch_bounds__(kSlabThreads) slab_absorbed_kernel(MergeArgs a
 // new number of every blob of THIS rank (blockIdx.y = sign) + the number of merged blobs per sign
 __global__ void __launch_bounds__(kSlabThreads)
     slab_number_kernel(MergeArgs a, int32_t *__restrict__ new_number /* 2 x cap_blobs */, int64_t *__restrict__ n_merged /* 2 */) {
+    if (*a.bad) return;
     const int k = blockIdx.y;
     const SlabLayout L = slab_layout(a.cap_blobs, a.cap_plane);
     const int64_t nb = min(blob_count(a, a.rank, k), a.cap_blobs);
@@ -241,6 +268,7 @@ __global__ void __launch_bounds__(kSlabThreads)
                         const uint32_t *__restrict__ key, const float *__restrict__ value, int32_t *__restrict__ label, int Uslab,
                         int s0, int64_t cap_blobs, const int32_t *__restrict__ new_number, const int64_t *__restrict__ n_merged,
                         int64_t cap_merged, double *__restrict__ stats /* 2 x cap_merged x 8 */, int *__restrict__ d_bad) {
+    if (*d_bad) return;  // the merge did not run: new_number / n_merged are not this call's
     const int k = blockIdx.y;
     const int lane = threadIdx.x & 31;
     const int64_t n = counts[2 * k];
@@ -342,6 +370,7 @@ int pe_slab_boundary(const pe_geom *g_slab, int32_t u2_whole, int32_t s0, int32_
     if (int rc = check_geom(g_slab)) return rc;
     PE_CHECK_ARG(d_counts && d_key && d_label && d_exchange && d_ws, "pe_slab_boundary: null pointer");
     PE_CHECK_ARG(cap_voxels > 0 && cap_blobs > 0 && cap_plane > 0, "pe_slab_boundary: capacities must be positive");
+    PE_CHECK_ARG(cap_blobs < (1ll << 31) && cap_plane < (1ll << 32), "pe_slab_boundary: capacities out of range");
     cudaStream_t st = (cudaStream_t)stream;
     const SlabLayout L = slab_layout(cap_blobs, cap_plane);
     char *buf = (char *)d_exchange;
@@ -364,6 +393,7 @@ int pe_slab_merge(int32_t world, int32_t rank, const void *d_gathered, int64_t c
     PE_CHECK_ARG(world >= 1 && rank >= 0 && rank < world, "pe_slab_merge: bad rank / world");
     PE_CHECK_ARG(d_gathered && d_new_number && d_n_merged && d_ws, "pe_slab_merge: null pointer");
     PE_CHECK_ARG(2ll * world * cap_blobs < (1ll << 31), "pe_slab_merge: too many blobs for 32-bit ids");
+    PE_CHECK_ARG(cap_blobs > 0 && cap_plane > 0 && cap_plane < (1ll << 32), "pe_slab_merge: capacities out of range");
     cudaStream_t st = (cudaStream_t)stream;
     const MergeWs w = merge_ws(world, cap_blobs, u0, u1);
     char *ws = (char *)d_ws;
@@ -381,6 +411,7 @@ int pe_slab_merge(int32_t world, int32_t rank, const void *d_gathered, int64_t c
     a.compkey = (unsigned long long *)(ws + w.compkey);
     a.absorbed = (uint32_t *)(ws + w.absorbed);
     a.absorbed_scan = (uint32_t *)(ws + w.absorbed_scan);
+    a.bad = (int *)(ws + w.flags);
     const int64_t ids = 2ll * world * cap_blobs + 1;
     PE_LAUNCH("slab_init_kernel", st, slab_init_kernel<<<slab_grid(ids), kSlabThreads, 0, st>>>(a));
     if (world > 1) {

@@ -13,7 +13,8 @@ The reference holds a whole map in one process and clusters with an N x N distan
   4. ``pe_slab_relabel`` rewrites the labels and accumulates the per-blob sums (DensityBlob.fromCrsList,
      pdb_eda/ccp4.py:522-545) with the whole map's geometry; ONE ``all_reduce`` completes them.
 
-Two collectives and one host synchronisation (to size the all-reduce) per call: ``SlabLabeller``.
+Two collectives and one host synchronisation (to size the all-reduce) per call: ``SlabLabeller``.  The exchange buffers'
+layout follows the capacities, so these are per decomposition (``slabCapacities`` of the largest slab), never per slab.
 ``labelSlabsEmulated`` runs all "ranks" one after another on a single GPU through the same kernels (no kernel ever waits
 on another), which is how the merge is verified against the whole-map labelling on one device.
 ``mergeBlobIds`` / ``mergeDistributed`` state the same merge in device-agnostic torch with ragged all-gathers: the gloo
@@ -40,6 +41,48 @@ def slabRanges(nSections, world):
         out.append((s, s + n))
         s += n
     return out
+
+
+def checkRanges(ranges, nSections):
+    """Rejects a decomposition that is not contiguous, non-empty [s0, s1) slabs covering [0, nSections) in order."""
+    ranges = [(int(s0), int(s1)) for s0, s1 in ranges]
+    if not ranges:
+        raise ValueError("slab ranges: no slab")
+    at = 0
+    for s0, s1 in ranges:
+        if s0 != at:
+            raise ValueError("slab ranges %s: [%d, %d) does not start where the previous slab ends (%d)" % (ranges, s0, s1, at))
+        if s1 <= s0:
+            raise ValueError("slab ranges %s: [%d, %d) is empty" % (ranges, s0, s1))
+        at = s1
+    if at != nSections:
+        raise ValueError("slab ranges %s: cover [0, %d), the map has %d sections" % (ranges, at, nSections))
+    return ranges
+
+
+def coveredSections(s0, s1, u2):
+    """Sections of the slab [s0, s1) inside the unique volume (0 when it lies entirely in the repeated part of the map)."""
+    return max(min(int(s1), int(u2)) - int(s0), 0)
+
+
+def slabCapacities(u0, u1, maxCovered, capVoxels=None, capBlobs=None, capPlane=None):
+    """(capVoxels, capBlobs, capPlane) of one decomposition: the explicit values where given, else a function of the plane
+    size and the LARGEST slab's covered sections only.  The exchange buffer layout and ``pe_slab_merge``'s reading of the
+    gathered buffers follow capBlobs and capPlane, so they must be equal on every rank; sizing them from each rank's own
+    slab breaks that whenever slabs cover different numbers of sections (uneven splits, over-sampled maps)."""
+    capVoxels = int(capVoxels or max(4096, u0 * u1 * max(int(maxCovered), 1) // 64))
+    return capVoxels, int(capBlobs or max(1024, capVoxels // 4)), int(capPlane or max(4096, u0 * u1 // 16))
+
+
+def agreedCapacities(u0, u1, covered, world=1, group=None, device=None, capVoxels=None, capBlobs=None, capPlane=None):
+    """``slabCapacities`` of the decomposition as one rank sees it (``covered``: its own slab's covered sections).  With
+    ``world > 1`` and no ``capVoxels``, one all_reduce(MAX) over ``group`` (a tensor on ``device``) finds the largest slab."""
+    maxCovered = int(covered)
+    if int(world) > 1 and not capVoxels:
+        t = torch.tensor([maxCovered], dtype=torch.int64, device=device)
+        dist.all_reduce(t, op=dist.ReduceOp.MAX, group=group)
+        maxCovered = int(t.item())
+    return slabCapacities(u0, u1, maxCovered, capVoxels, capBlobs, capPlane)
 
 
 def _slabGeom(full, s0, s1):
@@ -129,7 +172,11 @@ class SlabLabeller:
     (e.g. on the slabs of successive maps of one geometry) without allocating.
 
     ``fullHeader``: the whole map's DensityHeader; [s0, s1): this rank's sections; ``world`` / ``rank`` / ``group``: the
-    ranks that hold the slabs in section order (``group=None``: the default process group; ``world == 1`` needs none)."""
+    ranks that hold the slabs in section order (``group=None``: the default process group; ``world == 1`` needs none).
+
+    Capacities are per decomposition, not per slab: by default ``slabCapacities`` of the largest slab, which the ranks agree
+    on with one all-reduce here (``world > 1`` and no ``capVoxels``).  Explicit ``capVoxels`` / ``capBlobs`` / ``capPlane``
+    must be the same on every rank; ``pe_slab_merge`` flags buffers packed with other capacities and ``label`` raises."""
 
     def __init__(self, fullHeader, s0, s1, world=1, rank=0, device=None, origin=None, group=None, capVoxels=None, capBlobs=None,
                  capPlane=None):
@@ -142,12 +189,12 @@ class SlabLabeller:
         self.geom = _device.geom_from_header(fullHeader, origin)
         U = (self.geom.unique_ncrs[0], self.geom.unique_ncrs[1], self.geom.unique_ncrs[2])
         self.U = U
-        self.covered = max(min(self.s1, U[2]) - self.s0, 0)          # sections of the slab inside the unique volume
+        if not 0 <= self.s0 < self.s1 <= self.geom.ncrs[2]:
+            raise ValueError("slab [%d, %d) of a map of %d sections" % (self.s0, self.s1, self.geom.ncrs[2]))
+        self.covered = coveredSections(self.s0, self.s1, U[2])
         self.slabGeom = _slabGeom(self.geom, self.s0, self.s1)
-        nvox = U[0] * U[1] * max(self.covered, 1)
-        self.capVoxels = int(capVoxels or max(4096, nvox // 64))
-        self.capBlobs = int(capBlobs or max(1024, self.capVoxels // 4))
-        self.capPlane = int(capPlane or max(4096, U[0] * U[1] // 16))
+        self.capVoxels, self.capBlobs, self.capPlane = agreedCapacities(U[0], U[1], self.covered, self.world, group, self.device,
+                                                                        capVoxels, capBlobs, capPlane)
         self.capMerged = self.capBlobs * self.world
         dev = self.device
         self.counts = torch.zeros(5, dtype=torch.int64, device=dev)
@@ -199,7 +246,8 @@ class SlabLabeller:
         check(self.lib.pe_slab_status(_ptr(self.mergeWs), _stream(), ctypes.byref(bad)), "pe_slab_status")
         c = self.hostTail.tolist()
         if c[4] or bad.value:
-            raise RuntimeError("slab labelling: a capacity was exceeded (voxels %d / %d of %d, blobs %d / %d of %d, plane %d)"
+            raise RuntimeError("slab labelling: a capacity was exceeded here or on another rank, or the ranks' capacities differ "
+                               "(voxels %d / %d of %d, blobs %d / %d of %d, plane %d)"
                                % (c[0], c[2], self.capVoxels, c[1], c[3], self.capBlobs, self.capPlane))
         return c
 
@@ -240,8 +288,8 @@ _labellers = {}
 
 def labelSlabDistributed(fullHeader, rhoSlab, s0, s1, cutPos, cutNeg, origin=None, group=None):
     """One rank's call: label this rank's slab [s0, s1) of the map and merge across ranks (a cached ``SlabLabeller`` per
-    geometry).  Returns per sign a dict with this rank's voxels (global crs, value, global blob number) and the all-reduced
-    per-blob statistics."""
+    geometry: the ranks agree on its capacities once, when a geometry is new).  Returns per sign a dict with this rank's
+    voxels (global crs, value, global blob number) and the all-reduced per-blob statistics."""
     rank, world = (dist.get_rank(group), dist.get_world_size(group)) if dist.is_initialized() else (0, 1)
     keyOf = (tuple(fullHeader.ncrs), tuple(fullHeader.crsStart), tuple(fullHeader.xyzInterval), int(s0), int(s1), world, rank,
              rhoSlab.device.index, id(group))
@@ -252,15 +300,25 @@ def labelSlabDistributed(fullHeader, rhoSlab, s0, s1, cutPos, cutNeg, origin=Non
     return lab.label(rhoSlab, cutPos, cutNeg)
 
 
-def labelSlabsEmulated(fullHeader, rho, world, cutPos, cutNeg, origin=None):
+def labelSlabsEmulated(fullHeader, rho, world, cutPos, cutNeg, origin=None, ranges=None, capVoxels=None, capBlobs=None,
+                       capPlane=None):
     """All ranks of ``SlabLabeller.label`` executed one after another on ONE GPU (``rho``: the whole map on the device) through
     the same kernels; the exchange buffers are concatenated instead of all-gathered and the partial sums added instead of
-    all-reduced.  Returns per sign the complete voxel list in canonical order with whole-map blob numbers and statistics."""
+    all-reduced.  ``ranges``: the slabs [s0, s1) (default ``slabRanges(ns, world)``; ``world`` may then be None); capacities
+    as in ``SlabLabeller``, the same for every slab.  Returns per sign the complete voxel list in canonical order with
+    whole-map blob numbers and statistics."""
     geom = _device.geom_from_header(fullHeader, origin)
     ns, nr, nc = geom.ncrs[2], geom.ncrs[1], geom.ncrs[0]
+    if ranges is None:
+        ranges = slabRanges(ns, world)
+    elif world is not None and int(world) != len(ranges):
+        raise ValueError("slab ranges: %d slabs for world %d" % (len(ranges), world))
+    ranges = checkRanges(ranges, ns)
+    world = len(ranges)
     vol = rho.reshape(ns, nr, nc)
-    ranges = slabRanges(ns, world)
-    labs = [SlabLabeller(fullHeader, s0, s1, world, r, rho.device, origin) for r, (s0, s1) in enumerate(ranges)]
+    U = geom.unique_ncrs
+    caps = slabCapacities(U[0], U[1], max(coveredSections(s0, s1, U[2]) for s0, s1 in ranges), capVoxels, capBlobs, capPlane)
+    labs = [SlabLabeller(fullHeader, s0, s1, world, r, rho.device, origin, None, *caps) for r, (s0, s1) in enumerate(ranges)]
     for lab, (s0, s1) in zip(labs, ranges):
         lab._labelLocal(vol[s0:s1].contiguous(), cutPos, cutNeg)
         lab._boundary()

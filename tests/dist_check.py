@@ -3,7 +3,8 @@
   (a) multiple-structures mode: synthetic structures sharded over the ranks, cumulative statistics all-reduced and
       rows all-gathered, compared on rank 0 with a single-process pass over all structures;
   (b) slab-decomposed blob labelling of one map across the ranks (halo exchange over NCCL), compared on every rank
-      with the whole-map labelling.
+      with the whole-map labelling;
+  (c) the same on a non-cubic, permuted, shifted map whose section count splits into unequal slabs.
 Prints DIST_CHECK_OK on success."""
 import io
 import os
@@ -71,6 +72,25 @@ def main():
         order = torch.argsort(key)
         assert torch.equal(wc, p["crs"][order]) and torch.equal(wl, p["label"][order])
         assert w["n_blobs"] == p["n_blobs"]
+        torch.testing.assert_close(p["stats"], w["stats"], rtol=1e-9, atol=1e-9)
+    # ---- (c) a non-cubic, permuted, shifted map of 67 sections (a prime: every world > 1 gives unequal slabs), slabs above
+    # the capacity floors, so the ranks must agree on one exchange layout
+    import cases
+    shape = (67, 120, 160)                                   # (sections, rows, columns)
+    host = cases._noise(shape, 17)
+    hdr2 = ccp4.DensityHeader.fromFileHeader(synthetic.ccp4Header(shape[::-1], (64.0, 40.0, 90.0, 90, 90, 90), (128, 80, 180),
+                                                                  crsStart=(5, -7, 3), axisOrder=(3, 1, 2)))
+    vol2 = torch.from_numpy(host).to(device)
+    s0, s1 = slab.slabRanges(shape[0], world)[rank]
+    parts2 = slab.labelSlabDistributed(hdr2, vol2[s0:s1].contiguous(), s0, s1, 2.5, -2.5)
+    whole2 = _device.DeviceMap(_device.geom_from_header(hdr2), vol2.reshape(-1)).blob_label(2.5, -2.5)
+    U = hdr2.uniqueNcrs
+    for w, p in zip(whole2, parts2):
+        sel = (w["crs"][:, 2] >= s0) & (w["crs"][:, 2] < s1)
+        key = (p["crs"][:, 0] * U[1] + p["crs"][:, 1]) * U[2] + p["crs"][:, 2]
+        order = torch.argsort(key)
+        assert torch.equal(w["crs"][sel].long(), p["crs"][order]) and torch.equal(w["label"][sel].long(), p["label"][order])
+        assert w["n_blobs"] == p["n_blobs"] > 100
         torch.testing.assert_close(p["stats"], w["stats"], rtol=1e-9, atol=1e-9)
     dist.barrier()
     if rank == 0:

@@ -1,5 +1,6 @@
 """Slab-decomposed blob labelling: CPU tier = the cross-rank merge over gloo (world_size 2 and 3) against a
-single-process merge; GPU tier = all slabs emulated on one GPU against the whole-map labelling."""
+single-process merge, the ranks' agreement on one set of capacities (gloo) and the host checks of slab ranges; GPU tier =
+all slabs emulated on one GPU against the whole-map labelling (tests/test_slab_vs_host.py: against host references)."""
 import os
 import socket
 
@@ -104,6 +105,82 @@ def test_merge_blob_ids_single_process():
     number, n = slab.mergeBlobIds(3, torch.zeros((0, 2), dtype=torch.int64), torch.tensor([3, 1, 2]))
     assert n == 3 and number.tolist() == [2, 0, 1]
     assert slab.slabRanges(10, 4) == [(0, 3), (3, 6), (6, 8), (8, 10)]
+
+
+def _own_slab_rule(u0, u1, covered):
+    """The capacities a slab would get if it were sized for itself (the rule, applied to one slab)."""
+    capVoxels = max(4096, u0 * u1 * max(covered, 1) // 64)
+    return capVoxels, max(1024, capVoxels // 4), max(4096, u0 * u1 // 16)
+
+
+# (U0, U1, U2, stored sections, ranges): three ranks each
+CAPACITY_LAYOUTS = {
+    "1024^3": (1024, 1024, 1024, 1024, None),
+    "1000^3": (1000, 1000, 1000, 1000, None),
+    "over-sampled": (1024, 1024, 512, 600, None),                   # 200 / 200 / 112 covered sections
+    "thin": (160, 120, 67, 67, [(0, 1), (1, 33), (33, 67)]),
+    "beyond": (256, 192, 40, 67, [(0, 34), (34, 40), (40, 67)]),    # the last slab lies beyond the unique volume
+}
+
+
+def _capacity_worker(rank, world, port, out):
+    import torch.distributed as dist
+    from pdb_eda_b200 import _lib, slab
+    os.environ["MASTER_ADDR"] = "127.0.0.1"
+    os.environ["MASTER_PORT"] = str(port)
+    dist.init_process_group("gloo", rank=rank, world_size=world)
+    lib = _lib.load()
+    res = {}
+    for name, (u0, u1, u2, ns, ranges) in CAPACITY_LAYOUTS.items():
+        s0, s1 = (ranges or slab.slabRanges(ns, world))[rank]
+        caps = slab.agreedCapacities(u0, u1, slab.coveredSections(s0, s1, u2), world, device="cpu")
+        res[name] = caps + (int(lib.pe_slab_exchange_bytes(caps[1], caps[2])),)
+    out[rank] = res
+    dist.destroy_process_group()
+
+
+@pytest.mark.timeout(180)
+def test_every_rank_gets_the_same_capacities():
+    """The ranks of uneven, thin, over-sampled and beyond-the-unique-volume decompositions agree (one all-reduce over gloo) on
+    capacities and exchange bytes, those of the largest slab; sizing each slab for itself would give them different layouts."""
+    from pdb_eda_b200 import _lib, slab
+    world = 3
+    manager = mp.Manager()
+    out = manager.dict()
+    mp.spawn(_capacity_worker, args=(world, _free_port(), out), nprocs=world, join=True)
+    lib = _lib.load()
+    for name, (u0, u1, u2, ns, ranges) in CAPACITY_LAYOUTS.items():
+        ranges = ranges or slab.slabRanges(ns, world)
+        got = {out[r][name] for r in range(world)}
+        assert len(got) == 1, (name, got)
+        capVoxels, capBlobs, capPlane, nbytes = got.pop()
+        own = [_own_slab_rule(u0, u1, slab.coveredSections(s0, s1, u2)) for s0, s1 in ranges]
+        assert len({o[1] for o in own}) > 1, name                     # the case the agreement exists for
+        assert (capVoxels, capBlobs, capPlane) == max(own)             # the largest slab's
+        assert nbytes == lib.pe_slab_exchange_bytes(capBlobs, capPlane) >= max(lib.pe_slab_exchange_bytes(o[1], o[2]) for o in own)
+    # the rule as a function: largest slab of slabRanges(1024, 6) and of an explicit override
+    own = [_own_slab_rule(1024, 1024, s1 - s0) for s0, s1 in slab.slabRanges(1024, 6)]
+    assert slab.slabCapacities(1024, 1024, 171) == max(own) and own[0][1] != own[-1][1]
+    assert slab.slabCapacities(1024, 1024, 171, capVoxels=8192) == (8192, 2048, 65536)
+    assert slab.agreedCapacities(160, 120, 0) == (4096, 1024, 4096)
+
+
+def test_slab_ranges_are_checked_before_any_device_work():
+    """A gap, an overlap, an empty slab, ranges that stop short or run past the map, more slabs than sections and a world that
+    contradicts the ranges are rejected on the host (ValueError) before a labeller or a device buffer exists: the map here is
+    a CPU tensor and there may be no GPU at all."""
+    from pdb_eda_b200 import ccp4, slab, synthetic
+    hdr = ccp4.DensityHeader.fromFileHeader(synthetic.ccp4Header((20, 16, 12), (10.0, 8.0, 6.0, 90, 90, 90), (20, 16, 12)))
+    rho = torch.zeros(20 * 16 * 12)
+    for ranges in ([(0, 5), (6, 12)], [(0, 6), (5, 12)], [(0, 6), (6, 6), (6, 12)], [(0, 6), (6, 11)], [(0, 6), (6, 13)],
+                   [(1, 6), (6, 12)], [(6, 12), (0, 6)], []):
+        with pytest.raises(ValueError):
+            slab.labelSlabsEmulated(hdr, rho, None, 1.0, -1.0, ranges=ranges)
+    with pytest.raises(ValueError):
+        slab.labelSlabsEmulated(hdr, rho, 13, 1.0, -1.0)
+    with pytest.raises(ValueError):
+        slab.labelSlabsEmulated(hdr, rho, 3, 1.0, -1.0, ranges=[(0, 6), (6, 12)])
+    assert slab.checkRanges([(0, 1), (1, 12)], 12) == [(0, 1), (1, 12)]
 
 
 @pytest.mark.gpu
