@@ -76,6 +76,17 @@ void pe_profile_reset(void);
 int pe_profile_entries(void);
 int pe_profile_get(int index, const char **name, long long *count, double *total_ms);
 
+/* SM partition of device `device` (CUDA green contexts): blob_sms SMs with *stream_blob on them, the device's other SMs with
+ * *stream_rest; both are non-blocking streams.  Kernels enqueued on one run only on its SMs, so two passes limited by different
+ * resources overlap at their full per-SM occupancy.  Every entry point sizes its resident grids (persistent and cooperative
+ * kernels) by the SMs of the stream it launches on.  *sms_blob / *sms_rest: the SM counts provisioned.  PE_ERR_ARG for null
+ * pointers or a count the driver does not split exactly (from compute capability 9.0 on: a multiple of 8, below the device's
+ * SM count), PE_ERR_NO_DEVICE without a device, PE_ERR_CUDA when the driver has no green contexts or refuses; nothing is
+ * left behind on failure.  pe_sm_partition_destroy synchronises both streams, then releases streams and contexts. */
+int pe_sm_partition_create(int32_t device, int32_t blob_sms, void **stream_blob, void **stream_rest, int32_t *sms_blob,
+                           int32_t *sms_rest);
+int pe_sm_partition_destroy(void *stream_blob, void *stream_rest);
+
 /* ---------------------------------------------------------------- map statistics --------------------------- */
 /* DensityMatrix.meanDensity / stdDensity (pdb_eda/ccp4.py:343-363): population mean and standard deviation of
  * all n stored voxels in float64.  d_out[0] = mean, d_out[1] = std.  d_ws: >= pe_stats_workspace_bytes(). */

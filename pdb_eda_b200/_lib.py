@@ -68,6 +68,8 @@ SIGNATURES = {
     "pe_profile_entries": (ctypes.c_int, []),
     "pe_profile_get": (ctypes.c_int, [ctypes.c_int, ctypes.POINTER(ctypes.c_char_p), ctypes.POINTER(ctypes.c_longlong),
                                       ctypes.POINTER(ctypes.c_double)]),
+    "pe_sm_partition_create": (ctypes.c_int, [_I32, _I32, ctypes.POINTER(_P), ctypes.POINTER(_P), ctypes.POINTER(_I32), ctypes.POINTER(_I32)]),
+    "pe_sm_partition_destroy": (ctypes.c_int, [_P, _P]),
     "pe_stats_workspace_bytes": (_I64, []),
     "pe_map_mean_std": (ctypes.c_int, [_P, _I64, _P, _P, _P]),
     "pe_map_sum_abs": (ctypes.c_int, [_P, _I64, _F32, _P, _P, _P]),

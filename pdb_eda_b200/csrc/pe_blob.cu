@@ -771,11 +771,14 @@ int pe_blob_label(const pe_geom *g, const float *d_rho, float cut_pos, float cut
         PE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, blob_sparse_kernel, kSparseThreads, 0));
         PE_CHECK_ARG(blocks_per_sm > 0, "pe_blob_label: the sparse kernel does not fit an SM");
     }
-    const int nblocks = sm_count() * (blocks_per_sm < 3 ? blocks_per_sm : 3);
+    // the SMs of the launching stream: on an SM partition the grid fills exactly the partition's SMs (a larger cooperative grid is
+    // a launch error, never a wait), so that "3 blocks on every SM" below still holds there
+    const int sms = stream_sm_count(st);
+    const int nblocks = sms * (blocks_per_sm < 3 ? blocks_per_sm : 3);
     // P1 runs on two blocks per SM (384^3: 13.7 us against 16.7 us with all three scanning; 768^3 / 1024^3: no difference)
     // -- only when exactly 3 blocks fill an SM, so that every SM is known to hold 3 of the grid's blocks; otherwise every block scans
     a.p1_per_sm = blocks_per_sm == 3 ? kScanBlocksPerSm : (blocks_per_sm < 3 ? blocks_per_sm : 3);
-    a.p1_blocks = sm_count() * a.p1_per_sm;
+    a.p1_blocks = sms * a.p1_per_sm;
     a.sm_rank = (int *)(ws + p.off_seg + align_up(p.nseg * 4, 256));
     pe_geom geom = *g;
     void *args[] = {(void *)&geom, (void *)&a};

@@ -57,6 +57,9 @@ struct ProfScope {
     } while (0)
 
 int sm_count();  // cached SM count of the current device (148 on B200)
+// SMs a kernel launched on st can use: those of the stream's green context (pe_sm_partition_create), else sm_count().  Grids
+// sized to be resident (persistent and cooperative kernels) take this, so that they fill a partition and never exceed it.
+int stream_sm_count(cudaStream_t st);
 int check_geom(const pe_geom *g);  // host-side validation shared by the entry points (pe_map.cu)
 int check_geom_shape(const pe_geom *g, int64_t *nvox_out);  // the same without the 2^31-voxel limit of one call
 

@@ -378,7 +378,7 @@ int launch_union_warp(const pe_geom *g, const float *d_rho, int n_groups, const 
     PE_CUDA(cudaMemsetAsync(d_counter, 0, sizeof(int), st));
     const int warps_needed = n_groups + (n_quad_atoms + kAtomsPerWarp - 1) / kAtomsPerWarp;
     int grid = (warps_needed + kUW - 1) / kUW;
-    const int max_grid = sm_count() * kUCtas;
+    const int max_grid = stream_sm_count(st) * kUCtas;
     if (grid > max_grid) grid = max_grid;
     if (mode == 0)
         PE_LAUNCH("sphere_union_kernel", st, sphere_union_warp_kernel<0><<<grid, kUW * 32, 0, st>>>(

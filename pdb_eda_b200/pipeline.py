@@ -11,14 +11,67 @@ workspaces) and enqueues, without host synchronisation, the three voxel workload
 
 It is what ``bench.py`` times and what ``DensityAnalysis`` uses for its batched queries.
 """
+import atexit
 import ctypes
+import os
+import warnings
 
 import numpy as np
 import torch
 
-from . import _device
+from . import _device, _lib
 from ._device import _ptr, _stream
 from ._lib import PE_SPHERE_NOUT, check
+
+# SMs the blob pass gets in VoxelPass.step, the other SMs running the sphere kernel (profiles/r05_partitioned_step.md);
+# PDB_EDA_B200_BLOB_SMS overrides it, 0 shares all SMs between the two passes.
+BLOB_SMS = 48
+_partitions = {}   # (device index, blob SMs) -> (blob stream, sphere stream) of a live SM partition, or None where there is none
+
+
+def blobSms():
+    """The blob pass's SM count for VoxelPass.step: PDB_EDA_B200_BLOB_SMS when set, else BLOB_SMS."""
+    text = os.environ.get("PDB_EDA_B200_BLOB_SMS")
+    if text is None:
+        return BLOB_SMS
+    try:
+        return int(text)
+    except ValueError:
+        return -1                                   # not a count: smPartition refuses it and says so once
+
+
+def smPartition(device, blobSms):
+    """(blob stream, sphere stream) of a partition of ``device`` into ``blobSms`` SMs and the rest (pe_sm_partition_create), as
+    torch streams, made once per process, device and count; None for 0, and None with one warning when the count is not one the
+    driver splits exactly or the driver has no green contexts."""
+    index = device.index if device.index is not None else torch.cuda.current_device()
+    key = (index, blobSms)
+    if key in _partitions:
+        return _partitions[key]
+    part = None
+    if blobSms != 0:
+        lib = _lib.load()
+        sb, sr, nb, nr = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_int32(), ctypes.c_int32()
+        rc = lib.pe_sm_partition_create(index, blobSms, ctypes.byref(sb), ctypes.byref(sr), ctypes.byref(nb), ctypes.byref(nr))
+        if rc == 0:
+            dev = torch.device("cuda", index)
+            part = (torch.cuda.ExternalStream(sb.value, device=dev), torch.cuda.ExternalStream(sr.value, device=dev))
+        else:
+            warnings.warn("VoxelPass.step: no partition of %d SMs for the blob pass on cuda:%d (%s); the blob and sphere passes "
+                          "share the SMs" % (blobSms, index, lib.pe_last_error().decode("utf-8", "replace")), RuntimeWarning, stacklevel=3)
+    _partitions[key] = part
+    return part
+
+
+@atexit.register
+def releasePartitions():
+    """Destroys every SM partition made so far (their streams are synchronised first); the next step makes them again."""
+    lib = _lib.load() if _partitions else None
+    for key in list(_partitions):
+        part = _partitions.pop(key)
+        if part is not None:
+            check(lib.pe_sm_partition_destroy(ctypes.c_void_p(part[0].cuda_stream), ctypes.c_void_p(part[1].cuda_stream)),
+                  "pe_sm_partition_destroy")
 
 
 class VoxelPass:
@@ -77,19 +130,29 @@ class VoxelPass:
 
     def step(self):
         """One pass.  The blob pass reads only the Fo-Fc map and the sphere passes only the 2Fo-Fc map, so the two run on two
-        streams (fork / join by events): the HBM-bound threshold kernel overlaps the issue-bound sphere kernel, and the sphere
-        kernel fills the SMs that the latency-bound sparse labelling leaves idle (C2 on one B200: 0.2347 against 0.2414 ms
-        per step in series, profiles/r03_fused_cloud.md)."""
+        streams forked from and joined back to torch's current stream by events.  Each kernel fills every SM it is given up to
+        its occupancy, so on shared SMs the block scheduler runs them nearly one after the other; by default the blob pass
+        therefore runs on its own partition of blobSms() SMs and the sphere kernel on the other SMs, each at its full per-SM
+        occupancy (profiles/r05_partitioned_step.md).  With 0 SMs, or where no partition can be made, both share all SMs."""
+        part = smPartition(self.device, blobSms())
         if getattr(self, "_side", None) is None:
             self._side = torch.cuda.Stream(device=self.device)
-            self._fork, self._join = torch.cuda.Event(), torch.cuda.Event()
+            self._fork, self._join, self._join_rest = torch.cuda.Event(), torch.cuda.Event(), torch.cuda.Event()
         main = torch.cuda.current_stream()
         self._fork.record(main)
-        self._side.wait_event(self._fork)
-        with torch.cuda.stream(self._side):
+        blob_stream = part[0] if part is not None else self._side
+        blob_stream.wait_event(self._fork)
+        with torch.cuda.stream(blob_stream):
             self.blobs()
-        self.spheres()
-        self._join.record(self._side)
+        if part is not None:
+            part[1].wait_event(self._fork)
+            with torch.cuda.stream(part[1]):
+                self.spheres()
+            self._join_rest.record(part[1])
+            main.wait_event(self._join_rest)
+        else:
+            self.spheres()
+        self._join.record(blob_stream)
         main.wait_event(self._join)
 
     def stepFromHost(self, hostDensity, hostDiff, hostXyz=None):
